@@ -104,6 +104,28 @@ int ljmd_run(ljmd_t* h, const float* R_in, const float* V_in, float* R_out, floa
              int64_t energy_every, float* ke_pe,
              float thermostat_kT, int64_t thermostat_every);
 
+/* ---- pair virial and pressure (new; the reference has neither - see DESIGN.md) ---------- */
+/* W(R) = sum over unordered pairs i<j with r^2 < rc^2 of r_ij . f_ij = sum 24 eps (2 (sigma/r)^12 - (sigma/r)^6),
+ * with the minimum image, the fp32 pair set {r^2 < rc^2} and the 1/r^2 (MUFU.RCP) of the force that moves the
+ * particles: per pair w = t * (1/r^2)^3 with t = c12 (1/r^2)^3 - c6 the force's own factor, accumulated where and
+ * with the weight that PE is, and finished with PE's 1/2.  rc = none: all pairs, as the reference.  No tail and
+ * no impulsive correction for the truncation at rc (PE has neither): W is the virial of exactly the forces the
+ * integrator applies.  The pressure of the 2-D fluid (unit mass, k_B = 1) is P = (KE + W/2) / box^2.
+ * Single-GPU handles only: multi-GPU handles return LJMD_E_UNSUPPORTED from both calls.
+ *
+ * ljmd_virial: W of R as one device float, like ljmd_energy.  w_dev: device float[1].                    */
+int ljmd_virial(ljmd_t* h, const float* R, float* w_dev);
+
+/* ljmd_run plus the virial trace: w[i / energy_every] = W of the post-step state on exactly the rows where
+ * ke_pe is written (the KE of a thermostat step there is the value before the rescale, as for ke_pe).
+ * w: device float[ceil(nsteps/energy_every)].  w == NULL: this is ljmd_run.  w != NULL without ke_pe and
+ * energy_every > 0: LJMD_E_INVALID.  The trajectory, the final state and ke_pe are bit for bit those of
+ * ljmd_run: W is summed on the energy steps only, by a separate instantiation of the step kernel.        */
+int ljmd_run_virial(ljmd_t* h, const float* R_in, const float* V_in, float* R_out, float* V_out,
+                    int64_t nsteps, int64_t sample_every, float* traj,
+                    int64_t energy_every, float* ke_pe,
+                    float thermostat_kT, int64_t thermostat_every, float* w);
+
 /* calculate_g_r histogram stage (get_histogram, MD:117-124) for S snapshots:
  * counts[s*nbins + k] = number of unordered pairs (i<j) of snapshot s whose minimum-image
  * distance r satisfies edges[k] <= r < edges[k+1] (last bin right-closed, values outside

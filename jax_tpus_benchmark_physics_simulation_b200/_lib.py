@@ -22,7 +22,7 @@ EXPORTS = (
     "ljmd_forces", "ljmd_run", "ljmd_gr_hist", "ljmd_cell_geometry", "ljmd_cell_assign",
     "ljmd_neighbor_count", "ljmd_last_rebuilds", "ljmd_get_unique_id", "ljmd_create_dist",
     "ljmd_last_run_ms", "ljmd_launch_count", "ljmd_fp32_peak_probe", "ljmd_allpairs_mode",
-    "ljmd_check", "ljmd_pair_accel", "ljmd_run_blocked",
+    "ljmd_check", "ljmd_pair_accel", "ljmd_run_blocked", "ljmd_virial", "ljmd_run_virial",
 )
 
 
@@ -74,6 +74,8 @@ def load() -> ctypes.CDLL:
     lib.ljmd_energy.argtypes = [vp, vp, vp]
     lib.ljmd_forces.argtypes = [vp, vp, vp, vp]
     lib.ljmd_run.argtypes = [vp, vp, vp, vp, vp, i64, i64, vp, i64, vp, f32, i64]
+    lib.ljmd_virial.argtypes = [vp, vp, vp]
+    lib.ljmd_run_virial.argtypes = [vp, vp, vp, vp, vp, i64, i64, vp, i64, vp, f32, i64, vp]
     lib.ljmd_run_blocked.argtypes = [vp, vp, vp, vp, vp, i64, i64, vp]
     lib.ljmd_gr_hist.argtypes = [vp, vp, i64, i32, vp, vp]
     lib.ljmd_cell_geometry.argtypes = [vp, ctypes.POINTER(i32), ctypes.POINTER(i32), ctypes.POINTER(i32),

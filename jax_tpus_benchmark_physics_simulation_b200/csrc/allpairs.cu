@@ -26,6 +26,7 @@
 
 #include <algorithm>
 #include <cstdio>
+#include <type_traits>
 
 namespace cg = cooperative_groups;
 
@@ -99,15 +100,20 @@ struct ApArgs {
     float2*          V_out;
     float2*          F_out;
     float*           pe_out;
+    // virial kernels (VIR): per-CTA / per-patch partial virial like pe_part, and the output: W of R_in
+    // when nsteps == 0, else one float per ke_pe row
+    float*           vir_part;    // [2*npe]
+    float*           vir_out;
 };
 
 // ---- phase [b]: one segment = (i-block ib) x (j units [ju0, ju0+julen)) ---------------------
 // Shared-memory tile layout: one float4 per j particle = (-xj, -xj, -yj, -yj): a single
 // broadcast LDS.128 feeds the packed (two i per thread) pair evaluation.
-template <int IPT, bool CUTOFF, bool PE>
+template <int IPT, bool CUTOFF, bool PE, bool VIR>
 __device__ __forceinline__ void ap_segment(const ApArgs& a, const float2* __restrict__ Rcur,
                                            int ib, int ju0, int julen, float4* sj,
-                                           float (&fx)[IPT], float (&fy)[IPT], float& pe_acc) {
+                                           float (&fx)[IPT], float (&fy)[IPT], float& pe_acc,
+                                           float& vir_acc) {
     constexpr int BI = AP_THREADS * IPT;
     const int tid = threadIdx.x;
     const PairConsts pc = a.pc;
@@ -140,7 +146,7 @@ __device__ __forceinline__ void ap_segment(const ApArgs& a, const float2* __rest
         const int qd0 = min(max(i_lo - jt, 0), cnt), qd1 = min(max(i_hi - jt, 0), cnt);
         if constexpr (IPT == 2) {
             const float2 xi2 = make_float2(xi[0], xi[1]), yi2 = make_float2(yi[0], yi[1]);
-            float2 tfx = make_float2(0.0f, 0.0f), tfy = tfx, tpe = tfx;   // per-tile sums
+            float2 tfx = make_float2(0.0f, 0.0f), tfy = tfx, tpe = tfx, tvir = tfx;   // per-tile sums
 #pragma unroll 1
             for (int part = 0; part < 3; ++part) {
                 const int qa = (part == 0) ? 0 : (part == 1 ? qd0 : qd1);
@@ -149,23 +155,24 @@ __device__ __forceinline__ void ap_segment(const ApArgs& a, const float2* __rest
 #pragma unroll kApUnroll
                     for (int q = qa; q < qb; ++q) {
                         const float4 v = sj[q];            // one j particle, warp broadcast
-                        pair2_accum<CUTOFF, PE, false>(xi2, yi2, make_float2(v.x, v.y), make_float2(v.z, v.w),
-                                                       true, true, pc, pc2, tfx, tfy, tpe);
+                        pair2_accum<CUTOFF, PE, false, VIR>(xi2, yi2, make_float2(v.x, v.y), make_float2(v.z, v.w),
+                                                            true, true, pc, pc2, tfx, tfy, tpe, tvir);
                     }
                 } else {
 #pragma unroll kApUnroll
                     for (int q = qa; q < qb; ++q) {
                         const float4 v = sj[q];
                         const int j = jt + q;
-                        pair2_accum<CUTOFF, PE, true>(xi2, yi2, make_float2(v.x, v.y), make_float2(v.z, v.w),
-                                                      j != ii[0], j != ii[1], pc, pc2, tfx, tfy, tpe);
+                        pair2_accum<CUTOFF, PE, true, VIR>(xi2, yi2, make_float2(v.x, v.y), make_float2(v.z, v.w),
+                                                           j != ii[0], j != ii[1], pc, pc2, tfx, tfy, tpe, tvir);
                     }
                 }
             }
             fx[0] += tfx.x; fx[1] += tfx.y; fy[0] += tfy.x; fy[1] += tfy.y;
             if (PE) pe_acc += tpe.x + tpe.y;
+            if (VIR) vir_acc += tvir.x + tvir.y;
         } else {
-            float tfx = 0.0f, tfy = 0.0f, tpe = 0.0f;
+            float tfx = 0.0f, tfy = 0.0f, tpe = 0.0f, tvir = 0.0f;
 #pragma unroll 1
             for (int part = 0; part < 3; ++part) {
                 const int qa = (part == 0) ? 0 : (part == 1 ? qd0 : qd1);
@@ -174,18 +181,20 @@ __device__ __forceinline__ void ap_segment(const ApArgs& a, const float2* __rest
 #pragma unroll kApUnroll
                     for (int q = qa; q < qb; ++q) {
                         const float4 v = sj[q];
-                        pair_accum<CUTOFF, PE, false>(xi[0], yi[0], -v.x, -v.z, true, pc, tfx, tfy, tpe);
+                        pair_accum<CUTOFF, PE, false, VIR>(xi[0], yi[0], -v.x, -v.z, true, pc, tfx, tfy, tpe, tvir);
                     }
                 } else {
 #pragma unroll kApUnroll
                     for (int q = qa; q < qb; ++q) {
                         const float4 v = sj[q];
-                        pair_accum<CUTOFF, PE, true>(xi[0], yi[0], -v.x, -v.z, (jt + q) != ii[0], pc, tfx, tfy, tpe);
+                        pair_accum<CUTOFF, PE, true, VIR>(xi[0], yi[0], -v.x, -v.z, (jt + q) != ii[0], pc, tfx, tfy, tpe,
+                                                          tvir);
                     }
                 }
             }
             fx[0] += tfx; fy[0] += tfy;
             if (PE) pe_acc += tpe;
+            if (VIR) vir_acc += tvir;
         }
     }
 }
@@ -199,10 +208,11 @@ constexpr int T3_BLK = 64;
 
 __device__ __forceinline__ int tri_base(int pa, int npr) { return pa * npr - (pa * (pa - 1)) / 2; }
 
-template <bool CUTOFF, bool PE, bool N3L>
+template <bool CUTOFF, bool PE, bool N3L, bool VIR>
 __device__ __forceinline__ void tile_half(const PairConsts& pc, const PairConsts2& pc2, float2 xi2,
                                           float2 yi2, float xj, float yj, bool self0, bool self1,
-                                          float2& fx2, float2& fy2, float2& pe2, float& fjx, float& fjy) {
+                                          float2& fx2, float2& fy2, float2& pe2, float2& vir2,
+                                          float& fjx, float& fjy) {
     const int src = (threadIdx.x + 1) & 31;
     // the reaction on the travelling j is accumulated as ONE scalar per component (the two i of this
     // lane are added in a fixed order), so only two values per component... per step two shuffles
@@ -211,8 +221,8 @@ __device__ __forceinline__ void tile_half(const PairConsts& pc, const PairConsts
     // step 0 peeled: the only step at which j can be one of this lane's own i (diagonal tiles)
     {
         float2 f, dx, dy;
-        if (N3L) pair2_eval<CUTOFF, PE, false>(xi2, yi2, xj, yj, true, true, pc, pc2, f, dx, dy, pe2);
-        else     pair2_eval<CUTOFF, PE, true >(xi2, yi2, xj, yj, !self0, !self1, pc, pc2, f, dx, dy, pe2);
+        if (N3L) pair2_eval<CUTOFF, PE, false, VIR>(xi2, yi2, xj, yj, true, true, pc, pc2, f, dx, dy, pe2, vir2);
+        else     pair2_eval<CUTOFF, PE, true,  VIR>(xi2, yi2, xj, yj, !self0, !self1, pc, pc2, f, dx, dy, pe2, vir2);
         fx2 = __ffma2_rn(f, dx, fx2);
         fy2 = __ffma2_rn(f, dy, fy2);
         if (N3L) {
@@ -226,7 +236,7 @@ __device__ __forceinline__ void tile_half(const PairConsts& pc, const PairConsts
 #pragma unroll 4
     for (int s = 1; s < 32; ++s) {
         float2 f, dx, dy;
-        pair2_eval<CUTOFF, PE, false>(xi2, yi2, xj, yj, true, true, pc, pc2, f, dx, dy, pe2);
+        pair2_eval<CUTOFF, PE, false, VIR>(xi2, yi2, xj, yj, true, true, pc, pc2, f, dx, dy, pe2, vir2);
         fx2 = __ffma2_rn(f, dx, fx2);
         fy2 = __ffma2_rn(f, dy, fy2);
         if (N3L) {
@@ -246,10 +256,10 @@ __device__ __forceinline__ void tile_half(const PairConsts& pc, const PairConsts
 // j + 32) are independent dependency chains (evaluate -> accumulate the reaction -> four shuffles), so
 // interleaving them doubles the instruction-level parallelism of a warp that shares its scheduler with
 // only three others (107 registers: 4 CTAs of 4 warps per SM).  Same arithmetic per pair as tile_half.
-template <bool CUTOFF, bool PE, bool N3L>
+template <bool CUTOFF, bool PE, bool N3L, bool VIR>
 __device__ __forceinline__ void tile_both(const PairConsts& pc, const PairConsts2& pc2, float2 xi2, float2 yi2,
                                           float xja, float yja, float xjb, float yjb,
-                                          float2& fx2, float2& fy2, float2& pe2,
+                                          float2& fx2, float2& fy2, float2& pe2, float2& vir2,
                                           float& fjxa, float& fjya, float& fjxb, float& fjyb) {
     const int src = (threadIdx.x + 1) & 31;
     float aax = 0.0f, aay = 0.0f, abx = 0.0f, aby = 0.0f;
@@ -258,11 +268,11 @@ __device__ __forceinline__ void tile_both(const PairConsts& pc, const PairConsts
         // half a meets i0 (self0), half b meets i1 (self1)
         float2 fa, dxa, dya, fb, dxb, dyb;
         if (N3L) {
-            pair2_eval<CUTOFF, PE, false>(xi2, yi2, xja, yja, true, true, pc, pc2, fa, dxa, dya, pe2);
-            pair2_eval<CUTOFF, PE, false>(xi2, yi2, xjb, yjb, true, true, pc, pc2, fb, dxb, dyb, pe2);
+            pair2_eval<CUTOFF, PE, false, VIR>(xi2, yi2, xja, yja, true, true, pc, pc2, fa, dxa, dya, pe2, vir2);
+            pair2_eval<CUTOFF, PE, false, VIR>(xi2, yi2, xjb, yjb, true, true, pc, pc2, fb, dxb, dyb, pe2, vir2);
         } else {
-            pair2_eval<CUTOFF, PE, true>(xi2, yi2, xja, yja, false, true, pc, pc2, fa, dxa, dya, pe2);
-            pair2_eval<CUTOFF, PE, true>(xi2, yi2, xjb, yjb, true, false, pc, pc2, fb, dxb, dyb, pe2);
+            pair2_eval<CUTOFF, PE, true, VIR>(xi2, yi2, xja, yja, false, true, pc, pc2, fa, dxa, dya, pe2, vir2);
+            pair2_eval<CUTOFF, PE, true, VIR>(xi2, yi2, xjb, yjb, true, false, pc, pc2, fb, dxb, dyb, pe2, vir2);
         }
         fx2 = __ffma2_rn(fa, dxa, fx2); fy2 = __ffma2_rn(fa, dya, fy2);
         gx2 = __ffma2_rn(fb, dxb, gx2); gy2 = __ffma2_rn(fb, dyb, gy2);
@@ -280,8 +290,8 @@ __device__ __forceinline__ void tile_both(const PairConsts& pc, const PairConsts
 #pragma unroll kTileBothUnroll
     for (int s = 1; s < 32; ++s) {
         float2 fa, dxa, dya, fb, dxb, dyb;
-        pair2_eval<CUTOFF, PE, false>(xi2, yi2, xja, yja, true, true, pc, pc2, fa, dxa, dya, pe2);
-        pair2_eval<CUTOFF, PE, false>(xi2, yi2, xjb, yjb, true, true, pc, pc2, fb, dxb, dyb, pe2);
+        pair2_eval<CUTOFF, PE, false, VIR>(xi2, yi2, xja, yja, true, true, pc, pc2, fa, dxa, dya, pe2, vir2);
+        pair2_eval<CUTOFF, PE, false, VIR>(xi2, yi2, xjb, yjb, true, true, pc, pc2, fb, dxb, dyb, pe2, vir2);
         fx2 = __ffma2_rn(fa, dxa, fx2); fy2 = __ffma2_rn(fa, dya, fy2);
         gx2 = __ffma2_rn(fb, dxb, gx2); gy2 = __ffma2_rn(fb, dyb, gy2);
         if (N3L) {
@@ -303,7 +313,7 @@ __device__ __forceinline__ float2 ld_pos(const float2* __restrict__ R, int j, in
     return (j < N) ? __ldcg(&R[j]) : make_float2(sent, sent);
 }
 
-template <bool CUTOFF, bool PE>
+template <bool CUTOFF, bool PE, bool VIR>
 __device__ __forceinline__ void ap3_phase_forces(const ApArgs& a, const float2* __restrict__ Rcur,
                                                  float2* sacc /* 4 warps x 2 x q x 64 */, float* sred,
                                                  int par) {
@@ -322,7 +332,7 @@ __device__ __forceinline__ void ap3_phase_forces(const ApArgs& a, const float2* 
         __syncthreads();
         const int pi = s_pi;
         if (pi >= a.npatch) break;
-        float pe_thread = 0.0f;
+        float pe_thread = 0.0f, vir_thread = 0.0f;
         const int2 pp = a.patches[pi];
         // the partial vectors are indexed by position in the patch list (on one GPU the list is the whole
         // triangle in (pa, pb) order: that index is tri_base(pa) + pb - pa, which the reduction relies on)
@@ -338,7 +348,7 @@ __device__ __forceinline__ void ap3_phase_forces(const ApArgs& a, const float2* 
             for (int cc = 0; cc < q; ++cc) {
                 const int bb = pp.y * Pt + wc * q + cc;         // j block
                 if (ba > bb) continue;                          // lower triangle (diagonal patches only)
-                float2 pe2 = make_float2(0.0f, 0.0f);
+                float2 pe2 = make_float2(0.0f, 0.0f), vir2 = pe2;
                 float2 tfx = make_float2(0.0f, 0.0f), tfy = tfx;   // per-tile sums (bounded chains)
 #if AP_TILE_BOTH
                 {
@@ -346,8 +356,8 @@ __device__ __forceinline__ void ap3_phase_forces(const ApArgs& a, const float2* 
                     const float2 pa = ld_pos(Rcur, ja, a.N, SENT_J), pb = ld_pos(Rcur, jb, a.N, SENT_J);
                     float fjxa, fjya, fjxb, fjyb;
                     if (ba < bb) {
-                        tile_both<CUTOFF, PE, true>(pc, pc2, xi2, yi2, pa.x, pa.y, pb.x, pb.y, tfx, tfy, pe2,
-                                                    fjxa, fjya, fjxb, fjyb);
+                        tile_both<CUTOFF, PE, true, VIR>(pc, pc2, xi2, yi2, pa.x, pa.y, pb.x, pb.y, tfx, tfy, pe2, vir2,
+                                                         fjxa, fjya, fjxb, fjyb);
                         float2 acc = colacc[cc * T3_BLK + lane];
                         acc.x += fjxa; acc.y += fjya;
                         colacc[cc * T3_BLK + lane] = acc;
@@ -355,8 +365,8 @@ __device__ __forceinline__ void ap3_phase_forces(const ApArgs& a, const float2* 
                         acc.x += fjxb; acc.y += fjyb;
                         colacc[cc * T3_BLK + 32 + lane] = acc;
                     } else {
-                        tile_both<CUTOFF, PE, false>(pc, pc2, xi2, yi2, pa.x, pa.y, pb.x, pb.y, tfx, tfy, pe2,
-                                                     fjxa, fjya, fjxb, fjyb);
+                        tile_both<CUTOFF, PE, false, VIR>(pc, pc2, xi2, yi2, pa.x, pa.y, pb.x, pb.y, tfx, tfy, pe2, vir2,
+                                                          fjxa, fjya, fjxb, fjyb);
                     }
                 }
 #else
@@ -366,12 +376,12 @@ __device__ __forceinline__ void ap3_phase_forces(const ApArgs& a, const float2* 
                     const float2 pj = ld_pos(Rcur, j, a.N, SENT_J);
                     float fjx, fjy;
                     if (ba < bb) {
-                        tile_half<CUTOFF, PE, true>(pc, pc2, xi2, yi2, pj.x, pj.y, false, false, tfx, tfy, pe2, fjx, fjy);
+                        tile_half<CUTOFF, PE, true, VIR>(pc, pc2, xi2, yi2, pj.x, pj.y, false, false, tfx, tfy, pe2, vir2, fjx, fjy);
                         float2 acc = colacc[cc * T3_BLK + h * 32 + lane];
                         acc.x += fjx; acc.y += fjy;
                         colacc[cc * T3_BLK + h * 32 + lane] = acc;
                     } else {
-                        tile_half<CUTOFF, PE, false>(pc, pc2, xi2, yi2, pj.x, pj.y, h == 0, h == 1, tfx, tfy, pe2, fjx, fjy);
+                        tile_half<CUTOFF, PE, false, VIR>(pc, pc2, xi2, yi2, pj.x, pj.y, h == 0, h == 1, tfx, tfy, pe2, vir2, fjx, fjy);
                     }
                 }
 #endif
@@ -379,6 +389,7 @@ __device__ __forceinline__ void ap3_phase_forces(const ApArgs& a, const float2* 
                 // energy bookkeeping in the ORDERED-pair convention of the caller (0.5 * sum):
                 // an unordered pair of an off-diagonal tile counts twice, a diagonal tile is ordered
                 if (PE) pe_thread += (ba < bb ? 2.0f : 1.0f) * (pe2.x + pe2.y);
+                if (VIR) vir_thread += (ba < bb ? 2.0f : 1.0f) * (vir2.x + vir2.y);   // same weights
             }
             rowacc[r * T3_BLK + lane]      = make_float2(fx2.x, fy2.x);
             rowacc[r * T3_BLK + 32 + lane] = make_float2(fx2.y, fy2.y);
@@ -401,11 +412,15 @@ __device__ __forceinline__ void ap3_phase_forces(const ApArgs& a, const float2* 
             float t = block_sum<AP_THREADS>(pe_thread, sred);
             if (tid == 0) __stcg(&a.pe_part[par * a.npe + pid], t);
         }
+        if (VIR) {
+            float t = block_sum<AP_THREADS>(vir_thread, sred);
+            if (tid == 0) __stcg(&a.vir_part[par * a.npe + pid], t);
+        }
         __syncthreads();
     }
 }
 
-template <int IPT, bool CUTOFF, bool PE>
+template <int IPT, bool CUTOFF, bool PE, bool VIR>
 __device__ __forceinline__ void ap_phase_forces(const ApArgs& a, const float2* __restrict__ Rcur,
                                                 float4* sj, float* sred, int par) {
     constexpr int BI = AP_THREADS * IPT;
@@ -413,13 +428,13 @@ __device__ __forceinline__ void ap_phase_forces(const ApArgs& a, const float2* _
     long long w = a.cta_start[c];
     const long long w1 = a.cta_start[c + 1];
     int seg = 0;
-    float pe_thread = 0.0f;
+    float pe_thread = 0.0f, vir_thread = 0.0f;
     while (w < w1) {
         const int ib = (int)(w / a.NJu);
         const int ju0 = (int)(w - (long long)ib * a.NJu);
         const int len = (int)min((long long)(a.NJu - ju0), w1 - w);
         float fx[IPT], fy[IPT];
-        ap_segment<IPT, CUTOFF, PE>(a, Rcur, ib, ju0, len, sj, fx, fy, pe_thread);
+        ap_segment<IPT, CUTOFF, PE, VIR>(a, Rcur, ib, ju0, len, sj, fx, fy, pe_thread, vir_thread);
         float2* dst = a.part + ((size_t)c * a.maxseg + seg) * BI;
 #pragma unroll
         for (int k = 0; k < IPT; ++k) __stcg(&dst[k * AP_THREADS + tid], make_float2(fx[k], fy[k]));
@@ -430,6 +445,10 @@ __device__ __forceinline__ void ap_phase_forces(const ApArgs& a, const float2* _
         float t = block_sum<AP_THREADS>(pe_thread, sred);
         if (tid == 0) __stcg(&a.pe_part[par * a.npe + c], t);
     }
+    if (VIR) {
+        float t = block_sum<AP_THREADS>(vir_thread, sred);
+        if (tid == 0) __stcg(&a.vir_part[par * a.npe + c], t);
+    }
 }
 
 // fixed-order sum of a per-CTA partial array by one warp, in double
@@ -439,7 +458,9 @@ __device__ __forceinline__ double warp_sum_array(const float* p, int n) {
     return warp_sum(s);
 }
 
-template <int IPT, bool CUTOFF>
+// VIR: the energy steps also accumulate the pair virial (a separate instantiation, launched only when the
+// caller asked for it, so that the force-only kernels stay exactly as they are)
+template <int IPT, bool CUTOFF, bool VIR>
 __global__ void __launch_bounds__(AP_THREADS, AP_MINBLOCKS)
 ap_persistent_kernel(const ApArgs a) {
     constexpr int BI = AP_THREADS * (IPT == 3 ? 1 : IPT);
@@ -463,7 +484,8 @@ ap_persistent_kernel(const ApArgs a) {
         const bool kick1   = (s >= 0);                     // prologue only evaluates F(R_in)
         const bool final   = (s == rc.nsteps - 1);
         const bool want_e  = kick1 && rc.energy_every > 0 && (s % rc.energy_every == 0);
-        const bool want_pe = want_e || (rc.nsteps == 0 && a.pe_out != nullptr);
+        bool       want_pe = want_e || (rc.nsteps == 0 && a.pe_out != nullptr);
+        if constexpr (VIR) want_pe = want_pe || (rc.nsteps == 0 && a.vir_out != nullptr);   // ljmd_virial
         const bool thermo  = kick1 && rc.thermo_every > 0 && rc.thermo_kT > 0.0f &&
                              ((s + 1) % rc.thermo_every == 0);
         const bool sample  = kick1 && rc.sample_every > 0 && (s % rc.sample_every == 0) &&
@@ -473,11 +495,11 @@ ap_persistent_kernel(const ApArgs a) {
         // ---- [b] partial forces of R_cur ------------------------------------------------------
         if constexpr (V3) {
             if (c == 0 && tid == 0) __stcg(&a.sched[par ^ 1], 0);   // the other parity's patch counter
-            if (want_pe) ap3_phase_forces<CUTOFF, true >(a, Rcur, reinterpret_cast<float2*>(smem_buf), sred, par);
-            else         ap3_phase_forces<CUTOFF, false>(a, Rcur, reinterpret_cast<float2*>(smem_buf), sred, par);
+            if (want_pe) ap3_phase_forces<CUTOFF, true,  VIR  >(a, Rcur, reinterpret_cast<float2*>(smem_buf), sred, par);
+            else         ap3_phase_forces<CUTOFF, false, false>(a, Rcur, reinterpret_cast<float2*>(smem_buf), sred, par);
         } else {
-            if (want_pe) ap_phase_forces<IPT, CUTOFF, true >(a, Rcur, sj, sred, par);
-            else         ap_phase_forces<IPT, CUTOFF, false>(a, Rcur, sj, sred, par);
+            if (want_pe) ap_phase_forces<IPT, CUTOFF, true,  VIR  >(a, Rcur, sj, sred, par);
+            else         ap_phase_forces<IPT, CUTOFF, false, false>(a, Rcur, sj, sred, par);
         }
         if (prof) { long long t = clock64(); pt[0] += t - pt[4]; pt[4] = t; }
         grid_barrier(a.bar, (++epoch) * (unsigned)a.G, a.err, a.spin_limit);
@@ -696,13 +718,16 @@ ap_persistent_kernel(const ApArgs a) {
         if (c == 0 && tid < 32 && want_pe) {
             double pe2 = warp_sum_array(a.pe_part + par * a.npe, a.npe);
             double ke2 = want_e ? warp_sum_array(a.ke_part + par * a.G, a.G) : 0.0;
+            double w2 = VIR ? warp_sum_array(a.vir_part + par * a.npe, a.npe) : 0.0;
             if (tid == 0) {
                 if (want_e) {
                     float* o = rc.ke_pe + 2 * (s / rc.energy_every);
                     o[0] = (float)(0.5 * ke2);
                     o[1] = (float)(0.5 * pe2);             // MD:61  0.5 * sum over ordered pairs
+                    if (VIR) a.vir_out[s / rc.energy_every] = (float)(0.5 * w2);   // same weights, same 1/2
                 } else {
-                    a.pe_out[0] = (float)(0.5 * pe2);
+                    if (!VIR || a.pe_out) a.pe_out[0] = (float)(0.5 * pe2);
+                    if (VIR) a.vir_out[0] = (float)(0.5 * w2);
                 }
             }
         }
@@ -741,6 +766,7 @@ struct CluArgs {
     float2 *R_out, *V_out, *F_out;
     float*  pe_out;
     long long* prof;                    // optional [C][4] phase clocks (debug: LJMD_AP_PROF=1)
+    float*  vir_out;                    // virial kernel: W of R_in (nsteps == 0) or one float per ke_pe row
 };
 
 // The force-only slice loop is PREDICATE-FREE.  Inside the kernel the seven predicate registers are held
@@ -754,6 +780,7 @@ struct CluArgs {
 //     diagonal mask does (MD:54-55).  Distinct particles closer than sqrt(r2min) ~ 0.003 sigma overflow
 //     fp32 in the reference itself.  The energy variant (rare steps) keeps the exact index test.
 struct SliceSum { float2 fx, fy, pe; };
+struct SliceSumVir { float2 fx, fy, pe, vir; };     // energy steps of the virial kernel
 
 __device__ __forceinline__ float min_image_bf(float d, float box, float timg) {
     return fmaf(-set_ge_f32(fabsf(d), timg), copysignf(box, d), d);
@@ -790,22 +817,25 @@ __device__ __forceinline__ SliceSum clu_slice_f(const float4* cur, int j0, int j
     return r;
 }
 
-template <bool CUTOFF>
-__device__ __noinline__ SliceSum clu_slice_pe(const float4* cur, int j0, int j1, int i0, int i1, float2 xi2,
-                                              float2 yi2, PairConsts pc) {
+template <bool CUTOFF, bool VIR>
+__device__ __noinline__ std::conditional_t<VIR, SliceSumVir, SliceSum>
+clu_slice_pe(const float4* cur, int j0, int j1, int i0, int i1, float2 xi2, float2 yi2, PairConsts pc) {
     const PairConsts2 pc2 = make_pair_consts2(pc);
-    SliceSum r;
+    std::conditional_t<VIR, SliceSumVir, SliceSum> r;
     r.fx = make_float2(0.0f, 0.0f); r.fy = r.fx; r.pe = r.fx;
+    float2 vir = r.fx;
 #pragma unroll 2
     for (int j = j0; j < j1; ++j) {
         const float4 q = cur[j];
-        pair2_accum<CUTOFF, true, true>(xi2, yi2, make_float2(q.x, q.y), make_float2(q.z, q.w), j != i0, j != i1,
-                                        pc, pc2, r.fx, r.fy, r.pe);
+        pair2_accum<CUTOFF, true, true, VIR>(xi2, yi2, make_float2(q.x, q.y), make_float2(q.z, q.w), j != i0,
+                                             j != i1, pc, pc2, r.fx, r.fy, r.pe, vir);
     }
+    if constexpr (VIR) r.vir = vir;
     return r;
 }
 
-template <bool CUTOFF>
+// VIR: energy steps also sum the pair virial (own instantiation; its per-CTA partials follow sred)
+template <bool CUTOFF, bool VIR>
 __global__ void __launch_bounds__(CLU_THREADS, 1)
 ap_cluster_kernel(const CluArgs a) {
     cg::cluster_group cluster = cg::this_cluster();
@@ -815,6 +845,7 @@ ap_cluster_kernel(const CluArgs a) {
     float*  sE   = reinterpret_cast<float*>(spos + 2 * (size_t)a.N);   // [2 parity][pe, ke][CLU_MAXC] (CTA 0 sums)
     float*  sK   = sE + 4 * CLU_MAXC;                                  // [CLU_MAXC] thermostat kinetic partials
     float*  sred = sK + CLU_MAXC;                                      // [CLU_THREADS / 32]
+    float*  sW   = sred + CLU_THREADS / 32;                            // VIR: [2 parity][CLU_MAXC] (CTA 0 sums)
     __shared__ float s_lambda;
     const RunCtl rc = a.rc;
     const PairConsts pc = a.pc;
@@ -847,7 +878,8 @@ ap_cluster_kernel(const CluArgs a) {
         const bool kick1   = (s >= 0);
         const bool final   = (s == rc.nsteps - 1);
         const bool want_e  = kick1 && rc.energy_every > 0 && (s % rc.energy_every == 0);
-        const bool want_pe = want_e || (rc.nsteps == 0 && a.pe_out != nullptr);
+        bool       want_pe = want_e || (rc.nsteps == 0 && a.pe_out != nullptr);
+        if constexpr (VIR) want_pe = want_pe || (rc.nsteps == 0 && a.vir_out != nullptr);   // ljmd_virial
         const bool thermo  = kick1 && rc.thermo_every > 0 && rc.thermo_kT > 0.0f &&
                              ((s + 1) % rc.thermo_every == 0);
         const bool sample  = kick1 && rc.sample_every > 0 && (s % rc.sample_every == 0) &&
@@ -861,8 +893,19 @@ ap_cluster_kernel(const CluArgs a) {
         if (has0) c0 = cur[i0];
         if (has1) c1 = cur[i1];
         const float2 xi2 = make_float2(-c0.x, -c1.x), yi2 = make_float2(-c0.z, -c1.z);
-        const SliceSum ss = want_pe ? clu_slice_pe<CUTOFF>(cur, j0, j1, i0, i1, xi2, yi2, pc)
-                                    : clu_slice_f<CUTOFF>(cur, j0, j1, xi2, yi2, a.r2min, pc);
+        SliceSum ss;
+        float2 tvir = make_float2(0.0f, 0.0f);
+        if constexpr (VIR) {
+            if (want_pe) {
+                const SliceSumVir sv = clu_slice_pe<CUTOFF, true>(cur, j0, j1, i0, i1, xi2, yi2, pc);
+                ss.fx = sv.fx; ss.fy = sv.fy; ss.pe = sv.pe; tvir = sv.vir;
+            } else {
+                ss = clu_slice_f<CUTOFF>(cur, j0, j1, xi2, yi2, a.r2min, pc);
+            }
+        } else {
+            ss = want_pe ? clu_slice_pe<CUTOFF, false>(cur, j0, j1, i0, i1, xi2, yi2, pc)
+                         : clu_slice_f<CUTOFF>(cur, j0, j1, xi2, yi2, a.r2min, pc);
+        }
         float2 tfx = ss.fx, tfy = ss.fy;
         const float2 tpe = ss.pe;
         for (int o = a.S >> 1; o > 0; o >>= 1) {          // commutative adds: all lanes end bit-identical
@@ -874,6 +917,10 @@ ap_cluster_kernel(const CluArgs a) {
         if (want_pe) {                     // fixed tree: per-CTA potential energy -> CTA 0
             const float t = block_sum<CLU_THREADS>((has0 ? tpe.x : 0.0f) + (has1 ? tpe.y : 0.0f), sred);
             if (tid == 0) *cluster.map_shared_rank(&sE[(par * 2 + 0) * CLU_MAXC + k], 0) = t;
+        }
+        if (VIR && want_pe) {              // the virial partial takes the same route
+            const float t = block_sum<CLU_THREADS>((has0 ? tvir.x : 0.0f) + (has1 ? tvir.y : 0.0f), sred);
+            if (tid == 0) *cluster.map_shared_rank(&sW[par * CLU_MAXC + k], 0) = t;
         }
         if (prof) { const long long t = clock64(); pt[0] += t - tl; tl = t; }
 
@@ -945,15 +992,19 @@ ap_cluster_kernel(const CluArgs a) {
         b ^= 1;
 
         if (k == 0 && tid == 0 && want_pe) {     // energies of the post-step state (fixed order, double)
-            double pe2 = 0.0, ke2 = 0.0;
+            double pe2 = 0.0, ke2 = 0.0, w2 = 0.0;
             for (int q = 0; q < a.C; ++q) pe2 += (double)sE[(par * 2 + 0) * CLU_MAXC + q];
+            if (VIR)
+                for (int q = 0; q < a.C; ++q) w2 += (double)sW[par * CLU_MAXC + q];
             if (want_e) {
                 for (int q = 0; q < a.C; ++q) ke2 += (double)sE[(par * 2 + 1) * CLU_MAXC + q];
                 float* o = rc.ke_pe + 2 * (s / rc.energy_every);
                 o[0] = (float)(0.5 * ke2);
                 o[1] = (float)(0.5 * pe2);       // MD:61  0.5 * sum over ordered pairs
+                if (VIR) a.vir_out[s / rc.energy_every] = (float)(0.5 * w2);
             } else {
-                a.pe_out[0] = (float)(0.5 * pe2);
+                if (!VIR || a.pe_out) a.pe_out[0] = (float)(0.5 * pe2);
+                if (VIR) a.vir_out[0] = (float)(0.5 * w2);
             }
         }
     }
@@ -973,10 +1024,11 @@ using CluKernel = void (*)(const CluArgs);
 
 using ApKernel = void (*)(const ApArgs);
 
+template <bool VIR>
 ApKernel pick_kernel(int ipt, bool cutoff) {
-    if (ipt == 3) return cutoff ? ap_persistent_kernel<3, true> : ap_persistent_kernel<3, false>;
-    if (ipt == 1) return cutoff ? ap_persistent_kernel<1, true> : ap_persistent_kernel<1, false>;
-    return cutoff ? ap_persistent_kernel<2, true> : ap_persistent_kernel<2, false>;
+    if (ipt == 3) return cutoff ? ap_persistent_kernel<3, true, VIR> : ap_persistent_kernel<3, false, VIR>;
+    if (ipt == 1) return cutoff ? ap_persistent_kernel<1, true, VIR> : ap_persistent_kernel<1, false, VIR>;
+    return cutoff ? ap_persistent_kernel<2, true, VIR> : ap_persistent_kernel<2, false, VIR>;
 }
 
 // ---- g(r): pair-distance histogram (get_histogram, MD:117-124) -------------------------------
@@ -1045,7 +1097,7 @@ struct AllPairs {
     int*       d_cta_ib0 = nullptr;
     int2*      d_iblk = nullptr;
     float2 *Rbuf0 = nullptr, *Rbuf1 = nullptr, *Vh = nullptr, *Ftmp = nullptr, *part = nullptr;
-    float *pe_part = nullptr, *ke_part = nullptr;
+    float *pe_part = nullptr, *ke_part = nullptr, *vir_part = nullptr;
     int i_lo = 0, Nloc = 0;
     void* shared = nullptr;             // one allocation (IPC-shareable): Rbuf0 | Rbuf1 | arrival words
     unsigned* xflags = nullptr;
@@ -1057,10 +1109,13 @@ struct AllPairs {
     int* err = nullptr;
     long long* prof = nullptr;
     ApKernel kernel = nullptr;
+    ApKernel kernel_vir = nullptr;      // the same kernel with the virial on energy steps (nullptr: it does not
+                                        // fit the grid of `kernel`)
     // single-cluster kernel for small systems (nullptr: not used)
     CluKernel clu_kernel = nullptr;
+    CluKernel clu_kernel_vir = nullptr;
     int cluC = 0, clu_n_i = 0, clu_half = 0, clu_S = 0, clu_jl = 0;
-    size_t clu_smem = 0;
+    size_t clu_smem = 0, clu_smem_vir = 0;
 };
 
 int ap_mode(ljmd_handle* h) { return h->ap ? (h->ap->clu_kernel ? 4 : h->ap->ipt) : 0; }
@@ -1073,8 +1128,10 @@ static int clu_setup(ljmd_handle* h, AllPairs* ap) {
     long long nmax = 640;
     if (const char* e = getenv("LJMD_AP_CLUSTER_NMAX")) nmax = atoll(e);
     if (std::max(1, h->nranks) != 1 || N > nmax || N > 4096) return 0;
-    CluKernel kern = h->pc.cutoff != 0 ? ap_cluster_kernel<true> : ap_cluster_kernel<false>;
+    CluKernel kern = h->pc.cutoff != 0 ? ap_cluster_kernel<true, false> : ap_cluster_kernel<false, false>;
+    CluKernel kern_vir = h->pc.cutoff != 0 ? ap_cluster_kernel<true, true> : ap_cluster_kernel<false, true>;
     const size_t smem = 32 * (size_t)N + sizeof(float) * (5 * CLU_MAXC + CLU_THREADS / 32);
+    const size_t smem_vir = smem + sizeof(float) * 2 * CLU_MAXC;         // + the virial partials
     if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) { cudaGetLastError(); return 0; }
     int want = CLU_MAXC;
     if (const char* e = getenv("LJMD_AP_CLUSTER_SIZE")) want = std::max(1, std::min(CLU_MAXC, atoi(e)));
@@ -1089,9 +1146,18 @@ static int clu_setup(ljmd_handle* h, AllPairs* ap) {
         int nclusters = 0;
         if (cudaOccupancyMaxActiveClusters(&nclusters, kern, &cfg) != cudaSuccess || nclusters < 1) { cudaGetLastError(); continue; }
         ap->clu_kernel = kern; ap->cluC = C; ap->clu_smem = smem;
+        {   // the virial variant runs with the same cluster (or not at all: ljmd_virial then reports it)
+            cfg.dynamicSmemBytes = smem_vir;
+            if (cudaFuncSetAttribute(kern_vir, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_vir) == cudaSuccess &&
+                (C <= 8 || cudaFuncSetAttribute(kern_vir, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) == cudaSuccess) &&
+                cudaOccupancyMaxActiveClusters(&nclusters, kern_vir, &cfg) == cudaSuccess && nclusters >= 1) {
+                ap->clu_kernel_vir = kern_vir; ap->clu_smem_vir = smem_vir;
+            }
+            cudaGetLastError();
+        }
         ap->clu_n_i = (int)((N + C - 1) / C);
         ap->clu_half = (ap->clu_n_i + 1) / 2;
-        if (ap->clu_half > CLU_THREADS) { ap->clu_kernel = nullptr; return 0; }
+        if (ap->clu_half > CLU_THREADS) { ap->clu_kernel = ap->clu_kernel_vir = nullptr; return 0; }
         int S = 32;                                        // lanes per particle pair (one warp at most)
         while (S > 1 && ap->clu_half * S > CLU_THREADS) S >>= 1;
         while (S > 1 && (long long)S > N) S >>= 1;
@@ -1119,7 +1185,7 @@ int ap_create(ljmd_handle* h) {
     ap->i_lo = h->rank * ap->Nloc;
     ap->nI  = (ap->Nloc + BI - 1) / BI;             // i-blocks of THIS rank's slab
     ap->NJu = (int)((N + J_UNIT - 1) / J_UNIT);
-    ap->kernel = pick_kernel(ap->ipt, h->pc.cutoff != 0);
+    ap->kernel = pick_kernel<false>(ap->ipt, h->pc.cutoff != 0);
     if (!getenv("LJMD_AP_IPT")) clu_setup(h, ap);      // (forcing a grid-kernel variant disables the cluster path)
 
     int per_sm = 0;
@@ -1128,6 +1194,12 @@ int ap_create(ljmd_handle* h) {
     if (const char* e = getenv("LJMD_AP_CTAS_PER_SM")) want = std::max(1, atoi(e));
     per_sm = std::min(per_sm, want);
     if (per_sm < 1) { set_error("all-pairs kernel does not fit on an SM"); return LJMD_E_STATE; }
+    {   // the virial variant must be co-resident on the same grid (its launch bounds make it so)
+        ApKernel kv = pick_kernel<true>(ap->ipt, h->pc.cutoff != 0);
+        int per_sm_vir = 0;
+        LJ_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm_vir, kv, AP_THREADS, 0));
+        if (per_sm_vir >= per_sm) ap->kernel_vir = kv;
+    }
     const long long W = (long long)ap->nI * ap->NJu;
     // at least ~64 j per thread per CTA so tiny systems do not pay for a wide barrier
     long long g_work = std::max<long long>(1, W / (64 / J_UNIT));
@@ -1283,7 +1355,7 @@ void ap_destroy(ljmd_handle* h) {
     if (!ap) return;
     cudaFree(ap->d_cta_start); cudaFree(ap->d_cta_ib0); cudaFree(ap->d_iblk);
     cudaFree(ap->shared); cudaFree(ap->Vh); cudaFree(ap->Ftmp);
-    cudaFree(ap->part); cudaFree(ap->pe_part); cudaFree(ap->ke_part);
+    cudaFree(ap->part); cudaFree(ap->pe_part); cudaFree(ap->ke_part); cudaFree(ap->vir_part);
     cudaFree(ap->d_patches); cudaFree(ap->d_blk_off); cudaFree(ap->d_blk_ent); cudaFree(ap->rowpart); cudaFree(ap->colpart);
     cudaFree(ap->sched);
     cudaFree(ap->bar); cudaFree(ap->err);
@@ -1292,10 +1364,18 @@ void ap_destroy(ljmd_handle* h) {
 }
 
 int ap_run(ljmd_handle* h, const float2* R_in, const float2* V_in, float2* R_out, float2* V_out,
-           float2* F_out, float* pe_out, const RunCtl& rc) {
+           float2* F_out, float* pe_out, const RunCtl& rc, float* vir_out) {
     AllPairs* ap = h->ap;
     const long long N = h->p.N;
     cudaStream_t st = h->stream;
+    const bool vir = vir_out != nullptr;
+    if (vir && (ap->clu_kernel ? ap->clu_kernel_vir == nullptr : ap->kernel_vir == nullptr)) {
+        set_error("the all-pairs virial kernel does not fit the launch configuration of this handle");
+        return LJMD_E_UNSUPPORTED;
+    }
+    // allocated on first use: a process that never asks for the virial places every buffer (the grid-barrier
+    // word among them, whose L2 home shows in the barrier-bound step time) where it was before the virial existed
+    if (vir && !ap->vir_part) LJ_CUDA(cudaMalloc(&ap->vir_part, sizeof(float) * 2 * ap->npe));
     if (rc.nsteps > 0) {
         LJ_CUDA(cudaMemcpyAsync(ap->Vh, V_in, sizeof(float2) * N, cudaMemcpyDeviceToDevice, st));
         if (rc.traj && rc.S > 0)
@@ -1320,6 +1400,7 @@ int ap_run(ljmd_handle* h, const float2* R_in, const float2* V_in, float2* R_out
     a.bar = ap->bar; a.err = ap->err; a.prof = ap->prof;
     a.rc = rc;
     a.R_out = R_out; a.V_out = V_out; a.F_out = F_out; a.pe_out = pe_out;
+    a.vir_part = ap->vir_part; a.vir_out = vir_out;
 
     // bound the duration of a single launch (~0.5 s at a conservative 2e11 pairs/s)
     const double est_step_s = (double)N * (double)N / 2.0e11 + 3.0e-6;
@@ -1337,8 +1418,10 @@ int ap_run(ljmd_handle* h, const float2* R_in, const float2* V_in, float2* R_out
         c.R_in = R_in; c.Rbuf0 = ap->Rbuf0; c.Rbuf1 = ap->Rbuf1; c.Vh = ap->Vh;
         c.rc = rc; c.R_out = R_out; c.V_out = V_out; c.F_out = F_out; c.pe_out = pe_out;
         c.prof = ap->prof;
+        c.vir_out = vir_out;
         cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3(ap->cluC); cfg.blockDim = dim3(CLU_THREADS); cfg.dynamicSmemBytes = ap->clu_smem; cfg.stream = st;
+        cfg.gridDim = dim3(ap->cluC); cfg.blockDim = dim3(CLU_THREADS); cfg.stream = st;
+        cfg.dynamicSmemBytes = vir ? ap->clu_smem_vir : ap->clu_smem;
         cudaLaunchAttribute at[1];
         at[0].id = cudaLaunchAttributeClusterDimension;
         at[0].val.clusterDim.x = ap->cluC; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
@@ -1346,7 +1429,7 @@ int ap_run(ljmd_handle* h, const float2* R_in, const float2* V_in, float2* R_out
         while (s < s_last) {
             const long long e = std::min(s_last, s + chunk);
             c.s_begin = s; c.s_end = e;
-            LJ_CUDA(cudaLaunchKernelEx(&cfg, ap->clu_kernel, c));
+            LJ_CUDA(cudaLaunchKernelEx(&cfg, vir ? ap->clu_kernel_vir : ap->clu_kernel, c));
             h->launches++;
             s = e;
         }
@@ -1377,7 +1460,8 @@ int ap_run(ljmd_handle* h, const float2* R_in, const float2* V_in, float2* R_out
         LJ_CUDA(cudaMemsetAsync(ap->bar, 0, sizeof(unsigned), st));
         LJ_CUDA(cudaMemsetAsync(ap->sched, 0, sizeof(int) * 2, st));
         void* args[] = {(void*)&a};
-        LJ_CUDA(cudaLaunchCooperativeKernel((void*)ap->kernel, dim3(ap->G), dim3(AP_THREADS), args, 0, st));
+        LJ_CUDA(cudaLaunchCooperativeKernel((void*)(vir ? ap->kernel_vir : ap->kernel), dim3(ap->G), dim3(AP_THREADS),
+                                            args, 0, st));
         h->launches++;
         ap->xepoch += (unsigned)(e - s) * ((ap->ipt == 3 && a.P > 1) ? 2u : 1u);   // cross-GPU epochs per step
         s = e;

@@ -122,15 +122,15 @@ void ljmd_destroy(ljmd_t* h) {
 }
 
 static int run_dispatch(ljmd_t* h, const float* R_in, const float* V_in, float* R_out, float* V_out,
-                        float* F_out, float* pe_out, const RunCtl& rc) {
+                        float* F_out, float* pe_out, const RunCtl& rc, float* w_out = nullptr) {
     LJ_CUDA(cudaSetDevice(h->p.device));
     const float2* R = reinterpret_cast<const float2*>(R_in);
     const float2* V = reinterpret_cast<const float2*>(V_in);
     if (h->path == LJMD_PATH_ALLPAIRS)
         return ap_run(h, R, V, reinterpret_cast<float2*>(R_out), reinterpret_cast<float2*>(V_out),
-                      reinterpret_cast<float2*>(F_out), pe_out, rc);
+                      reinterpret_cast<float2*>(F_out), pe_out, rc, w_out);
     return cells_run(h, R, V, reinterpret_cast<float2*>(R_out), reinterpret_cast<float2*>(V_out),
-                     reinterpret_cast<float2*>(F_out), pe_out, rc);
+                     reinterpret_cast<float2*>(F_out), pe_out, rc, w_out);
 }
 
 int ljmd_energy(ljmd_t* h, const float* R, float* pe_dev) {
@@ -145,14 +145,33 @@ int ljmd_forces(ljmd_t* h, const float* R, float* F, float* pe_dev) {
     return run_dispatch(h, R, nullptr, nullptr, nullptr, F, pe_dev, rc);
 }
 
+int ljmd_virial(ljmd_t* h, const float* R, float* w_dev) {
+    if (!h || !R || !w_dev) { set_error("null argument"); return LJMD_E_INVALID; }
+    if (h->nranks > 1) { set_error("ljmd_virial: single-GPU handles only"); return LJMD_E_UNSUPPORTED; }
+    RunCtl rc{};
+    return run_dispatch(h, R, nullptr, nullptr, nullptr, nullptr, nullptr, rc, w_dev);
+}
+
 int ljmd_run(ljmd_t* h, const float* R_in, const float* V_in, float* R_out, float* V_out,
              int64_t nsteps, int64_t sample_every, float* traj, int64_t energy_every, float* ke_pe,
              float thermostat_kT, int64_t thermostat_every) {
+    return ljmd_run_virial(h, R_in, V_in, R_out, V_out, nsteps, sample_every, traj, energy_every, ke_pe,
+                           thermostat_kT, thermostat_every, nullptr);
+}
+
+int ljmd_run_virial(ljmd_t* h, const float* R_in, const float* V_in, float* R_out, float* V_out,
+                    int64_t nsteps, int64_t sample_every, float* traj, int64_t energy_every, float* ke_pe,
+                    float thermostat_kT, int64_t thermostat_every, float* w) {
     if (!h || !R_in || !V_in || !R_out || !V_out) { set_error("null argument"); return LJMD_E_INVALID; }
     if (nsteps < 0 || sample_every < 0 || energy_every < 0 || thermostat_every < 0) {
         set_error("negative step count");
         return LJMD_E_INVALID;
     }
+    if (w && !(ke_pe && energy_every > 0)) {
+        set_error("ljmd_run_virial: the virial trace w needs ke_pe and energy_every > 0 (it has their rows)");
+        return LJMD_E_INVALID;
+    }
+    if (w && h->nranks > 1) { set_error("ljmd_run_virial: single-GPU handles only"); return LJMD_E_UNSUPPORTED; }
     const size_t bytes = sizeof(float) * 2 * (size_t)h->p.N;
     if (nsteps == 0) {   // fori_loop(0, 0, ...) returns the initial state (MD:82)
         LJ_CUDA(cudaSetDevice(h->p.device));
@@ -170,7 +189,7 @@ int ljmd_run(ljmd_t* h, const float* R_in, const float* V_in, float* R_out, floa
     rc.ke_pe = ke_pe;
     rc.thermo_kT = (thermostat_kT > 0.0f && thermostat_every > 0) ? thermostat_kT : 0.0f;
     rc.thermo_every = rc.thermo_kT > 0.0f ? thermostat_every : 0;
-    return run_dispatch(h, R_in, V_in, R_out, V_out, nullptr, nullptr, rc);
+    return run_dispatch(h, R_in, V_in, R_out, V_out, nullptr, nullptr, rc, w);
 }
 
 int ljmd_run_blocked(ljmd_t* h, const float* R_blk, const float* V_blk, float* R_blk_out, float* V_blk_out,
@@ -191,7 +210,7 @@ int ljmd_run_blocked(ljmd_t* h, const float* R_blk, const float* V_blk, float* R
     const float2* V = reinterpret_cast<const float2*>(V_blk);
     if (h->path != LJMD_PATH_ALLPAIRS)
         return cells_run(h, R, V, reinterpret_cast<float2*>(R_blk_out), reinterpret_cast<float2*>(V_blk_out),
-                         nullptr, nullptr, rc);
+                         nullptr, nullptr, rc, nullptr);
     // all-pairs: the state is at most 1 MiB, so the blocks are simply all-gathered (NCCL over NVLink), the
     // replicated run is used as it is, and the rank's block is sliced out of its result
     const size_t blk = sizeof(float2) * (size_t)(N / h->nranks);
@@ -201,7 +220,7 @@ int ljmd_run_blocked(ljmd_t* h, const float* R_blk, const float* V_blk, float* R
     if (!r) r = dist_allgather_from(h, V, h->blk_full[1], blk);
     if (r) return r;
     rc.blocked = 0;
-    r = ap_run(h, h->blk_full[0], h->blk_full[1], h->blk_full[2], h->blk_full[3], nullptr, nullptr, rc);
+    r = ap_run(h, h->blk_full[0], h->blk_full[1], h->blk_full[2], h->blk_full[3], nullptr, nullptr, rc, nullptr);
     if (r) return r;
     LJ_CUDA(cudaMemcpyAsync(R_blk_out, reinterpret_cast<char*>(h->blk_full[2]) + blk * h->rank, blk, cudaMemcpyDeviceToDevice, h->stream));
     LJ_CUDA(cudaMemcpyAsync(V_blk_out, reinterpret_cast<char*>(h->blk_full[3]) + blk * h->rank, blk, cudaMemcpyDeviceToDevice, h->stream));

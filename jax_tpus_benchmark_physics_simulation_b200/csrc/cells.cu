@@ -159,6 +159,10 @@ struct CellsArgs {
     int     mode;                   // 0 = run, 1 = build + count only
     long long* prof;                // optional [G][12] phase clocks (debug: LJMD_CELLS_PROF=1)
     float   count_r2;
+    // virial kernel: per-unit partial virial like pe_part, and the output: W of R_in when nsteps == 0,
+    // else one float per ke_pe row
+    float*  vir_part;               // [2*nchunks]
+    float*  vir_out;
 };
 
 // one fp32 multiply then truncation (x >= 0); the clamp handles x == box (MD:72 closed range)
@@ -726,9 +730,11 @@ __device__ void cells_rebuild(const CellsArgs& a, Ctx& ctx, int* sscan, float2* 
 // The cutoff is a select on the ALU pipe (FSETP + SEL); `two` masks the second neighbour when the
 // entry had an odd number of neighbours left.  (Measured: folding the cutoff in as a 1.0f / 0.0f mask with
 // one packed multiply saves an instruction but costs two FMA-pipe cycles: 166.4 vs 165.5 us/step.)
-template <bool PE, bool EDGE>
+// VIR: also accumulate the pair virial t * ir6 (t = c12*ir6 - c6, the force's own factor) into vir2.
+template <bool PE, bool EDGE, bool VIR>
 __device__ __forceinline__ void eval_two(const PairConsts& pc, const PairConsts2& c2, float2 nri,
-                                         float2 rj0, float2 rj1, bool two, float2& acc, float2& pe2) {
+                                         float2 rj0, float2 rj1, bool two, float2& acc, float2& pe2,
+                                         float2& vir2) {
     float2 d0 = __fadd2_rn(rj0, nri);
     float2 d1 = __fadd2_rn(rj1, nri);
     if (EDGE) {
@@ -741,19 +747,21 @@ __device__ __forceinline__ void eval_two(const PairConsts& pc, const PairConsts2
     ir2.x = (r20 < pc.rc2) ? ir2.x : 0.0f;
     ir2.y = (two & (r21 < pc.rc2)) ? ir2.y : 0.0f;
     const float2 ir6 = __fmul2_rn(__fmul2_rn(ir2, ir2), ir2);
-    const float2 f = __fmul2_rn(__ffma2_rn(ir6, c2.c12, c2.nc6), __fmul2_rn(ir6, ir2));
+    const float2 t = __ffma2_rn(ir6, c2.c12, c2.nc6);
+    const float2 f = __fmul2_rn(t, __fmul2_rn(ir6, ir2));
     acc = __ffma2_rn(d0, make_float2(f.x, f.x), acc);
     acc = __ffma2_rn(d1, make_float2(f.y, f.y), acc);
     if (PE) pe2 = __ffma2_rn(ir6, __ffma2_rn(ir6, c2.d12, c2.nd6), pe2);
+    if (VIR) vir2 = __ffma2_rn(t, ir6, vir2);
 }
 
 // all neighbours of particle i: the entries are walked as ONE sequence of set bits (a lane that
 // finishes an entry moves on to its next one at once), so a warp runs for the longest LIST, not for
 // the sum of the longest entries.  Every stored entry has a non-empty mask.
 // R = the array the entries index: the staged windows (shared memory) or the global positions
-template <bool PE, bool EDGE>
+template <bool PE, bool EDGE, bool VIR>
 __device__ __forceinline__ void list_force(const CellsArgs& a, const float2* R, int i, int n,
-                                           float2 ri, float& Fx, float& Fy, float& pe) {
+                                           float2 ri, float& Fx, float& Fy, float& pe, float& vir) {
     const PairConsts pc = a.pc;
     const PairConsts2 c2 = make_pair_consts2(pc);
     const uint2* __restrict__ ep = a.ent + i;
@@ -764,7 +772,7 @@ __device__ __forceinline__ void list_force(const CellsArgs& a, const float2* R, 
     if (n > 1) e1 = ep[stride];
     if (n > 2) e2 = ep[2 * stride];
     const float2 nri = make_float2(-ri.x, -ri.y);
-    float2 acc = make_float2(0.0f, 0.0f), pe2 = acc;
+    float2 acc = make_float2(0.0f, 0.0f), pe2 = acc, vir2 = acc;
     unsigned m = e0.y;
     const float2* base = R + e0.x;
     int k = 1;
@@ -781,11 +789,12 @@ __device__ __forceinline__ void list_force(const CellsArgs& a, const float2* R, 
         const bool two = (m != 0u);
         const int b1 = two ? 31 - __clz(m) : b0;
         m &= ~(1u << b1);
-        eval_two<PE, EDGE>(pc, c2, nri, base[b0], base[b1], two, acc, pe2);
+        eval_two<PE, EDGE, VIR>(pc, c2, nri, base[b0], base[b1], two, acc, pe2, vir2);
     }
     Fx = -acc.x;
     Fy = -acc.y;
     if (PE) pe = pe2.x + pe2.y;
+    if (VIR) vir = vir2.x + vir2.y;
 }
 
 // ---- bulk copies (cp.async.bulk = UBLKCP, the 1-D TMA path) completing on an mbarrier ---------------
@@ -831,38 +840,39 @@ __device__ __forceinline__ unsigned lds32(unsigned addr) {
 // staged units: the list is one byte per neighbour (index into the staged windows), four per word,
 // padded with the sentinel index to the warp's longest list (nw words, warp-uniform).  `win` is the
 // 32-bit shared-memory address of the staged windows: byte extract + scaled add + LDS.64 per neighbour.
-template <bool PE>
+template <bool PE, bool VIR>
 __device__ __forceinline__ void word_eval(const PairConsts& pc, const PairConsts2& c2, unsigned win,
-                                          unsigned word, float2 nri, float2& acc, float2& pe2) {
+                                          unsigned word, float2 nri, float2& acc, float2& pe2, float2& vir2) {
     const float2 r0 = lds64(win + (__byte_perm(word, 0u, 0x4440u) << 3));
     const float2 r1 = lds64(win + (__byte_perm(word, 0u, 0x4441u) << 3));
     const float2 r2 = lds64(win + (__byte_perm(word, 0u, 0x4442u) << 3));
     const float2 r3 = lds64(win + (__byte_perm(word, 0u, 0x4443u) << 3));
-    eval_two<PE, false>(pc, c2, nri, r0, r1, true, acc, pe2);
-    eval_two<PE, false>(pc, c2, nri, r2, r3, true, acc, pe2);
+    eval_two<PE, false, VIR>(pc, c2, nri, r0, r1, true, acc, pe2, vir2);
+    eval_two<PE, false, VIR>(pc, c2, nri, r2, r3, true, acc, pe2, vir2);
 }
 
 // all listed neighbours of one particle of a staged unit: the first CL_NWS words of every lane arrived
 // in shared memory with the windows, longer lists continue from global memory
-template <bool PE>
+template <bool PE, bool VIR>
 __device__ __forceinline__ void bytes_force_staged(const CellsArgs& a, unsigned win, unsigned sw, int unit,
-                                                   int nw, float2 ri, float& Fx, float& Fy, float& pe) {
+                                                   int nw, float2 ri, float& Fx, float& Fy, float& pe, float& vir) {
     const PairConsts pc = a.pc;
     const PairConsts2 c2 = make_pair_consts2(pc);
     const int lane = threadIdx.x & 31;
     const float2 nri = make_float2(-ri.x, -ri.y);
-    float2 acc = make_float2(0.0f, 0.0f), pe2 = acc;
+    float2 acc = make_float2(0.0f, 0.0f), pe2 = acc, vir2 = acc;
     const int nws = min(nw, CL_NWS);
     const unsigned swl = sw + lane * 4;
 #pragma unroll CL_WORD_UNROLL
-    for (int w = 0; w < nws; ++w) word_eval<PE>(pc, c2, win, lds32(swl + w * 128), nri, acc, pe2);
+    for (int w = 0; w < nws; ++w) word_eval<PE, VIR>(pc, c2, win, lds32(swl + w * 128), nri, acc, pe2, vir2);
     if (nw > CL_NWS) {
         const unsigned* __restrict__ gw = a.nb4 + (size_t)unit * CL_UNITWORDS + lane;
-        for (int w = CL_NWS; w < nw; ++w) word_eval<PE>(pc, c2, win, gw[w * 32], nri, acc, pe2);
+        for (int w = CL_NWS; w < nw; ++w) word_eval<PE, VIR>(pc, c2, win, gw[w * 32], nri, acc, pe2, vir2);
     }
     Fx = -acc.x;
     Fy = -acc.y;
     if (PE) pe = pe2.x + pe2.y;
+    if (VIR) vir = vir2.x + vir2.y;
 }
 
 // slow path of a buffer wait (try_wait itself sleeps in hardware; this is only reached after its time
@@ -896,7 +906,8 @@ struct WarpPipe {
 // bytes on the buffer's mbarrier) and the copy plan of unit k+2 is on its way to registers.
 // PLAIN = an ordinary step of a run (second kick of the previous step, first kick + drift of this one;
 // no sample, no energies, no thermostat, not the last step): the flag tests are compiled out.
-template <bool PE, bool PLAIN>
+// VIR (with PE): the per-unit virial partials ride along with the energy partials.
+template <bool PE, bool PLAIN, bool VIR>
 __device__ __forceinline__ void warp_pass(const CellsArgs& a, const Ctx& ctx, const StepFlags& fl,
                                           WarpPipe& wp, int& moved) {
     const RunCtl& rc = a.rc;
@@ -1033,7 +1044,7 @@ __device__ __forceinline__ void warp_pass(const CellsArgs& a, const Ctx& ctx, co
         float2 v = make_float2(0.0f, 0.0f), rb = make_float2(0.0f, 0.0f);
         if (live && (PLAIN || rc.nsteps > 0)) { v = V[i]; rb = a.Rb[i]; }
         float2 ri = make_float2(0.0f, 0.0f);
-        float Fx = 0.0f, Fy = 0.0f, pe = 0.0f, ke = 0.0f;
+        float Fx = 0.0f, Fy = 0.0f, pe = 0.0f, ke = 0.0f, vir = 0.0f;
 #if CL_COPY == 1
         cp_async_wait<1>();                               // this unit's copy group has landed
         __syncwarp();
@@ -1062,16 +1073,16 @@ __device__ __forceinline__ void warp_pass(const CellsArgs& a, const Ctx& ctx, co
             }
 #endif
             if (live) ri = lds64(win + (CL_WIN + (i - p.y)) * 8);      // own row window holds the own slot
-            bytes_force_staged<PE>(a, win, wp.base + 2 * CL_WINBYTES + buf * CL_SWBYTES, u,
-                                   (int)(((unsigned)p.w >> 24) & 0x7fu), ri, Fx, Fy, pe);
+            bytes_force_staged<PE, VIR>(a, win, wp.base + 2 * CL_WINBYTES + buf * CL_SWBYTES, u,
+                                        (int)(((unsigned)p.w >> 24) & 0x7fu), ri, Fx, Fy, pe, vir);
         } else {
             unsigned meta = 0u;
             const int ii = live ? i : ctx.own_s;
             if (live) { ri = R[i]; meta = a.meta[i]; }
             const int n = meta & 0xff;
             const bool wedge = __any_sync(0xffffffffu, (meta & 0x100u) != 0u);
-            if (wedge) list_force<PE, true >(a, R, ii, n, ri, Fx, Fy, pe);
-            else       list_force<PE, false>(a, R, ii, n, ri, Fx, Fy, pe);
+            if (wedge) list_force<PE, true,  VIR>(a, R, ii, n, ri, Fx, Fy, pe, vir);
+            else       list_force<PE, false, VIR>(a, R, ii, n, ri, Fx, Fy, pe, vir);
         }
 #if !CL_DEPTH3
         const int unn = fix(__shfl_sync(0xffffffffu, g, 0), k + 2);
@@ -1131,6 +1142,10 @@ __device__ __forceinline__ void warp_pass(const CellsArgs& a, const Ctx& ctx, co
             const float t = warp_sum(live ? pe : 0.0f);       // (idle lanes of a boundary unit evaluate a dummy)
             if (lane == 0) __stcg(&a.pe_part[fl.par * a.nchunks + (u - u_lo)], t);
         }
+        if (VIR) {
+            const float t = warp_sum(live ? vir : 0.0f);
+            if (lane == 0) __stcg(&a.vir_part[fl.par * a.nchunks + (u - u_lo)], t);
+        }
         if (want_ke) {
             const float t = warp_sum(ke);
             if (lane == 0) __stcg(&a.ke_part[fl.par * a.nchunks + (u - u_lo)], t);
@@ -1145,6 +1160,8 @@ __device__ __forceinline__ void warp_pass(const CellsArgs& a, const Ctx& ctx, co
 
 extern __shared__ __align__(16) unsigned char cells_smem[];
 
+// VIR: the energy steps also accumulate the pair virial (own instantiation, launched only on request)
+template <bool VIR>
 __global__ void __launch_bounds__(CL_THREADS, 1024 / CL_THREADS)
 cells_persistent_kernel(const CellsArgs a) {
     __shared__ int    sscan[CL_THREADS / 32 + 1];
@@ -1251,7 +1268,8 @@ cells_persistent_kernel(const CellsArgs a) {
         const bool kick1   = (s >= 0);
         const bool final   = (s == rc.nsteps - 1);
         const bool want_e  = kick1 && rc.energy_every > 0 && (s % rc.energy_every == 0);
-        const bool want_pe = want_e || (rc.nsteps == 0 && a.pe_out != nullptr);
+        bool       want_pe = want_e || (rc.nsteps == 0 && a.pe_out != nullptr);
+        if constexpr (VIR) want_pe = want_pe || (rc.nsteps == 0 && a.vir_out != nullptr);   // ljmd_virial
         const bool thermo  = kick1 && rc.thermo_every > 0 && rc.thermo_kT > 0.0f &&
                              ((s + 1) % rc.thermo_every == 0);
         const bool sample  = kick1 && rc.sample_every > 0 && (s % rc.sample_every == 0) &&
@@ -1273,11 +1291,11 @@ cells_persistent_kernel(const CellsArgs a) {
         for (int k = gtid; k < CL_QMAX; k += gsz) __stcg(&a.sched[(par ^ 1) * CL_QMAX + k], 0);   // the other parity's unit counters: idle this step
         int moved = 0;
         if (want_pe)
-            warp_pass<true, false>(a, ctx, fl, wp, moved);
+            warp_pass<true, false, VIR>(a, ctx, fl, wp, moved);
         else if (kick1 && !final && !thermo && !sample && !want_ke)
-            warp_pass<false, true>(a, ctx, fl, wp, moved);
+            warp_pass<false, true, false>(a, ctx, fl, wp, moved);
         else
-            warp_pass<false, false>(a, ctx, fl, wp, moved);
+            warp_pass<false, false, false>(a, ctx, fl, wp, moved);
         if (thermo) {
             CL_BARRIER();
             const double ke2 = block_sum_array(a.ke_part + par * a.nchunks, u_hi - u_lo, sdbl);
@@ -1336,15 +1354,18 @@ cells_persistent_kernel(const CellsArgs a) {
 
         if (blockIdx.x == 0 && want_pe) {
             const double pe2 = block_sum_array(a.pe_part + par * a.nchunks, u_hi - u_lo, sdbl);
-            double ke2 = 0.0;
+            double ke2 = 0.0, w2 = 0.0;
             if (want_e) ke2 = block_sum_array(a.ke_part + par * a.nchunks, u_hi - u_lo, sdbl);
+            if (VIR) w2 = block_sum_array(a.vir_part + par * a.nchunks, u_hi - u_lo, sdbl);
             if (tid == 0) {
                 if (want_e) {
                     float* o = rc.ke_pe + 2 * (s / rc.energy_every);
                     o[0] = (float)(0.5 * ke2);
                     o[1] = (float)(0.5 * pe2);
+                    if (VIR) a.vir_out[s / rc.energy_every] = (float)(0.5 * w2);
                 } else {
-                    a.pe_out[0] = (float)(0.5 * pe2);
+                    if (!VIR || a.pe_out) a.pe_out[0] = (float)(0.5 * pe2);
+                    if (VIR) a.vir_out[0] = (float)(0.5 * w2);
                 }
             }
         }
@@ -1391,7 +1412,8 @@ struct Cells {
     uint2* ent = nullptr;
     unsigned* nb4 = nullptr;
     int4* wplan = nullptr;
-    float *pe_part = nullptr, *ke_part = nullptr;
+    float *pe_part = nullptr, *ke_part = nullptr, *vir_part = nullptr;
+    bool vir_fits = false;          // the virial kernel is co-resident on the grid G of the force kernel
     int* state = nullptr;
     int* sched = nullptr;
     unsigned* bar = nullptr;
@@ -1450,14 +1472,17 @@ int cells_create(ljmd_handle* h) {
     cl->nchunks = cl->Nalloc / 32 + 2;              // capacity in 32-slot units (energy partials)
 
     const size_t smem = (size_t)CL_WARPS * CL_WARP_SMEM;
-    LJ_CUDA(cudaFuncSetAttribute(cells_persistent_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int per_sm = 0;
-    LJ_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, cells_persistent_kernel, CL_THREADS, smem));
+    LJ_CUDA(cudaFuncSetAttribute(cells_persistent_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    LJ_CUDA(cudaFuncSetAttribute(cells_persistent_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    int per_sm = 0, per_sm_vir = 0;
+    LJ_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, cells_persistent_kernel<false>, CL_THREADS, smem));
+    LJ_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm_vir, cells_persistent_kernel<true>, CL_THREADS, smem));
     if (per_sm < 1) { set_error("cell-list kernel does not fit on an SM"); return LJMD_E_STATE; }
     if (const char* e = getenv("LJMD_CELLS_CTAS_PER_SM")) per_sm = std::min(per_sm, std::max(1, atoi(e)));
     long long gg = (long long)per_sm * h->num_sms;
     gg = std::min<long long>(gg, std::max<long long>(1, (N / P + CL_THREADS - 1) / CL_THREADS));
     cl->G = (int)gg;
+    cl->vir_fits = (long long)per_sm_vir * h->num_sms >= gg;
 
     const size_t na = (size_t)cl->Nalloc;
     {   // the shared allocation
@@ -1514,7 +1539,7 @@ void cells_destroy(ljmd_handle* h) {
     cudaFree(cl->tmpk); cudaFree(cl->tmpo); cudaFree(cl->tmpc); cudaFree(cl->meta);
     cudaFree(cl->ent); cudaFree(cl->wplan); cudaFree(cl->nb4);
     cudaFree(cl->cell_start); cudaFree(cl->row_tot);
-    cudaFree(cl->pe_part); cudaFree(cl->ke_part);
+    cudaFree(cl->pe_part); cudaFree(cl->ke_part); cudaFree(cl->vir_part);
     cudaFree(cl->state); cudaFree(cl->bar); cudaFree(cl->prof); cudaFree(cl->sched);
     delete cl;
     h->cells = nullptr;
@@ -1564,15 +1589,21 @@ static int launch(ljmd_handle* h, CellsArgs& a) {
     LJ_CUDA(cudaMemsetAsync(cl->bar, 0, sizeof(unsigned), h->stream));
     LJ_CUDA(cudaMemsetAsync(cl->sched, 0, sizeof(int) * (3 * CL_QMAX + 1), h->stream));
     void* args[] = {(void*)&a};
-    LJ_CUDA(cudaLaunchCooperativeKernel((void*)cells_persistent_kernel, dim3(cl->G), dim3(CL_THREADS),
-                                        args, (size_t)CL_WARPS * CL_WARP_SMEM, h->stream));
+    void* kern = a.vir_out ? (void*)cells_persistent_kernel<true> : (void*)cells_persistent_kernel<false>;
+    LJ_CUDA(cudaLaunchCooperativeKernel(kern, dim3(cl->G), dim3(CL_THREADS), args, (size_t)CL_WARPS * CL_WARP_SMEM,
+                                        h->stream));
     h->launches++;
     return 0;
 }
 
 int cells_run(ljmd_handle* h, const float2* R_in, const float2* V_in, float2* R_out, float2* V_out,
-              float2* F_out, float* pe_out, const RunCtl& rc) {
+              float2* F_out, float* pe_out, const RunCtl& rc, float* vir_out) {
     Cells* cl = h->cells;
+    if (vir_out && (cl->P > 1 || !cl->vir_fits)) {
+        set_error("the cell-list virial is single-GPU only and needs its kernel to fit this handle's grid");
+        return LJMD_E_UNSUPPORTED;
+    }
+    if (vir_out && !cl->vir_part) LJ_CUDA(cudaMalloc(&cl->vir_part, sizeof(float) * 2 * cl->nchunks));   // see ap_run
     const long long N = h->p.N;
     const int P = cl->P;
     cudaStream_t st = h->stream;
@@ -1619,6 +1650,7 @@ int cells_run(ljmd_handle* h, const float2* R_in, const float2* V_in, float2* R_
     a.R_in = R_in; a.V_in = V_in;
     a.rc = rc;
     a.R_out = R_out; a.V_out = V_out; a.F_out = F_out; a.pe_out = pe_out;
+    a.vir_part = cl->vir_part; a.vir_out = vir_out;
     a.blk = blocked ? (int)(N / P) : 0;
     a.mode = 0;
     // bound one launch to roughly half a second (conservative 2e10 particle-steps/s)

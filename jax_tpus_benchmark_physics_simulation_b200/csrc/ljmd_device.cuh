@@ -33,9 +33,12 @@ __device__ __forceinline__ float min_image(float d, float box, float timg) {
 //   {r2 < rc2} is decided on the same fp32 r2 as the CPU restatement;
 //   ir2 = 1/r2 (MUFU.RCP); force scalar and pair energy in the sigma/epsilon-folded form.
 // KEEPTEST: an additional "j is not i" predicate is applied (diagonal mask MD:54-55,60).
-template <bool CUTOFF, bool PE, bool KEEPTEST>
+// VIR: also accumulate the pair virial r.f = t * ir6 (t = c12*ir6 - c6, the force's own factor)
+// into vir, with the same pair set and ir2 as the force (see ljmd_virial in include/ljmd.h).
+template <bool CUTOFF, bool PE, bool KEEPTEST, bool VIR>
 __device__ __forceinline__ void pair_accum(float xi, float yi, float xj, float yj, bool keep,
-                                           const PairConsts& c, float& fx, float& fy, float& pe) {
+                                           const PairConsts& c, float& fx, float& fy, float& pe,
+                                           float& vir) {
     float dx = min_image(__fsub_rn(xi, xj), c.box, c.timg);
     float dy = min_image(__fsub_rn(yi, yj), c.box, c.timg);
     float r2 = __fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy));
@@ -47,10 +50,12 @@ __device__ __forceinline__ void pair_accum(float xi, float yi, float xj, float y
         ir2 = keep ? ir2 : 0.0f;
     }
     float ir6 = ir2 * ir2 * ir2;
-    float f = fmaf(ir6, c.c12, -c.c6) * (ir6 * ir2);
+    const float t = fmaf(ir6, c.c12, -c.c6);
+    float f = t * (ir6 * ir2);
     fx = fmaf(f, dx, fx);
     fy = fmaf(f, dy, fy);
     if (PE) pe = fmaf(ir6, fmaf(ir6, c.d12, -c.d6), pe);
+    if (VIR) vir = fmaf(t, ir6, vir);
 }
 
 // Two ordered pairs at once, (i0 <- j) and (i1 <- j), on Blackwell's packed-FP32 pipe
@@ -88,11 +93,11 @@ __device__ __forceinline__ float2 pack_pinned(float lo, float hi) {
     return *reinterpret_cast<float2*>(&r);
 }
 
-template <bool CUTOFF, bool PE, bool KEEPTEST>
+template <bool CUTOFF, bool PE, bool KEEPTEST, bool VIR>
 __device__ __forceinline__ void pair2_accum(float2 xi2, float2 yi2, float2 nxj2, float2 nyj2,
                                             bool keep0, bool keep1, const PairConsts& c,
                                             const PairConsts2& c2, float2& fx2, float2& fy2,
-                                            float2& pe2) {
+                                            float2& pe2, float2& vir2) {
     float2 dx = __fadd2_rn(xi2, nxj2);
     float2 dy = __fadd2_rn(yi2, nyj2);
     dx.x = min_image(dx.x, c.box, c.timg);
@@ -113,19 +118,22 @@ __device__ __forceinline__ void pair2_accum(float2 xi2, float2 yi2, float2 nxj2,
         ir2.y = keep1 ? ir2.y : 0.0f;
     }
     const float2 ir6 = __fmul2_rn(__fmul2_rn(ir2, ir2), ir2);
-    const float2 f = __fmul2_rn(__ffma2_rn(ir6, c2.c12, c2.nc6), __fmul2_rn(ir6, ir2));
+    const float2 t = __ffma2_rn(ir6, c2.c12, c2.nc6);
+    const float2 f = __fmul2_rn(t, __fmul2_rn(ir6, ir2));
     fx2 = __ffma2_rn(f, dx, fx2);
     fy2 = __ffma2_rn(f, dy, fy2);
     if (PE) pe2 = __ffma2_rn(ir6, __ffma2_rn(ir6, c2.d12, c2.nd6), pe2);
+    if (VIR) vir2 = __ffma2_rn(t, ir6, vir2);
 }
 
 // Packed evaluation of the two pairs (i0 <- j), (i1 <- j) against ONE j (broadcast): returns the
 // force scalars f2 and the displacements so that the caller can apply the term to BOTH sides
 // (Newton's third law: f_ji = -f_ij bit for bit, because the min-image and r2 are symmetric).
-template <bool CUTOFF, bool PE, bool KEEPTEST>
+template <bool CUTOFF, bool PE, bool KEEPTEST, bool VIR>
 __device__ __forceinline__ void pair2_eval(float2 xi2, float2 yi2, float xj, float yj, bool keep0,
                                            bool keep1, const PairConsts& c, const PairConsts2& c2,
-                                           float2& f, float2& dx, float2& dy, float2& pe2) {
+                                           float2& f, float2& dx, float2& dy, float2& pe2,
+                                           float2& vir2) {
     dx = __fadd2_rn(xi2, make_float2(-xj, -xj));
     dy = __fadd2_rn(yi2, make_float2(-yj, -yj));
     dx.x = min_image(dx.x, c.box, c.timg);
@@ -144,8 +152,10 @@ __device__ __forceinline__ void pair2_eval(float2 xi2, float2 yi2, float xj, flo
         ir2.y = keep1 ? ir2.y : 0.0f;
     }
     const float2 ir6 = __fmul2_rn(__fmul2_rn(ir2, ir2), ir2);
-    f = __fmul2_rn(__ffma2_rn(ir6, c2.c12, c2.nc6), __fmul2_rn(ir6, ir2));
+    const float2 t = __ffma2_rn(ir6, c2.c12, c2.nc6);
+    f = __fmul2_rn(t, __fmul2_rn(ir6, ir2));
     if (PE) pe2 = __ffma2_rn(ir6, __ffma2_rn(ir6, c2.d12, c2.nd6), pe2);
+    if (VIR) vir2 = __ffma2_rn(t, ir6, vir2);
 }
 
 // jnp.mod(x, box) of MD:72 (result has the divisor's sign; can return exactly `box` for tiny

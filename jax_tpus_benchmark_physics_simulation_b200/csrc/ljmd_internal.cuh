@@ -88,9 +88,11 @@ namespace ljmd {
 // allpairs.cu
 int  ap_create(ljmd_handle* h);
 void ap_destroy(ljmd_handle* h);
-// nsteps == 0: evaluate F (optional) and PE (optional) of R_in only.
+// nsteps == 0: evaluate F (optional), PE (optional) and the virial W (optional) of R_in only.
+// vir_out != nullptr selects the virial kernels: W of R_in (nsteps == 0), else vir_out[i / energy_every]
+// = W of the post-step state on every row that ke_pe receives (single GPU only).
 int  ap_run(ljmd_handle* h, const float2* R_in, const float2* V_in, float2* R_out, float2* V_out,
-            float2* F_out, float* pe_out, const RunCtl& rc);
+            float2* F_out, float* pe_out, const RunCtl& rc, float* vir_out);
 int  ap_check_error(ljmd_handle* h);
 int  ap_mode(ljmd_handle* h);
 int  ap_gr_hist(ljmd_handle* h, const float2* R_hist, long long S, int nbins, const float* edges,
@@ -100,7 +102,7 @@ int  ap_gr_hist(ljmd_handle* h, const float2* R_hist, long long S, int nbins, co
 int  cells_create(ljmd_handle* h);
 void cells_destroy(ljmd_handle* h);
 int  cells_run(ljmd_handle* h, const float2* R_in, const float2* V_in, float2* R_out,
-               float2* V_out, float2* F_out, float* pe_out, const RunCtl& rc);
+               float2* V_out, float2* F_out, float* pe_out, const RunCtl& rc, float* vir_out);   // as ap_run
 int  cells_geometry(ljmd_handle* h, int* nrows, int* nbx, int* kbins, float* inv_hy, float* inv_wx);
 int  cells_assign(ljmd_handle* h, const float2* R, int* cell_id, int* cell_count);
 int  cells_neighbor_count(ljmd_handle* h, const float2* R, float radius, int* nbr_count);

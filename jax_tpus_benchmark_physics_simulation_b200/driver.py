@@ -8,7 +8,8 @@ reference's behaviour): ``--rc`` (cutoff, default none), ``--path`` (auto|allpai
 ``--ic`` (uniform|lattice; ``uniform`` = the reference's own placement, MD:133-135, and therefore
 the default: like the reference's run it overflows fp32 within a few steps - SURVEY.md §0 - and
 finishes with non-finite positions; ``lattice`` is the physical lattice+jitter state that the
-parity tests and bench.py use), ``--energy_every``.  matplotlib is imported
+parity tests and bench.py use), ``--energy_every``, ``--pressure`` (records the pair virial on the
+energy rows and reports the mean and spread of P over the production).  matplotlib is imported
 lazily (absent in this image): without it g(r) is written as ``.npy``/``.csv`` next to
 ``--output``.
 """
@@ -28,7 +29,7 @@ def main(args):
     N, rho, kT, dt = args.N, args.rho, args.kT, args.dt
     sim = LJSimulation(N, rho=rho, dt=dt, eq_steps=args.eq_steps, prod_steps=args.prod_steps,
                        sample_every=args.sample_every, rc=args.rc, path=args.path,
-                       energy_every=args.energy_every)
+                       energy_every=args.energy_every, virial=args.pressure)
     box_size = sim.box_size                                                    # MD:30
     print(f"Molecular Dynamics Simulation (B200 native)\n"
           f"Particles (N): {N}\nDensity (rho): {rho:.2f}\nTemperature (kT): {kT:.1f}\n"
@@ -75,6 +76,9 @@ def main(args):
     if sim.last_energies is not None:
         e = sim.last_energies.numpy()
         print(f"  Energy (KE+PE) first/last sample: {e[0].sum():.4f} / {e[-1].sum():.4f}")
+    if sim.last_pressure is not None:
+        P = sim.last_pressure.numpy()
+        print(f"  Pressure (production): mean {P.mean():.4f}  std {P.std():.4f}  over {P.size} samples")
 
     r_np, g_np = np.asarray(r_bins_g), np.asarray(g_r)
     try:
@@ -116,8 +120,19 @@ def build_parser():
                         help="initial positions: uniform = the reference's (MD:133-135, default); "
                              "lattice = square lattice + 5%% jitter (physical)")
     parser.add_argument("--energy_every", type=int, default=0)
+    parser.add_argument("--pressure", action="store_true",
+                        help="record the pair virial on the energy rows and report the pressure "
+                             "(needs --energy_every > 0)")
     return parser
 
 
+def parse_args(argv=None):
+    parser = build_parser()
+    args = parser.parse_args(argv)
+    if args.pressure and args.energy_every <= 0:
+        parser.error("--pressure needs --energy_every > 0")
+    return args
+
+
 if __name__ == "__main__":
-    main(build_parser().parse_args())
+    main(parse_args())

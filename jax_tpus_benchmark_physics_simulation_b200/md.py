@@ -83,7 +83,10 @@ class LJSimulation:
 
     Parameters mirror the reference's CLI / closure captures (MD:16-31,196-213).  ``rc=None``
     reproduces the reference (no cutoff).  ``thermostat_kT`` / ``energy_every`` are additions
-    that default to the reference's behaviour (pure NVE, no energy output).
+    that default to the reference's behaviour (pure NVE, no energy output).  ``virial=True``
+    (also an addition, off by default) makes ``equilibrate_fn`` / ``production_fn`` record the pair
+    virial W on the energy rows: ``last_virial`` (ne,) and ``last_pressure`` (ne,) next to
+    ``last_energies`` (ne, 2); ``run(..., virial=...)`` overrides it per call.
     """
 
     def __init__(self, N: int, rho: float = 0.8, dt: float = 1e-3, eq_steps: int = 10000,
@@ -92,7 +95,7 @@ class LJSimulation:
                  skin: float = 0.3, device: Optional[int] = None,
                  box_size: Optional[float] = None, thermostat_kT: float = 0.0,
                  thermostat_every: int = 0, energy_every: int = 0,
-                 dist: Optional[Tuple[bytes, int, int]] = None):
+                 dist: Optional[Tuple[bytes, int, int]] = None, virial: bool = False):
         if not torch.cuda.is_available():
             raise _lib.LjmdError("no CUDA device: the LJ-MD hot path has no CPU fallback")
         self.lib = _lib.load()
@@ -108,9 +111,12 @@ class LJSimulation:
         self.thermostat_kT = float(thermostat_kT)
         self.thermostat_every = int(thermostat_every)
         self.energy_every = int(energy_every)
+        self.virial = bool(virial)
         self.device_index = torch.cuda.current_device() if device is None else int(device)
         self.device = torch.device("cuda", self.device_index)
         self.last_energies: Optional[DeviceArray] = None
+        self.last_virial: Optional[DeviceArray] = None
+        self.last_pressure: Optional[DeviceArray] = None
         p = _lib.LjmdParams()
         p.N = self.N
         p.box = float(self.box_size)
@@ -218,8 +224,34 @@ class LJSimulation:
         self._after()
         return self._arr(F), self._arr(pe[0])
 
+    # ------------------------------------------------------------------ virial / pressure (new)
+    def virial_fn(self, R) -> DeviceArray:
+        """Pair virial W(R) = sum_{i<j, r < rc} r_ij . f_ij as a device scalar (ljmd_virial): the
+        same pair set, minimum image and fp32 arithmetic as the force; no tail correction."""
+        R = self._dev(R, (self.N, 2))
+        out = torch.empty(1, dtype=torch.float32, device=self.device)
+        self._check_stream()
+        _lib.check(self.lib.ljmd_virial(self._h, R.data_ptr(), out.data_ptr()), "ljmd_virial")
+        self._after()
+        return self._arr(out[0])
+
+    def _pressure(self, ke: torch.Tensor, w: torch.Tensor) -> torch.Tensor:
+        """P = (KE + W/2) / box^2 of the 2-D fluid (unit mass, k_B = 1), in float64."""
+        box = float(self.box_size)
+        return (ke.to(torch.float64) + 0.5 * w.to(torch.float64)) / (box * box)
+
+    def pressure_fn(self, state) -> DeviceArray:
+        """Instantaneous pressure (KE(V) + W(R)/2) / box^2 of state = (R, V), a float64 device scalar;
+        KE = 0.5 sum |v|^2 with the centre-of-mass motion included (as the reference's energies)."""
+        R, V = state
+        V = self._dev(V, (self.N, 2))
+        w = self.virial_fn(R).tensor
+        ke = 0.5 * torch.sum(V.to(torch.float64) ** 2)
+        return self._arr(self._pressure(ke, w))
+
     # ------------------------------------------------------------------ MD:66-106
-    def _run(self, state, nsteps: int, sample_every: int = 0, energy_every: int = 0):
+    def _run(self, state, nsteps: int, sample_every: int = 0, energy_every: int = 0,
+             virial: bool = False):
         R, V = state
         R = self._dev(R, (self.N, 2))
         V = self._dev(V, (self.N, 2))
@@ -229,23 +261,36 @@ class LJSimulation:
         traj = torch.empty((S, self.N, 2), dtype=torch.float32, device=self.device)
         ne = -(-nsteps // energy_every) if energy_every > 0 else 0
         ke_pe = torch.zeros((ne, 2), dtype=torch.float32, device=self.device) if ne else None
+        w = torch.zeros(ne, dtype=torch.float32, device=self.device) if (virial and ne) else None
         self._check_stream()
-        _lib.check(self.lib.ljmd_run(
-            self._h, R.data_ptr(), V.data_ptr(), R_out.data_ptr(), V_out.data_ptr(), nsteps,
-            sample_every if S > 0 else 0, traj.data_ptr() if S > 0 else None,
-            energy_every if ne else 0, ke_pe.data_ptr() if ne else None,
-            self.thermostat_kT, self.thermostat_every), "ljmd_run")
+        if w is None:
+            _lib.check(self.lib.ljmd_run(
+                self._h, R.data_ptr(), V.data_ptr(), R_out.data_ptr(), V_out.data_ptr(), nsteps,
+                sample_every if S > 0 else 0, traj.data_ptr() if S > 0 else None,
+                energy_every if ne else 0, ke_pe.data_ptr() if ne else None,
+                self.thermostat_kT, self.thermostat_every), "ljmd_run")
+        else:
+            _lib.check(self.lib.ljmd_run_virial(
+                self._h, R.data_ptr(), V.data_ptr(), R_out.data_ptr(), V_out.data_ptr(), nsteps,
+                sample_every if S > 0 else 0, traj.data_ptr() if S > 0 else None,
+                energy_every, ke_pe.data_ptr(), self.thermostat_kT, self.thermostat_every,
+                w.data_ptr()), "ljmd_run_virial")
         self._after()
         self.last_energies = self._arr(ke_pe) if ne else None
+        self.last_virial = self._arr(w) if w is not None else None
+        self.last_pressure = self._arr(self._pressure(ke_pe[:, 0], w)) if w is not None else None
         return (self._arr(R_out), self._arr(V_out)), self._arr(traj)
 
     def verlet_step(self, state):
         """One velocity-Verlet step (MD:66-75)."""
         return self._run(state, 1)[0]
 
-    def run(self, state, nsteps: int, sample_every: int = 0, energy_every: int = 0):
-        """nsteps velocity-Verlet steps in one device dispatch; returns (state, traj)."""
-        return self._run(state, int(nsteps), int(sample_every), int(energy_every))
+    def run(self, state, nsteps: int, sample_every: int = 0, energy_every: int = 0,
+            virial: Optional[bool] = None):
+        """nsteps velocity-Verlet steps in one device dispatch; returns (state, traj).
+        ``virial`` (default: the constructor's) also records W and P on the energy rows."""
+        virial = self.virial if virial is None else bool(virial)
+        return self._run(state, int(nsteps), int(sample_every), int(energy_every), virial)
 
     def block_range(self) -> Tuple[int, int]:
         """Index block [lo, hi) of this rank in the block-distributed convention of run_blocked."""
@@ -272,14 +317,14 @@ class LJSimulation:
 
     def equilibrate_fn(self, initial_state):
         """fori_loop(0, equilibration_steps, verlet_step) — one dispatch, NVE (MD:77-83)."""
-        return self._run(initial_state, self.equilibration_steps, 0, self.energy_every)[0]
+        return self._run(initial_state, self.equilibration_steps, 0, self.energy_every, self.virial)[0]
 
     def production_fn(self, initial_state):
         """production_steps steps, snapshot after step i when i % sample_every == 0 into row
         i // sample_every of R_history (S, N, 2), S = production_steps // sample_every
         (MD:85-106)."""
         return self._run(initial_state, self.production_steps, self.sample_every,
-                         self.energy_every)
+                         self.energy_every, self.virial)
 
     # ------------------------------------------------------------------ MD:108-131
     def calculate_g_r(self, R_history, N_local=None, box_size_local=None, nbins=None, r_max=None):
