@@ -35,20 +35,9 @@ namespace ljmd {
 namespace {
 
 constexpr int AP_THREADS = 128;   // 4 warps: one per SM sub-partition
-#ifndef AP_UNROLL
-#define AP_UNROLL 8
-#endif
-#ifndef AP_MINBLOCKS
-#define AP_MINBLOCKS 4
-#endif
-#ifndef AP_TB_UNROLL
-#define AP_TB_UNROLL 4
-#endif
-constexpr int kTileBothUnroll = AP_TB_UNROLL;
-#ifndef AP_TILE_BOTH
-#define AP_TILE_BOTH 1      // 1 = both halves of a 64 x 64 tile in one rotation loop (tile_both), 0 = one after the other
-#endif
-constexpr int kApUnroll = AP_UNROLL;   // j particles per unrolled inner-loop body
+constexpr int AP_MINBLOCKS = 4;   // CTAs per SM the grid kernel's register budget is sized for
+constexpr int AP_UNROLL  = 8;     // j particles per unrolled inner-loop body (ordered pairs)
+constexpr int AP_TB_UNROLL = 4;   // rotation steps per unrolled body of tile_both
 constexpr int J_UNIT     = 8;     // granularity of the j split (particles)
 constexpr int TILE_J     = 512;   // j particles staged per shared-memory tile (8 KB)
 constexpr int RED_LANES  = 8;     // lanes that cooperate on one particle's partial sum
@@ -152,14 +141,14 @@ __device__ __forceinline__ void ap_segment(const ApArgs& a, const float2* __rest
                 const int qa = (part == 0) ? 0 : (part == 1 ? qd0 : qd1);
                 const int qb = (part == 0) ? qd0 : (part == 1 ? qd1 : cnt);
                 if (part != 1) {
-#pragma unroll kApUnroll
+#pragma unroll AP_UNROLL
                     for (int q = qa; q < qb; ++q) {
                         const float4 v = sj[q];            // one j particle, warp broadcast
                         pair2_accum<CUTOFF, PE, false, VIR>(xi2, yi2, make_float2(v.x, v.y), make_float2(v.z, v.w),
                                                             true, true, pc, pc2, tfx, tfy, tpe, tvir);
                     }
                 } else {
-#pragma unroll kApUnroll
+#pragma unroll AP_UNROLL
                     for (int q = qa; q < qb; ++q) {
                         const float4 v = sj[q];
                         const int j = jt + q;
@@ -178,13 +167,13 @@ __device__ __forceinline__ void ap_segment(const ApArgs& a, const float2* __rest
                 const int qa = (part == 0) ? 0 : (part == 1 ? qd0 : qd1);
                 const int qb = (part == 0) ? qd0 : (part == 1 ? qd1 : cnt);
                 if (part != 1) {
-#pragma unroll kApUnroll
+#pragma unroll AP_UNROLL
                     for (int q = qa; q < qb; ++q) {
                         const float4 v = sj[q];
                         pair_accum<CUTOFF, PE, false, VIR>(xi[0], yi[0], -v.x, -v.z, true, pc, tfx, tfy, tpe, tvir);
                     }
                 } else {
-#pragma unroll kApUnroll
+#pragma unroll AP_UNROLL
                     for (int q = qa; q < qb; ++q) {
                         const float4 v = sj[q];
                         pair_accum<CUTOFF, PE, true, VIR>(xi[0], yi[0], -v.x, -v.z, (jt + q) != ii[0], pc, tfx, tfy, tpe,
@@ -208,54 +197,12 @@ constexpr int T3_BLK = 64;
 
 __device__ __forceinline__ int tri_base(int pa, int npr) { return pa * npr - (pa * (pa - 1)) / 2; }
 
-template <bool CUTOFF, bool PE, bool N3L, bool VIR>
-__device__ __forceinline__ void tile_half(const PairConsts& pc, const PairConsts2& pc2, float2 xi2,
-                                          float2 yi2, float xj, float yj, bool self0, bool self1,
-                                          float2& fx2, float2& fy2, float2& pe2, float2& vir2,
-                                          float& fjx, float& fjy) {
-    const int src = (threadIdx.x + 1) & 31;
-    // the reaction on the travelling j is accumulated as ONE scalar per component (the two i of this
-    // lane are added in a fixed order), so only two values per component... per step two shuffles
-    // move (xj, yj) and two move the accumulators
-    float ajx = 0.0f, ajy = 0.0f;
-    // step 0 peeled: the only step at which j can be one of this lane's own i (diagonal tiles)
-    {
-        float2 f, dx, dy;
-        if (N3L) pair2_eval<CUTOFF, PE, false, VIR>(xi2, yi2, xj, yj, true, true, pc, pc2, f, dx, dy, pe2, vir2);
-        else     pair2_eval<CUTOFF, PE, true,  VIR>(xi2, yi2, xj, yj, !self0, !self1, pc, pc2, f, dx, dy, pe2, vir2);
-        fx2 = __ffma2_rn(f, dx, fx2);
-        fy2 = __ffma2_rn(f, dy, fy2);
-        if (N3L) {
-            ajx = fmaf(f.y, dx.y, __fmul_rn(f.x, dx.x));
-            ajy = fmaf(f.y, dy.y, __fmul_rn(f.x, dy.x));
-        }
-        xj = __shfl_sync(0xffffffffu, xj, src);
-        yj = __shfl_sync(0xffffffffu, yj, src);
-        if (N3L) { ajx = __shfl_sync(0xffffffffu, ajx, src); ajy = __shfl_sync(0xffffffffu, ajy, src); }
-    }
-#pragma unroll 4
-    for (int s = 1; s < 32; ++s) {
-        float2 f, dx, dy;
-        pair2_eval<CUTOFF, PE, false, VIR>(xi2, yi2, xj, yj, true, true, pc, pc2, f, dx, dy, pe2, vir2);
-        fx2 = __ffma2_rn(f, dx, fx2);
-        fy2 = __ffma2_rn(f, dy, fy2);
-        if (N3L) {
-            ajx = fmaf(f.y, dx.y, fmaf(f.x, dx.x, ajx));
-            ajy = fmaf(f.y, dy.y, fmaf(f.x, dy.x, ajy));
-        }
-        xj = __shfl_sync(0xffffffffu, xj, src);
-        yj = __shfl_sync(0xffffffffu, yj, src);
-        if (N3L) { ajx = __shfl_sync(0xffffffffu, ajx, src); ajy = __shfl_sync(0xffffffffu, ajy, src); }
-    }
-    // 32 rotations: the travelling j (and its accumulator) is home again
-    fjx = -ajx;
-    fjy = -ajy;
-}
-
 // Both halves of a 64 x 64 tile in ONE rotation loop: the two travelling j sets (h = 0: lanes' j, h = 1:
 // j + 32) are independent dependency chains (evaluate -> accumulate the reaction -> four shuffles), so
 // interleaving them doubles the instruction-level parallelism of a warp that shares its scheduler with
-// only three others (107 registers: 4 CTAs of 4 warps per SM).  Same arithmetic per pair as tile_half.
+// only three others (107 registers: 4 CTAs of 4 warps per SM).  The reaction on a travelling j is
+// accumulated as ONE scalar per component (the two i of this lane added in a fixed order); after 32
+// rotations the travelling j and its accumulator are home again.
 template <bool CUTOFF, bool PE, bool N3L, bool VIR>
 __device__ __forceinline__ void tile_both(const PairConsts& pc, const PairConsts2& pc2, float2 xi2, float2 yi2,
                                           float xja, float yja, float xjb, float yjb,
@@ -268,11 +215,15 @@ __device__ __forceinline__ void tile_both(const PairConsts& pc, const PairConsts
         // half a meets i0 (self0), half b meets i1 (self1)
         float2 fa, dxa, dya, fb, dxb, dyb;
         if (N3L) {
-            pair2_eval<CUTOFF, PE, false, VIR>(xi2, yi2, xja, yja, true, true, pc, pc2, fa, dxa, dya, pe2, vir2);
-            pair2_eval<CUTOFF, PE, false, VIR>(xi2, yi2, xjb, yjb, true, true, pc, pc2, fb, dxb, dyb, pe2, vir2);
+            pair2_eval<CUTOFF, PE, false, VIR>(xi2, yi2, make_float2(-xja, -xja), make_float2(-yja, -yja),
+                                               true, true, pc, pc2, fa, dxa, dya, pe2, vir2);
+            pair2_eval<CUTOFF, PE, false, VIR>(xi2, yi2, make_float2(-xjb, -xjb), make_float2(-yjb, -yjb),
+                                               true, true, pc, pc2, fb, dxb, dyb, pe2, vir2);
         } else {
-            pair2_eval<CUTOFF, PE, true, VIR>(xi2, yi2, xja, yja, false, true, pc, pc2, fa, dxa, dya, pe2, vir2);
-            pair2_eval<CUTOFF, PE, true, VIR>(xi2, yi2, xjb, yjb, true, false, pc, pc2, fb, dxb, dyb, pe2, vir2);
+            pair2_eval<CUTOFF, PE, true, VIR>(xi2, yi2, make_float2(-xja, -xja), make_float2(-yja, -yja),
+                                              false, true, pc, pc2, fa, dxa, dya, pe2, vir2);
+            pair2_eval<CUTOFF, PE, true, VIR>(xi2, yi2, make_float2(-xjb, -xjb), make_float2(-yjb, -yjb),
+                                              true, false, pc, pc2, fb, dxb, dyb, pe2, vir2);
         }
         fx2 = __ffma2_rn(fa, dxa, fx2); fy2 = __ffma2_rn(fa, dya, fy2);
         gx2 = __ffma2_rn(fb, dxb, gx2); gy2 = __ffma2_rn(fb, dyb, gy2);
@@ -287,11 +238,13 @@ __device__ __forceinline__ void tile_both(const PairConsts& pc, const PairConsts
             abx = __shfl_sync(0xffffffffu, abx, src); aby = __shfl_sync(0xffffffffu, aby, src);
         }
     }
-#pragma unroll kTileBothUnroll
+#pragma unroll AP_TB_UNROLL
     for (int s = 1; s < 32; ++s) {
         float2 fa, dxa, dya, fb, dxb, dyb;
-        pair2_eval<CUTOFF, PE, false, VIR>(xi2, yi2, xja, yja, true, true, pc, pc2, fa, dxa, dya, pe2, vir2);
-        pair2_eval<CUTOFF, PE, false, VIR>(xi2, yi2, xjb, yjb, true, true, pc, pc2, fb, dxb, dyb, pe2, vir2);
+        pair2_eval<CUTOFF, PE, false, VIR>(xi2, yi2, make_float2(-xja, -xja), make_float2(-yja, -yja),
+                                           true, true, pc, pc2, fa, dxa, dya, pe2, vir2);
+        pair2_eval<CUTOFF, PE, false, VIR>(xi2, yi2, make_float2(-xjb, -xjb), make_float2(-yjb, -yjb),
+                                           true, true, pc, pc2, fb, dxb, dyb, pe2, vir2);
         fx2 = __ffma2_rn(fa, dxa, fx2); fy2 = __ffma2_rn(fa, dya, fy2);
         gx2 = __ffma2_rn(fb, dxb, gx2); gy2 = __ffma2_rn(fb, dyb, gy2);
         if (N3L) {
@@ -350,41 +303,22 @@ __device__ __forceinline__ void ap3_phase_forces(const ApArgs& a, const float2* 
                 if (ba > bb) continue;                          // lower triangle (diagonal patches only)
                 float2 pe2 = make_float2(0.0f, 0.0f), vir2 = pe2;
                 float2 tfx = make_float2(0.0f, 0.0f), tfy = tfx;   // per-tile sums (bounded chains)
-#if AP_TILE_BOTH
-                {
-                    const int ja = bb * T3_BLK + lane, jb = ja + 32;
-                    const float2 pa = ld_pos(Rcur, ja, a.N, SENT_J), pb = ld_pos(Rcur, jb, a.N, SENT_J);
-                    float fjxa, fjya, fjxb, fjyb;
-                    if (ba < bb) {
-                        tile_both<CUTOFF, PE, true, VIR>(pc, pc2, xi2, yi2, pa.x, pa.y, pb.x, pb.y, tfx, tfy, pe2, vir2,
-                                                         fjxa, fjya, fjxb, fjyb);
-                        float2 acc = colacc[cc * T3_BLK + lane];
-                        acc.x += fjxa; acc.y += fjya;
-                        colacc[cc * T3_BLK + lane] = acc;
-                        acc = colacc[cc * T3_BLK + 32 + lane];
-                        acc.x += fjxb; acc.y += fjyb;
-                        colacc[cc * T3_BLK + 32 + lane] = acc;
-                    } else {
-                        tile_both<CUTOFF, PE, false, VIR>(pc, pc2, xi2, yi2, pa.x, pa.y, pb.x, pb.y, tfx, tfy, pe2, vir2,
-                                                          fjxa, fjya, fjxb, fjyb);
-                    }
+                const int ja = bb * T3_BLK + lane, jb = ja + 32;
+                const float2 pa = ld_pos(Rcur, ja, a.N, SENT_J), pb = ld_pos(Rcur, jb, a.N, SENT_J);
+                float fjxa, fjya, fjxb, fjyb;
+                if (ba < bb) {
+                    tile_both<CUTOFF, PE, true, VIR>(pc, pc2, xi2, yi2, pa.x, pa.y, pb.x, pb.y, tfx, tfy, pe2, vir2,
+                                                     fjxa, fjya, fjxb, fjyb);
+                    float2 acc = colacc[cc * T3_BLK + lane];
+                    acc.x += fjxa; acc.y += fjya;
+                    colacc[cc * T3_BLK + lane] = acc;
+                    acc = colacc[cc * T3_BLK + 32 + lane];
+                    acc.x += fjxb; acc.y += fjyb;
+                    colacc[cc * T3_BLK + 32 + lane] = acc;
+                } else {
+                    tile_both<CUTOFF, PE, false, VIR>(pc, pc2, xi2, yi2, pa.x, pa.y, pb.x, pb.y, tfx, tfy, pe2, vir2,
+                                                      fjxa, fjya, fjxb, fjyb);
                 }
-#else
-#pragma unroll 1
-                for (int h = 0; h < 2; ++h) {
-                    const int j = bb * T3_BLK + h * 32 + lane;
-                    const float2 pj = ld_pos(Rcur, j, a.N, SENT_J);
-                    float fjx, fjy;
-                    if (ba < bb) {
-                        tile_half<CUTOFF, PE, true, VIR>(pc, pc2, xi2, yi2, pj.x, pj.y, false, false, tfx, tfy, pe2, vir2, fjx, fjy);
-                        float2 acc = colacc[cc * T3_BLK + h * 32 + lane];
-                        acc.x += fjx; acc.y += fjy;
-                        colacc[cc * T3_BLK + h * 32 + lane] = acc;
-                    } else {
-                        tile_half<CUTOFF, PE, false, VIR>(pc, pc2, xi2, yi2, pj.x, pj.y, h == 0, h == 1, tfx, tfy, pe2, vir2, fjx, fjy);
-                    }
-                }
-#endif
                 fx2.x += tfx.x; fx2.y += tfx.y; fy2.x += tfy.x; fy2.y += tfy.y;
                 // energy bookkeeping in the ORDERED-pair convention of the caller (0.5 * sum):
                 // an unordered pair of an off-diagonal tile counts twice, a diagonal tile is ordered
@@ -480,26 +414,17 @@ ap_persistent_kernel(const ApArgs a) {
         // (s = -1: the caller's positions, wrapped into the box by ap_load_kernel, are in Rbuf1)
         const float2* Rcur  = (s & 1) ? a.Rbuf1 : a.Rbuf0;
         float2*       Rnext = ((s + 1) & 1) ? a.Rbuf1 : a.Rbuf0;
-        const int  par     = (int)((s + 1) & 1);
-        const bool kick1   = (s >= 0);                     // prologue only evaluates F(R_in)
-        const bool final   = (s == rc.nsteps - 1);
-        const bool want_e  = kick1 && rc.energy_every > 0 && (s % rc.energy_every == 0);
-        bool       want_pe = want_e || (rc.nsteps == 0 && a.pe_out != nullptr);
-        if constexpr (VIR) want_pe = want_pe || (rc.nsteps == 0 && a.vir_out != nullptr);   // ljmd_virial
-        const bool thermo  = kick1 && rc.thermo_every > 0 && rc.thermo_kT > 0.0f &&
-                             ((s + 1) % rc.thermo_every == 0);
-        const bool sample  = kick1 && rc.sample_every > 0 && (s % rc.sample_every == 0) &&
-                             (s / rc.sample_every < rc.S);   // MD:93-100
+        const StepFlags fl = step_flags<VIR>(rc, s, a.pe_out, a.vir_out);
 
         if (prof) pt[4] = clock64();
         // ---- [b] partial forces of R_cur ------------------------------------------------------
         if constexpr (V3) {
-            if (c == 0 && tid == 0) __stcg(&a.sched[par ^ 1], 0);   // the other parity's patch counter
-            if (want_pe) ap3_phase_forces<CUTOFF, true,  VIR  >(a, Rcur, reinterpret_cast<float2*>(smem_buf), sred, par);
-            else         ap3_phase_forces<CUTOFF, false, false>(a, Rcur, reinterpret_cast<float2*>(smem_buf), sred, par);
+            if (c == 0 && tid == 0) __stcg(&a.sched[fl.par ^ 1], 0);   // the other parity's patch counter
+            if (fl.want_pe) ap3_phase_forces<CUTOFF, true,  VIR  >(a, Rcur, reinterpret_cast<float2*>(smem_buf), sred, fl.par);
+            else            ap3_phase_forces<CUTOFF, false, false>(a, Rcur, reinterpret_cast<float2*>(smem_buf), sred, fl.par);
         } else {
-            if (want_pe) ap_phase_forces<IPT, CUTOFF, true,  VIR  >(a, Rcur, sj, sred, par);
-            else         ap_phase_forces<IPT, CUTOFF, false, false>(a, Rcur, sj, sred, par);
+            if (fl.want_pe) ap_phase_forces<IPT, CUTOFF, true,  VIR  >(a, Rcur, sj, sred, fl.par);
+            else            ap_phase_forces<IPT, CUTOFF, false, false>(a, Rcur, sj, sred, fl.par);
         }
         if (prof) { long long t = clock64(); pt[0] += t - pt[4]; pt[4] = t; }
         grid_barrier(a.bar, (++epoch) * (unsigned)a.G, a.err, a.spin_limit);
@@ -645,15 +570,15 @@ ap_persistent_kernel(const ApArgs a) {
                 Fy += __shfl_xor_sync(0xffffffffu, Fy, o);
             }
             if (!live || gl != 0) continue;
-            if (kick1) { v.x = kick(v.x, Fx, a.dt); v.y = kick(v.y, Fy, a.dt); }   // MD:74
-            if (want_e || thermo) ke_thread += v.x * v.x + v.y * v.y;
-            if (sample) rc.traj[(size_t)(s / rc.sample_every) * a.N + g] = r;
-            if (thermo) {                                   // finish after the KE barrier
+            if (fl.kick1) { v.x = kick(v.x, Fx, a.dt); v.y = kick(v.y, Fy, a.dt); }   // MD:74
+            if (fl.want_e || fl.thermo) ke_thread += v.x * v.x + v.y * v.y;
+            if (fl.sample) rc.traj[(size_t)(s / rc.sample_every) * a.N + g] = r;
+            if (fl.thermo) {                                // finish after the KE barrier
                 a.Vh[g] = v;
                 a.Ftmp[g] = make_float2(Fx, Fy);
                 continue;
             }
-            if (final) {
+            if (fl.final) {
                 if (a.R_out) a.R_out[g] = r;
                 if (a.V_out) a.V_out[g] = v;
                 if (a.F_out) a.F_out[g] = make_float2(Fx, Fy);
@@ -671,19 +596,16 @@ ap_persistent_kernel(const ApArgs a) {
             }
         }
         if (a.P > 1) __threadfence_system();                 // peer stores visible before the arrival
-        if (want_e || thermo) {
+        if (fl.want_e || fl.thermo) {
             float t = block_sum<AP_THREADS>(ke_thread, sred);
-            if (tid == 0) __stcg(&a.ke_part[par * a.G + c], t);
+            if (tid == 0) __stcg(&a.ke_part[fl.par * a.G + c], t);
         }
-        if (thermo) {
-            // velocity rescale: V *= sqrt(kT_target / (KE/N)), KE = 0.5*sum|V|^2 (SURVEY App. A)
+        if (fl.thermo) {
+            // velocity rescale (single-GPU only)
             grid_barrier(a.bar, (++epoch) * (unsigned)a.G, a.err, a.spin_limit);
             if (tid < 32) {
-                double ke2 = warp_sum_array(a.ke_part + par * a.G, a.G);
-                if (tid == 0) {
-                    float ke = (float)(0.5 * ke2);
-                    s_lambda = ke > 0.0f ? sqrtf(rc.thermo_kT / (ke / (float)a.N)) : 1.0f;   // (single-GPU only)
-                }
+                double ke2 = warp_sum_array(a.ke_part + fl.par * a.G, a.G);
+                if (tid == 0) s_lambda = rescale_lambda(ke2, rc.thermo_kT, a.N);
             }
             __syncthreads();
             const float lam = s_lambda;
@@ -693,7 +615,7 @@ ap_persistent_kernel(const ApArgs a) {
                 const float2 F = a.Ftmp[g];
                 float2 v = a.Vh[g];
                 v.x *= lam; v.y *= lam;
-                if (final) {
+                if (fl.final) {
                     if (a.R_out) a.R_out[g] = r;
                     if (a.V_out) a.V_out[g] = v;
                     if (a.F_out) a.F_out[g] = F;
@@ -707,7 +629,7 @@ ap_persistent_kernel(const ApArgs a) {
         }
         if (prof) { long long t = clock64(); pt[2] += t - pt[4]; pt[4] = t; }
         grid_barrier(a.bar, (++epoch) * (unsigned)a.G, a.err, a.spin_limit);
-        if (a.P > 1 && !final) {
+        if (a.P > 1 && !fl.final) {
             // every rank has pushed its slab into our next-position buffer: one NVLink round trip per step,
             // no NCCL on the step path
             peer_wait(xe0 + xper);
@@ -715,21 +637,11 @@ ap_persistent_kernel(const ApArgs a) {
         if (prof) { long long t = clock64(); pt[3] += t - pt[4]; pt[4] = t; }
 
         // ---- energies of the post-step state (one warp, fixed order, double combine) ----------
-        if (c == 0 && tid < 32 && want_pe) {
-            double pe2 = warp_sum_array(a.pe_part + par * a.npe, a.npe);
-            double ke2 = want_e ? warp_sum_array(a.ke_part + par * a.G, a.G) : 0.0;
-            double w2 = VIR ? warp_sum_array(a.vir_part + par * a.npe, a.npe) : 0.0;
-            if (tid == 0) {
-                if (want_e) {
-                    float* o = rc.ke_pe + 2 * (s / rc.energy_every);
-                    o[0] = (float)(0.5 * ke2);
-                    o[1] = (float)(0.5 * pe2);             // MD:61  0.5 * sum over ordered pairs
-                    if (VIR) a.vir_out[s / rc.energy_every] = (float)(0.5 * w2);   // same weights, same 1/2
-                } else {
-                    if (!VIR || a.pe_out) a.pe_out[0] = (float)(0.5 * pe2);
-                    if (VIR) a.vir_out[0] = (float)(0.5 * w2);
-                }
-            }
+        if (c == 0 && tid < 32 && fl.want_pe) {
+            double pe2 = warp_sum_array(a.pe_part + fl.par * a.npe, a.npe);
+            double ke2 = fl.want_e ? warp_sum_array(a.ke_part + fl.par * a.G, a.G) : 0.0;
+            double w2 = VIR ? warp_sum_array(a.vir_part + fl.par * a.npe, a.npe) : 0.0;
+            if (tid == 0) store_energy_row<VIR>(rc, fl, pe2, ke2, w2, a.pe_out, a.vir_out);
         }
     }
     if (prof) {
@@ -874,16 +786,7 @@ ap_cluster_kernel(const CluArgs a) {
     cluster.sync();                       // every CTA of the cluster is resident before remote stores start
 
     for (long long s = a.s_begin; s < a.s_end; ++s) {
-        const int  par     = (int)((s + 1) & 1);
-        const bool kick1   = (s >= 0);
-        const bool final   = (s == rc.nsteps - 1);
-        const bool want_e  = kick1 && rc.energy_every > 0 && (s % rc.energy_every == 0);
-        bool       want_pe = want_e || (rc.nsteps == 0 && a.pe_out != nullptr);
-        if constexpr (VIR) want_pe = want_pe || (rc.nsteps == 0 && a.vir_out != nullptr);   // ljmd_virial
-        const bool thermo  = kick1 && rc.thermo_every > 0 && rc.thermo_kT > 0.0f &&
-                             ((s + 1) % rc.thermo_every == 0);
-        const bool sample  = kick1 && rc.sample_every > 0 && (s % rc.sample_every == 0) &&
-                             (s / rc.sample_every < rc.S);
+        const StepFlags fl = step_flags<VIR>(rc, s, a.pe_out, a.vir_out);
         const float4* cur = spos + (size_t)b * a.N;
         float4*       nxt = spos + (size_t)(b ^ 1) * a.N;
         if (prof) tl = clock64();
@@ -896,14 +799,14 @@ ap_cluster_kernel(const CluArgs a) {
         SliceSum ss;
         float2 tvir = make_float2(0.0f, 0.0f);
         if constexpr (VIR) {
-            if (want_pe) {
+            if (fl.want_pe) {
                 const SliceSumVir sv = clu_slice_pe<CUTOFF, true>(cur, j0, j1, i0, i1, xi2, yi2, pc);
                 ss.fx = sv.fx; ss.fy = sv.fy; ss.pe = sv.pe; tvir = sv.vir;
             } else {
                 ss = clu_slice_f<CUTOFF>(cur, j0, j1, xi2, yi2, a.r2min, pc);
             }
         } else {
-            ss = want_pe ? clu_slice_pe<CUTOFF, false>(cur, j0, j1, i0, i1, xi2, yi2, pc)
+            ss = fl.want_pe ? clu_slice_pe<CUTOFF, false>(cur, j0, j1, i0, i1, xi2, yi2, pc)
                          : clu_slice_f<CUTOFF>(cur, j0, j1, xi2, yi2, a.r2min, pc);
         }
         float2 tfx = ss.fx, tfy = ss.fy;
@@ -914,52 +817,51 @@ ap_cluster_kernel(const CluArgs a) {
             tfy.x += __shfl_xor_sync(0xffffffffu, tfy.x, o);
             tfy.y += __shfl_xor_sync(0xffffffffu, tfy.y, o);
         }
-        if (want_pe) {                     // fixed tree: per-CTA potential energy -> CTA 0
+        if (fl.want_pe) {                  // fixed tree: per-CTA potential energy -> CTA 0
             const float t = block_sum<CLU_THREADS>((has0 ? tpe.x : 0.0f) + (has1 ? tpe.y : 0.0f), sred);
-            if (tid == 0) *cluster.map_shared_rank(&sE[(par * 2 + 0) * CLU_MAXC + k], 0) = t;
+            if (tid == 0) *cluster.map_shared_rank(&sE[(fl.par * 2 + 0) * CLU_MAXC + k], 0) = t;
         }
-        if (VIR && want_pe) {              // the virial partial takes the same route
+        if (VIR && fl.want_pe) {           // the virial partial takes the same route
             const float t = block_sum<CLU_THREADS>((has0 ? tvir.x : 0.0f) + (has1 ? tvir.y : 0.0f), sred);
-            if (tid == 0) *cluster.map_shared_rank(&sW[par * CLU_MAXC + k], 0) = t;
+            if (tid == 0) *cluster.map_shared_rank(&sW[fl.par * CLU_MAXC + k], 0) = t;
         }
         if (prof) { const long long t = clock64(); pt[0] += t - tl; tl = t; }
 
         // ---- finish the velocity-Verlet step of the pair (every lane of the group, redundantly) -------
         const float2 r0 = make_float2(-c0.x, -c0.z), r1 = make_float2(-c1.x, -c1.z);
-        if (kick1) {                                                                              // MD:74
+        if (fl.kick1) {                                                                           // MD:74
             v0.x = kick(v0.x, tfx.x, a.dt); v0.y = kick(v0.y, tfy.x, a.dt);
             v1.x = kick(v1.x, tfx.y, a.dt); v1.y = kick(v1.y, tfy.y, a.dt);
         }
-        if (sample && lead) {                                                                     // MD:93-100
+        if (fl.sample && lead) {                                                                  // MD:93-100
             float2* row = rc.traj + (size_t)(s / rc.sample_every) * a.N;
             if (has0) row[i0] = r0;
             if (has1) row[i1] = r1;
         }
-        if (want_e || thermo) {
+        if (fl.want_e || fl.thermo) {
             float ke_thread = 0.0f;
             if (lead && has0) ke_thread += v0.x * v0.x + v0.y * v0.y;
             if (lead && has1) ke_thread += v1.x * v1.x + v1.y * v1.y;
             const float t = block_sum<CLU_THREADS>(ke_thread, sred);
             if (tid == 0) {
-                if (want_e) *cluster.map_shared_rank(&sE[(par * 2 + 1) * CLU_MAXC + k], 0) = t;
-                if (thermo)
+                if (fl.want_e) *cluster.map_shared_rank(&sE[(fl.par * 2 + 1) * CLU_MAXC + k], 0) = t;
+                if (fl.thermo)
                     for (int q = 0; q < a.C; ++q) *cluster.map_shared_rank(&sK[k], q) = t;
             }
         }
-        if (thermo) {
-            // velocity rescale: V *= sqrt(kT_target / (KE/N)); every CTA sums the same C partials
+        if (fl.thermo) {
+            // velocity rescale; every CTA sums the same C partials
             cluster.sync();
             if (tid == 0) {
                 double ke2 = 0.0;
                 for (int q = 0; q < a.C; ++q) ke2 += (double)sK[q];
-                const float ke = (float)(0.5 * ke2);
-                s_lambda = ke > 0.0f ? sqrtf(rc.thermo_kT / (ke / (float)a.N)) : 1.0f;
+                s_lambda = rescale_lambda(ke2, rc.thermo_kT, a.N);
             }
             __syncthreads();
             const float lam = s_lambda;
             v0.x *= lam; v0.y *= lam; v1.x *= lam; v1.y *= lam;
         }
-        if (final) {
+        if (fl.final) {
             if (lead && has0) {
                 if (a.R_out) a.R_out[i0] = r0;
                 if (a.V_out) a.V_out[i0] = v0;
@@ -991,21 +893,14 @@ ap_cluster_kernel(const CluArgs a) {
         if (prof) { const long long t = clock64(); pt[2] += t - tl; tl = t; }
         b ^= 1;
 
-        if (k == 0 && tid == 0 && want_pe) {     // energies of the post-step state (fixed order, double)
+        if (k == 0 && tid == 0 && fl.want_pe) {  // energies of the post-step state (fixed order, double)
             double pe2 = 0.0, ke2 = 0.0, w2 = 0.0;
-            for (int q = 0; q < a.C; ++q) pe2 += (double)sE[(par * 2 + 0) * CLU_MAXC + q];
+            for (int q = 0; q < a.C; ++q) pe2 += (double)sE[(fl.par * 2 + 0) * CLU_MAXC + q];
             if (VIR)
-                for (int q = 0; q < a.C; ++q) w2 += (double)sW[par * CLU_MAXC + q];
-            if (want_e) {
-                for (int q = 0; q < a.C; ++q) ke2 += (double)sE[(par * 2 + 1) * CLU_MAXC + q];
-                float* o = rc.ke_pe + 2 * (s / rc.energy_every);
-                o[0] = (float)(0.5 * ke2);
-                o[1] = (float)(0.5 * pe2);       // MD:61  0.5 * sum over ordered pairs
-                if (VIR) a.vir_out[s / rc.energy_every] = (float)(0.5 * w2);
-            } else {
-                if (!VIR || a.pe_out) a.pe_out[0] = (float)(0.5 * pe2);
-                if (VIR) a.vir_out[0] = (float)(0.5 * w2);
-            }
+                for (int q = 0; q < a.C; ++q) w2 += (double)sW[fl.par * CLU_MAXC + q];
+            if (fl.want_e)
+                for (int q = 0; q < a.C; ++q) ke2 += (double)sE[(fl.par * 2 + 1) * CLU_MAXC + q];
+            store_energy_row<VIR>(rc, fl, pe2, ke2, w2, a.pe_out, a.vir_out);
         }
     }
     if (prof) {

@@ -50,14 +50,8 @@ namespace ljmd {
 
 namespace {
 
-#ifndef CL_B5_
-#define CL_B5_ 3
-#endif
-constexpr int CL_B5 = CL_B5_;     // slots per thread per trip of the rebuild gather (B5)
-#ifndef CL_THREADS_
-#define CL_THREADS_ 512
-#endif
-constexpr int CL_THREADS   = CL_THREADS_;
+constexpr int CL_B5        = 3;     // slots per thread per trip of the rebuild gather (B5)
+constexpr int CL_THREADS   = 512;
 constexpr int CL_K         = 4;     // bins per (rc + skin)
 constexpr int CL_E         = 8;     // list entries per particle (3 when every range fits 32 slots)
 constexpr int CL_WIN       = 84;    // staged window capacity per stencil row and warp (slots):
@@ -75,19 +69,7 @@ constexpr int CL_BROW      = 4 * CL_NW + 4;   // a lane's byte row while a list 
 constexpr int CL_WINBYTES  = CL_WSLOTS * 8;                 // 2048
 constexpr int CL_SWBYTES   = CL_NWS * 32 * 4;               // 1280
 constexpr int CL_WARP_SMEM = 2 * CL_WINBYTES + 2 * CL_SWBYTES;   // bytes per warp (6656)
-#ifndef CL_UNROLL
-#define CL_UNROLL 2
-#endif
-// how a unit's windows and list words reach shared memory: 0 = bulk copies (cp.async.bulk / UBLKCP issued by
-// four lanes, completion on an mbarrier), 1 = per-lane 16-byte cp.async (LDGSTS.128, commit / wait groups)
-#ifndef CL_COPY
-#define CL_COPY 0
-#endif
-#ifndef CL_DEPTH3
-#define CL_DEPTH3 0     // 1 = a warp holds three units in flight (the schedule before the two-unit pipeline)
-#endif
-
-constexpr int CL_WORD_UNROLL = CL_UNROLL;                   // list words per trip of the pair loop
+constexpr int CL_WORD_UNROLL = 2;                           // list words per trip of the pair loop
 constexpr int CL_UNITWORDS = CL_NW * 32;                    // list words of one 32-slot unit in nb4
 static_assert(CL_WINBYTES + 32 * CL_BROW <= CL_WARP_SMEM, "byte rows must fit behind window buffer 0");
 static_assert(CL_WARP_SMEM % 16 == 0 && CL_WIN % 2 == 0, "bulk copies need 16-byte granularity");
@@ -819,13 +801,6 @@ __device__ __forceinline__ bool mbar_try_wait(unsigned bar, unsigned parity) {
 //  the async-proxy reads of later bulk copies by one fence.proxy.async.global on each side of every grid
 //  barrier and after every cross-GPU sync: CL_BARRIER, peer_sync)
 
-__device__ __forceinline__ void cp_async16(unsigned dst, const void* src) {
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
-
 __device__ __forceinline__ float2 lds64(unsigned addr) {
     float2 v;
     asm volatile("ld.shared.v2.f32 {%0, %1}, [%2];" : "=f"(v.x), "=f"(v.y) : "r"(addr));
@@ -884,12 +859,6 @@ __device__ __noinline__ void mbar_wait_slow(const CellsArgs& a, unsigned bar, un
     }
 }
 
-struct StepFlags {
-    long long s;
-    int  par;
-    bool kick1, final, want_e, want_pe, want_ke, thermo, sample;
-};
-
 // per-warp pipeline state that outlives a step: shared-memory addresses and the mbarrier phases
 struct WarpPipe {
     unsigned base;      // this warp's block: window buffer 0 | window buffer 1 | word buffer 0 | word buffer 1
@@ -922,7 +891,7 @@ __device__ __forceinline__ void warp_pass(const CellsArgs& a, const Ctx& ctx, co
     const bool final  = PLAIN ? false : fl.final;
     const bool thermo = PLAIN ? false : fl.thermo;
     const bool sample = PLAIN ? false : fl.sample;
-    const bool want_ke = PLAIN ? false : fl.want_ke;
+    const bool want_ke = PLAIN ? false : (fl.want_e || fl.thermo);
     // halo pushes (slabs): slots of my first / last owned row and where they live in the neighbours
     const int dn = (a.me + a.P - 1) % a.P, up = (a.me + 1) % a.P;
     int first_e = 0, last_s = 0, peer_hi_start = 0;
@@ -948,29 +917,6 @@ __device__ __forceinline__ void warp_pass(const CellsArgs& a, const Ctx& ctx, co
     const char* Lbytes = reinterpret_cast<const char*>(a.nb4);
     const unsigned my_dst = wp.base + (lane < 3 ? lane * (CL_WIN * 8) : 2 * CL_WINBYTES);   // + buf * stride
     const unsigned my_stride = lane < 3 ? CL_WINBYTES : CL_SWBYTES;
-#if CL_COPY == 1
-    const unsigned l16 = lane * 16;
-    auto issue = [&](int u, const int4& p, int buf) {
-        if (u < u_hi && p.w < 0) {
-            const unsigned pw = (unsigned)p.w;
-            const unsigned win = wp.base + buf * CL_WINBYTES + l16, sw = wp.base + 2 * CL_WINBYTES + buf * CL_SWBYTES + l16;
-            const int wsk[3] = {p.x, p.y, p.z};
-#pragma unroll
-            for (int k = 0; k < 3; ++k) {           // a window is at most 84 slots = 672 bytes: chunks l16 and l16 + 512
-                const unsigned bytes = ((pw >> (8 * k)) & 0xffu) * 8u;
-                const char* src = Rbytes + (size_t)wsk[k] * 8 + l16;
-                if (l16 < bytes) cp_async16(win + k * (CL_WIN * 8), src);
-                if (l16 + 512 < bytes) cp_async16(win + k * (CL_WIN * 8) + 512, src + 512);
-            }
-            const unsigned wbytes = min((pw >> 24) & 0x7fu, (unsigned)CL_NWS) * 128u;
-            const char* src = Lbytes + (size_t)u * (CL_UNITWORDS * 4) + l16;
-#pragma unroll
-            for (int c = 0; c < CL_SWBYTES; c += 512)
-                if (l16 + c < wbytes) cp_async16(sw + c, src + c);
-        }
-        cp_async_commit();
-    };
-#else
     auto issue = [&](int u, const int4& p, int buf) {
         if (u < u_hi && p.w < 0) {
             const unsigned pw = (unsigned)p.w;
@@ -994,7 +940,6 @@ __device__ __forceinline__ void warp_pass(const CellsArgs& a, const Ctx& ctx, co
             }
         }
     };
-#endif
     // Schedule: the first ~60 % of the units statically interleaved (no traffic), the rest drawn one by
     // one from a per-step counter: warps that met several slow (edge) units take fewer of the tail.
     const int rounds0 = (int)(a.static_frac * (float)((u_hi - u_lo) / W));
@@ -1019,25 +964,14 @@ __device__ __forceinline__ void warp_pass(const CellsArgs& a, const Ctx& ctx, co
     if (u < u_hi) p = a.wplan[u];
     if (un < u_hi) q = a.wplan[un];
     issue(u, p, 0);
-#if CL_DEPTH3
-    int g3 = grab(2);
-#endif
 
     for (int k = 0; u < u_hi; ++k) {
         const int buf = k & 1;
         issue(un, q, buf ^ 1);                            // next unit's windows + words
-#if CL_DEPTH3
-        // (older schedule: a warp holds three units - the draw is made a whole unit before its plan is read)
-        const int unn = fix(__shfl_sync(0xffffffffu, g3, 0), k + 2);
-        g3 = grab(k + 3);
-        int4 r = z4;
-        if (unn < u_hi) r = a.wplan[unn];                 // consumed next iteration
-#else
         // the unit after next is drawn now; its number is broadcast and its plan requested after the pair
         // loop (the atomic's round trip hides behind it, the plan's behind the epilogue), so a warp holds
         // TWO units when the queue runs dry: a shorter tail at the step barrier
         const int g = grab(k + 2);
-#endif
         const int  i    = u * 32 + lane;
         const bool live = (i >= ctx.own_s) & (i < ctx.own_e);
         // epilogue operands requested now, consumed after the pair loop
@@ -1045,17 +979,11 @@ __device__ __forceinline__ void warp_pass(const CellsArgs& a, const Ctx& ctx, co
         if (live && (PLAIN || rc.nsteps > 0)) { v = V[i]; rb = a.Rb[i]; }
         float2 ri = make_float2(0.0f, 0.0f);
         float Fx = 0.0f, Fy = 0.0f, pe = 0.0f, ke = 0.0f, vir = 0.0f;
-#if CL_COPY == 1
-        cp_async_wait<1>();                               // this unit's copy group has landed
-        __syncwarp();
-#endif
         if (p.w < 0) {
-#if CL_COPY == 0
             // this unit's copies have landed when the buffer's mbarrier completes its phase
             const unsigned bar = wp.bar + buf * 8, par = (wp.phase >> buf) & 1u;
             if (!mbar_try_wait(bar, par)) mbar_wait_slow(a, bar, par);
             wp.phase ^= 1u << buf;
-#endif
             const unsigned win = wp.base + buf * CL_WINBYTES;
             CL_ASSERT(!live || (i - p.y >= 0 && i - p.y < (int)(((unsigned)p.w >> 8) & 0xffu)));
 #ifdef LJMD_DEBUG_CHECKS
@@ -1084,11 +1012,9 @@ __device__ __forceinline__ void warp_pass(const CellsArgs& a, const Ctx& ctx, co
             if (wedge) list_force<PE, true,  VIR>(a, R, ii, n, ri, Fx, Fy, pe, vir);
             else       list_force<PE, false, VIR>(a, R, ii, n, ri, Fx, Fy, pe, vir);
         }
-#if !CL_DEPTH3
         const int unn = fix(__shfl_sync(0xffffffffu, g, 0), k + 2);
         int4 r = z4;
         if (unn < u_hi) r = a.wplan[unn];                 // consumed at the top of the next iteration
-#endif
         if (live) {
             if (kick1) { v.x = kick(v.x, Fx, a.dt); v.y = kick(v.y, Fy, a.dt); }               // MD:74
             if (want_ke) ke = v.x * v.x + v.y * v.y;
@@ -1153,9 +1079,6 @@ __device__ __forceinline__ void warp_pass(const CellsArgs& a, const Ctx& ctx, co
         __syncwarp();                                     // all lanes are done with `buf`
         u = un; un = unn; p = q; q = r;
     }
-#if CL_COPY == 1
-    cp_async_wait<0>();
-#endif
 }
 
 extern __shared__ __align__(16) unsigned char cells_smem[];
@@ -1264,17 +1187,7 @@ cells_persistent_kernel(const CellsArgs a) {
     }
 
     for (long long s = a.s_begin; s < a.s_end; ++s) {
-        const int  par     = (int)((s + 1) & 1);
-        const bool kick1   = (s >= 0);
-        const bool final   = (s == rc.nsteps - 1);
-        const bool want_e  = kick1 && rc.energy_every > 0 && (s % rc.energy_every == 0);
-        bool       want_pe = want_e || (rc.nsteps == 0 && a.pe_out != nullptr);
-        if constexpr (VIR) want_pe = want_pe || (rc.nsteps == 0 && a.vir_out != nullptr);   // ljmd_virial
-        const bool thermo  = kick1 && rc.thermo_every > 0 && rc.thermo_kT > 0.0f &&
-                             ((s + 1) % rc.thermo_every == 0);
-        const bool sample  = kick1 && rc.sample_every > 0 && (s % rc.sample_every == 0) &&
-                             (s / rc.sample_every < rc.S);
-        const bool want_ke = want_e || thermo;
+        const StepFlags fl = step_flags<VIR>(rc, s, a.pe_out, a.vir_out);
         // rebuild requested by the previous step's displacement test?
         if (s > a.s_begin || a.s_begin >= 0) {
             if (__ldcg(a.state + ST_FLAG) == (int)(s + 1)) cells_rebuild(a, ctx, sscan, my_win, my_bytes, a.rlist2);
@@ -1284,22 +1197,19 @@ cells_persistent_kernel(const CellsArgs a) {
         float2*       Rnext = a.R[ctx.pr ^ 1];
         float2*       V     = a.V[ctx.pv];
         const int*    og    = a.orig[ctx.pv];
-        StepFlags fl;
-        fl.s = s; fl.par = par; fl.kick1 = kick1; fl.final = final; fl.want_e = want_e; fl.want_pe = want_pe;
-        fl.want_ke = want_ke; fl.thermo = thermo; fl.sample = sample;
         const int u_lo = ctx.own_s >> 5, u_hi = (ctx.own_e + 31) >> 5;      // 32-slot units
-        for (int k = gtid; k < CL_QMAX; k += gsz) __stcg(&a.sched[(par ^ 1) * CL_QMAX + k], 0);   // the other parity's unit counters: idle this step
+        for (int k = gtid; k < CL_QMAX; k += gsz) __stcg(&a.sched[(fl.par ^ 1) * CL_QMAX + k], 0);   // the other parity's unit counters: idle this step
         int moved = 0;
-        if (want_pe)
+        if (fl.want_pe)
             warp_pass<true, false, VIR>(a, ctx, fl, wp, moved);
-        else if (kick1 && !final && !thermo && !sample && !want_ke)
+        else if (fl.kick1 && !fl.final && !fl.thermo && !fl.sample && !fl.want_e)
             warp_pass<false, true, false>(a, ctx, fl, wp, moved);
         else
             warp_pass<false, false, false>(a, ctx, fl, wp, moved);
-        if (thermo) {
+        if (fl.thermo) {
             CL_BARRIER();
-            const double ke2 = block_sum_array(a.ke_part + par * a.nchunks, u_hi - u_lo, sdbl);
-            if (tid == 0) s_lambda = ke2 > 0.0 ? sqrtf(rc.thermo_kT / ((float)(0.5 * ke2) / (float)a.N)) : 1.0f;
+            const double ke2 = block_sum_array(a.ke_part + fl.par * a.nchunks, u_hi - u_lo, sdbl);
+            if (tid == 0) s_lambda = rescale_lambda(ke2, rc.thermo_kT, a.N);
             __syncthreads();
             const float lam = s_lambda;
             for (int i = ctx.own_s + gtid; i < ctx.own_e; i += gsz) {
@@ -1307,7 +1217,7 @@ cells_persistent_kernel(const CellsArgs a) {
                 const float2 F = a.Fs[i];
                 float2 v = V[i];
                 v.x *= lam; v.y *= lam;
-                if (final) {
+                if (fl.final) {
                     const int o = og[i];
                     if (a.R_out) a.R_out[o] = ri;
                     if (a.V_out) a.V_out[o] = v;
@@ -1328,9 +1238,9 @@ cells_persistent_kernel(const CellsArgs a) {
         // a particle left the skin/2 ball: ask for a rebuild before the next force evaluation.
         // The flag carries the step stamp, so it never needs clearing (no reset race).
         if (__syncthreads_or(moved) && tid == 0) __stcg(a.state + (a.P > 1 ? ST_LMOVED : ST_FLAG), (int)(s + 2));
-        if (!final) ctx.pr ^= 1;
+        if (!fl.final) ctx.pr ^= 1;
         CL_PROF(0);
-        if (final && a.blk > 0) __threadfence_system();      // the staged outputs live on peer GPUs
+        if (fl.final && a.blk > 0) __threadfence_system();      // the staged outputs live on peer GPUs
         unsigned long long gt0 = 0;
         if (ctx.pt && tid == 0) asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(gt0));
         CL_BARRIER();
@@ -1340,8 +1250,8 @@ cells_persistent_kernel(const CellsArgs a) {
             ctx.pt[9] = (long long)gt0; ctx.pt[10] = (long long)gt1;
         }
         CL_PROF(1);
-        if (a.P > 1 && final && a.blk > 0) (void)peer_sync(a, ctx, false);   // every rank's outputs have landed
-        if (a.P > 1 && !final) {
+        if (a.P > 1 && fl.final && a.blk > 0) (void)peer_sync(a, ctx, false);   // every rank's outputs have landed
+        if (a.P > 1 && !fl.final) {
             // one NVLink round trip per step: every rank's halo pushes have landed once all arrival
             // words carry this epoch; the words also carry "one of my particles left its skin/2 ball",
             // so that all ranks rebuild at the same step
@@ -1352,22 +1262,12 @@ cells_persistent_kernel(const CellsArgs a) {
         }
         CL_PROF(8);
 
-        if (blockIdx.x == 0 && want_pe) {
-            const double pe2 = block_sum_array(a.pe_part + par * a.nchunks, u_hi - u_lo, sdbl);
+        if (blockIdx.x == 0 && fl.want_pe) {
+            const double pe2 = block_sum_array(a.pe_part + fl.par * a.nchunks, u_hi - u_lo, sdbl);
             double ke2 = 0.0, w2 = 0.0;
-            if (want_e) ke2 = block_sum_array(a.ke_part + par * a.nchunks, u_hi - u_lo, sdbl);
-            if (VIR) w2 = block_sum_array(a.vir_part + par * a.nchunks, u_hi - u_lo, sdbl);
-            if (tid == 0) {
-                if (want_e) {
-                    float* o = rc.ke_pe + 2 * (s / rc.energy_every);
-                    o[0] = (float)(0.5 * ke2);
-                    o[1] = (float)(0.5 * pe2);
-                    if (VIR) a.vir_out[s / rc.energy_every] = (float)(0.5 * w2);
-                } else {
-                    if (!VIR || a.pe_out) a.pe_out[0] = (float)(0.5 * pe2);
-                    if (VIR) a.vir_out[0] = (float)(0.5 * w2);
-                }
-            }
+            if (fl.want_e) ke2 = block_sum_array(a.ke_part + fl.par * a.nchunks, u_hi - u_lo, sdbl);
+            if (VIR) w2 = block_sum_array(a.vir_part + fl.par * a.nchunks, u_hi - u_lo, sdbl);
+            if (tid == 0) store_energy_row<VIR>(rc, fl, pe2, ke2, w2, a.pe_out, a.vir_out);
         }
     }
     if (gtid == 0) {

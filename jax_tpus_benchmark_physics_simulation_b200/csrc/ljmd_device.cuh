@@ -93,13 +93,16 @@ __device__ __forceinline__ float2 pack_pinned(float lo, float hi) {
     return *reinterpret_cast<float2*>(&r);
 }
 
+// Packed evaluation of the two pairs (i0 <- j), (i1 <- j) against ONE j (broadcast): returns the
+// force scalars f2 and the displacements so that the caller can apply the term to BOTH sides
+// (Newton's third law: f_ji = -f_ij bit for bit, because the min-image and r2 are symmetric).
 template <bool CUTOFF, bool PE, bool KEEPTEST, bool VIR>
-__device__ __forceinline__ void pair2_accum(float2 xi2, float2 yi2, float2 nxj2, float2 nyj2,
-                                            bool keep0, bool keep1, const PairConsts& c,
-                                            const PairConsts2& c2, float2& fx2, float2& fy2,
-                                            float2& pe2, float2& vir2) {
-    float2 dx = __fadd2_rn(xi2, nxj2);
-    float2 dy = __fadd2_rn(yi2, nyj2);
+__device__ __forceinline__ void pair2_eval(float2 xi2, float2 yi2, float2 nxj2, float2 nyj2, bool keep0,
+                                           bool keep1, const PairConsts& c, const PairConsts2& c2,
+                                           float2& f, float2& dx, float2& dy, float2& pe2,
+                                           float2& vir2) {
+    dx = __fadd2_rn(xi2, nxj2);
+    dy = __fadd2_rn(yi2, nyj2);
     dx.x = min_image(dx.x, c.box, c.timg);
     dx.y = min_image(dx.y, c.box, c.timg);
     dy.x = min_image(dy.x, c.box, c.timg);
@@ -119,43 +122,21 @@ __device__ __forceinline__ void pair2_accum(float2 xi2, float2 yi2, float2 nxj2,
     }
     const float2 ir6 = __fmul2_rn(__fmul2_rn(ir2, ir2), ir2);
     const float2 t = __ffma2_rn(ir6, c2.c12, c2.nc6);
-    const float2 f = __fmul2_rn(t, __fmul2_rn(ir6, ir2));
-    fx2 = __ffma2_rn(f, dx, fx2);
-    fy2 = __ffma2_rn(f, dy, fy2);
+    f = __fmul2_rn(t, __fmul2_rn(ir6, ir2));
     if (PE) pe2 = __ffma2_rn(ir6, __ffma2_rn(ir6, c2.d12, c2.nd6), pe2);
     if (VIR) vir2 = __ffma2_rn(t, ir6, vir2);
 }
 
-// Packed evaluation of the two pairs (i0 <- j), (i1 <- j) against ONE j (broadcast): returns the
-// force scalars f2 and the displacements so that the caller can apply the term to BOTH sides
-// (Newton's third law: f_ji = -f_ij bit for bit, because the min-image and r2 are symmetric).
+// pair2_eval with the force on the two i accumulated
 template <bool CUTOFF, bool PE, bool KEEPTEST, bool VIR>
-__device__ __forceinline__ void pair2_eval(float2 xi2, float2 yi2, float xj, float yj, bool keep0,
-                                           bool keep1, const PairConsts& c, const PairConsts2& c2,
-                                           float2& f, float2& dx, float2& dy, float2& pe2,
-                                           float2& vir2) {
-    dx = __fadd2_rn(xi2, make_float2(-xj, -xj));
-    dy = __fadd2_rn(yi2, make_float2(-yj, -yj));
-    dx.x = min_image(dx.x, c.box, c.timg);
-    dx.y = min_image(dx.y, c.box, c.timg);
-    dy.x = min_image(dy.x, c.box, c.timg);
-    dy.y = min_image(dy.y, c.box, c.timg);
-    const float2 r2 = __ffma2_rn(__fmul2_rn(dx, dx), c2.one, __fmul2_rn(dy, dy));   // unfused sum
-    float2 ir2 = make_float2(rcp_approx(r2.x), rcp_approx(r2.y));
-    if (CUTOFF) {
-        const bool in0 = KEEPTEST ? (keep0 & (r2.x < c.rc2)) : (r2.x < c.rc2);
-        const bool in1 = KEEPTEST ? (keep1 & (r2.y < c.rc2)) : (r2.y < c.rc2);
-        ir2.x = in0 ? ir2.x : 0.0f;
-        ir2.y = in1 ? ir2.y : 0.0f;
-    } else if (KEEPTEST) {
-        ir2.x = keep0 ? ir2.x : 0.0f;
-        ir2.y = keep1 ? ir2.y : 0.0f;
-    }
-    const float2 ir6 = __fmul2_rn(__fmul2_rn(ir2, ir2), ir2);
-    const float2 t = __ffma2_rn(ir6, c2.c12, c2.nc6);
-    f = __fmul2_rn(t, __fmul2_rn(ir6, ir2));
-    if (PE) pe2 = __ffma2_rn(ir6, __ffma2_rn(ir6, c2.d12, c2.nd6), pe2);
-    if (VIR) vir2 = __ffma2_rn(t, ir6, vir2);
+__device__ __forceinline__ void pair2_accum(float2 xi2, float2 yi2, float2 nxj2, float2 nyj2,
+                                            bool keep0, bool keep1, const PairConsts& c,
+                                            const PairConsts2& c2, float2& fx2, float2& fy2,
+                                            float2& pe2, float2& vir2) {
+    float2 f, dx, dy;
+    pair2_eval<CUTOFF, PE, KEEPTEST, VIR>(xi2, yi2, nxj2, nyj2, keep0, keep1, c, c2, f, dx, dy, pe2, vir2);
+    fx2 = __ffma2_rn(f, dx, fx2);
+    fy2 = __ffma2_rn(f, dy, fy2);
 }
 
 // jnp.mod(x, box) of MD:72 (result has the divisor's sign; can return exactly `box` for tiny
@@ -230,6 +211,55 @@ __device__ __forceinline__ void grid_barrier(unsigned* counter, unsigned target,
         }
     }
     __syncthreads();                       // ... and the acquire is ordered before every thread's reads
+}
+
+// What step s of a persistent step kernel does (MD:77-106); s = -1 is the prologue force evaluation.
+struct StepFlags {
+    long long s;
+    int  par;        // parity of the partial-sum buffers this step writes
+    bool kick1, final, want_e, want_pe, thermo, sample;
+};
+
+// VIR: the virial instantiations also evaluate the energy terms for a one-shot ljmd_virial (nsteps == 0)
+template <bool VIR>
+__device__ __forceinline__ StepFlags step_flags(const RunCtl& rc, long long s, const float* pe_out,
+                                                const float* vir_out) {
+    StepFlags fl;
+    fl.s      = s;
+    fl.par    = (int)((s + 1) & 1);
+    fl.kick1  = (s >= 0);                              // the prologue only evaluates F(R_in)
+    fl.final  = (s == rc.nsteps - 1);
+    fl.want_e = fl.kick1 && rc.energy_every > 0 && (s % rc.energy_every == 0);
+    fl.want_pe = fl.want_e || (rc.nsteps == 0 && pe_out != nullptr);
+    // (under if constexpr: a short-circuit || here reshuffles the force-only kernels' prologue)
+    if constexpr (VIR) fl.want_pe = fl.want_pe || (rc.nsteps == 0 && vir_out != nullptr);
+    fl.thermo = fl.kick1 && rc.thermo_every > 0 && rc.thermo_kT > 0.0f && ((s + 1) % rc.thermo_every == 0);
+    fl.sample = fl.kick1 && rc.sample_every > 0 && (s % rc.sample_every == 0) &&
+                (s / rc.sample_every < rc.S);         // MD:93-100
+    return fl;
+}
+
+// The energies of an energy step from the kernel's fixed-order double sums over ordered pairs (pe2, and
+// w2 with the same weights) and over |v|^2 (ke2): a row of ke_pe (+ vir_out), or the one-shot results.
+template <bool VIR>
+__device__ __forceinline__ void store_energy_row(const RunCtl& rc, const StepFlags& fl, double pe2, double ke2,
+                                                 double w2, float* pe_out, float* vir_out) {
+    if (fl.want_e) {
+        float* o = rc.ke_pe + 2 * (fl.s / rc.energy_every);
+        o[0] = (float)(0.5 * ke2);
+        o[1] = (float)(0.5 * pe2);                     // MD:61  0.5 * sum over ordered pairs
+        if (VIR) vir_out[fl.s / rc.energy_every] = (float)(0.5 * w2);
+    } else {
+        if (!VIR || pe_out) pe_out[0] = (float)(0.5 * pe2);
+        if (VIR) vir_out[0] = (float)(0.5 * w2);
+    }
+}
+
+// Thermostat velocity rescale V *= lambda = sqrt(kT_target / (KE/N)), KE = 0.5 * ke2 (SURVEY App. A);
+// 1 when KE is 0 in fp32.
+__device__ __forceinline__ float rescale_lambda(double ke2, float kT, long long N) {
+    const float ke = (float)(0.5 * ke2);
+    return ke > 0.0f ? sqrtf(kT / (ke / (float)N)) : 1.0f;
 }
 
 // A caller's position on its way into the library: coordinates inside the closed interval [0, box]

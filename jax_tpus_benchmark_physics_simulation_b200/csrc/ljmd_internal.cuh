@@ -39,7 +39,7 @@ void set_error(const char* fmt, ...);
 struct PairConsts {
     float box, timg, rc2;
     float c12, c6, d12, d6;
-    float one;      // 1.0f passed at run time (blocks an unwanted FMA contraction, see pair2_accum)
+    float one;      // 1.0f passed at run time (blocks an unwanted FMA contraction, see pair2_eval)
     int   cutoff;   // 0 = none (the reference), 1 = plain truncation at rc
 };
 

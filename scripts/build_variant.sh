@@ -1,7 +1,7 @@
 #!/bin/bash
 # Build an A/B variant of libljmd.so with extra nvcc flags into variants/NAME/ (git-ignored, travels
 # with gpurun); select it at run time with LJMD_LIB=variants/NAME/libljmd.so.
-#   scripts/build_variant.sh maskcut -DCL_MASKCUT
+#   scripts/build_variant.sh debug -DLJMD_DEBUG_CHECKS
 set -e
 ROOT=$(cd "$(dirname "$0")/.." && pwd)
 NAME=$1; shift
