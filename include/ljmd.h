@@ -136,6 +136,17 @@ int ljmd_run_virial(ljmd_t* h, const float* R_in, const float* V_in, float* R_ou
 int ljmd_gr_hist(ljmd_t* h, const float* R_hist, int64_t S, int32_t nbins,
                  const float* edges, int64_t* counts);
 
+/* ljmd_gr_hist for callers that know on the host an upper bound r_max of the histogram range:
+ * counts exactly the pairs ljmd_gr_hist counts that also have r <= r_max, so with r_max >= edges[nbins]
+ * the result is ljmd_gr_hist's, bit for bit.  r_max: finite, > 0.  The library bins each snapshot into a
+ * periodic cell grid of edge >= r_max (at most N cells) and visits only neighbouring cells when that grid
+ * has >= 3 cells per side: O(S N rho pi r_max^2) work, which is what makes g(r) affordable for millions of
+ * particles.  Otherwise it runs the all-pairs histogram of ljmd_gr_hist.  nbins in [1, 8192].  S == 0 does
+ * nothing, and R_hist and counts may then be NULL.  Scratch for the grid is allocated on the first call
+ * that uses it and kept until ljmd_destroy.                                                          */
+int ljmd_gr_hist_rmax(ljmd_t* h, const float* R_hist, int64_t S, int32_t nbins,
+                      const float* edges, float r_max, int64_t* counts);
+
 /* ---- the other dense pairwise kernels of the reference repo (SURVEY.md 8f) -------- */
 /* All-pairs acceleration with the pair law as a functor: gravity r^-3 in an open plane.
  *   LJMD_LAW_GRAVITY_NBODY  pairwise_forces(positions, masses) of nbody_bh_merger_sim (NBODY:54-67):

@@ -929,13 +929,14 @@ ApKernel pick_kernel(int ipt, bool cutoff) {
 // ---- g(r): pair-distance histogram (get_histogram, MD:117-124) -------------------------------
 constexpr int GR_THREADS = 256;
 constexpr int GR_TILE    = 256;
-constexpr int GR_MAXBINS = 8192;
+constexpr int GR_MAXBINS = LJMD_GR_MAXBINS;
 
 __global__ void __launch_bounds__(GR_THREADS)
 gr_hist_kernel(const float2* __restrict__ Rh, int N, float box, float timg, int nbins,
                const float* __restrict__ edges, unsigned long long* __restrict__ counts,
-               int ntile) {
+               int ntile, float cap) {
     // blockIdx.x -> (tile_i <= tile_j) upper-triangular tile pair; blockIdx.y -> snapshot
+    // cap: pairs with r > cap are dropped as well (ljmd_gr_hist_rmax); +INFINITY for ljmd_gr_hist
     extern __shared__ unsigned char smem_raw[];
     float2*   sj     = reinterpret_cast<float2*>(smem_raw);                 // GR_TILE (8-byte aligned)
     float*    sedges = reinterpret_cast<float*>(sj + GR_TILE);              // nbins+1
@@ -955,19 +956,16 @@ gr_hist_kernel(const float2* __restrict__ Rh, int N, float box, float timg, int 
     const int i = ti * GR_TILE + tid;
     if (i < N) {
         const float2 ri = R[i];
-        const float lo = sedges[0], hi = sedges[nbins];
-        const float scale = (float)nbins / (hi - lo);
+        const float lo = sedges[0], hi = fminf(sedges[nbins], cap);
+        const float scale = (float)nbins / (sedges[nbins] - lo);
         for (int q = 0; q < GR_TILE; ++q) {
             const int j = tj * GR_TILE + q;
             if (j <= i || j >= N) continue;                                  // triu, k=1
             const float dx = min_image(__fsub_rn(ri.x, sj[q].x), box, timg);
             const float dy = min_image(__fsub_rn(ri.y, sj[q].y), box, timg);
             const float r = __fsqrt_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)));
-            if (!(r >= lo && r <= hi)) continue;                             // numpy drops outliers
-            int b = (int)((r - lo) * scale);
-            b = max(0, min(b, nbins - 1));
-            while (b > 0 && r < sedges[b]) --b;                              // exact against edges
-            while (b < nbins - 1 && r >= sedges[b + 1]) ++b;
+            const int b = gr_bin(r, sedges, nbins, lo, hi, scale);          // numpy drops outliers
+            if (b < 0) continue;
             atomicAdd(&shist[b], 1u);
         }
     }
@@ -1412,7 +1410,7 @@ int ap_check_error(ljmd_handle* h) {
 }
 
 int ap_gr_hist(ljmd_handle* h, const float2* R_hist, long long S, int nbins, const float* edges,
-               long long* counts) {
+               float cap, long long* counts) {
     const int N = (int)h->p.N;
     if (nbins < 1 || nbins > GR_MAXBINS) { set_error("g(r): nbins must be in [1,%d]", GR_MAXBINS); return LJMD_E_INVALID; }
     cudaStream_t st = h->stream;
@@ -1427,7 +1425,7 @@ int ap_gr_hist(ljmd_handle* h, const float2* R_hist, long long S, int nbins, con
         const int ns = (int)std::min<long long>(65535, S - s0);
         gr_hist_kernel<<<dim3((unsigned)npairs, ns), GR_THREADS, smem, st>>>(
             R_hist + (size_t)s0 * N, N, h->pc.box, h->pc.timg, nbins, edges,
-            reinterpret_cast<unsigned long long*>(counts) + (size_t)s0 * nbins, ntile);
+            reinterpret_cast<unsigned long long*>(counts) + (size_t)s0 * nbins, ntile, cap);
         LJ_CUDA(cudaGetLastError());
         h->launches++;
     }

@@ -115,6 +115,7 @@ void ljmd_destroy(ljmd_t* h) {
     ap_destroy(h);
     cells_destroy(h);
     dist_destroy(h);
+    gr_destroy(h);
     for (int k = 0; k < 4; ++k) cudaFree(h->blk_full[k]);
     if (h->ev0) cudaEventDestroy(h->ev0);
     if (h->ev1) cudaEventDestroy(h->ev1);
@@ -232,7 +233,24 @@ int ljmd_gr_hist(ljmd_t* h, const float* R_hist, int64_t S, int32_t nbins, const
     if (!h || !counts || !edges || (S > 0 && !R_hist) || S < 0) { set_error("bad argument"); return LJMD_E_INVALID; }
     LJ_CUDA(cudaSetDevice(h->p.device));
     return ap_gr_hist(h, reinterpret_cast<const float2*>(R_hist), S, nbins, edges,
-                      reinterpret_cast<long long*>(counts));
+                      std::numeric_limits<float>::infinity(), reinterpret_cast<long long*>(counts));
+}
+
+int ljmd_gr_hist_rmax(ljmd_t* h, const float* R_hist, int64_t S, int32_t nbins, const float* edges,
+                      float r_max, int64_t* counts) {
+    // with S == 0 there is nothing to read or write: R_hist and counts may then be NULL (empty arrays)
+    if (!h || !edges || (S > 0 && (!R_hist || !counts))) { set_error("ljmd_gr_hist_rmax: null argument"); return LJMD_E_INVALID; }
+    if (S < 0) { set_error("ljmd_gr_hist_rmax: S must be >= 0"); return LJMD_E_INVALID; }
+    if (nbins < 1 || nbins > LJMD_GR_MAXBINS) { set_error("ljmd_gr_hist_rmax: nbins must be in [1,%d]", LJMD_GR_MAXBINS); return LJMD_E_INVALID; }
+    if (!(r_max > 0.0f) || !std::isfinite(r_max)) { set_error("ljmd_gr_hist_rmax: r_max must be positive and finite"); return LJMD_E_INVALID; }
+    if (S == 0) return 0;
+    LJ_CUDA(cudaSetDevice(h->p.device));
+    const float2* R = reinterpret_cast<const float2*>(R_hist);
+    long long* c = reinterpret_cast<long long*>(counts);
+    // the cell grid needs 3 cells per side for its half stencil to visit every pair once
+    const int nc = gr_grid_side(h->p.N, h->p.box, r_max);
+    if (nc >= 3) return gr_cells_hist(h, R, S, nbins, edges, r_max, nc, c);
+    return ap_gr_hist(h, R, S, nbins, edges, r_max, c);
 }
 
 int ljmd_cell_geometry(ljmd_t* h, int32_t* nrows, int32_t* nbins_x, int32_t* kbins,

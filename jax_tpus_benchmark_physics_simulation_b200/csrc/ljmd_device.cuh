@@ -28,6 +28,20 @@ __device__ __forceinline__ float min_image(float d, float box, float timg) {
     return (fabsf(d) >= timg) ? __fsub_rn(d, copysignf(box, d)) : d;
 }
 
+// Histogram bin of the pair distance r with numpy.histogram's semantics (get_histogram, MD:117-124):
+// bin k holds e[k] <= r < e[k+1], the last bin is right-closed, r outside [lo, hi] gives -1.
+// e: the nbins+1 fp32 edges (ascending); lo = e[0]; hi = e[nbins], or less to drop longer pairs;
+// scale = nbins / (e[nbins] - lo).  The uniform guess is corrected against the fp32 edges, so the
+// result does not depend on how the edges were rounded.  Used by every g(r) kernel.
+__device__ __forceinline__ int gr_bin(float r, const float* e, int nbins, float lo, float hi, float scale) {
+    if (!(r >= lo && r <= hi)) return -1;
+    int b = (int)((r - lo) * scale);
+    b = max(0, min(b, nbins - 1));
+    while (b > 0 && r < e[b]) --b;
+    while (b < nbins - 1 && r >= e[b + 1]) ++b;
+    return b;
+}
+
 // One ordered pair (i <- j) of total_energy_fn / force_fn (MD:50-64):
 //   r2 = dx^2 + dy^2 with each operation rounded once (no FMA contraction), so the pair set
 //   {r2 < rc2} is decided on the same fp32 r2 as the CPU restatement;

@@ -11,6 +11,7 @@
 #include "../../include/ljmd.h"
 
 #define LJMD_MAX_RANKS 8
+#define LJMD_GR_MAXBINS 8192      // bins of a g(r) histogram: one 32-bit counter each in a CTA's shared memory
 
 namespace ljmd {
 
@@ -63,6 +64,7 @@ struct RunCtl {
 struct AllPairs;   // allpairs.cu
 struct Cells;      // cells.cu
 struct Dist;       // dist.cu
+struct Gr;         // gr.cu
 
 }  // namespace ljmd
 
@@ -75,6 +77,7 @@ struct ljmd_handle {
     ljmd::AllPairs*  ap;
     ljmd::Cells*     cells;
     ljmd::Dist*      dist;
+    ljmd::Gr*        gr;          // cell-grid g(r) scratch (allocated on the first ljmd_gr_hist_rmax that uses it)
     cudaEvent_t      ev0, ev1;
     bool             timed;
     long long        launches;
@@ -95,8 +98,9 @@ int  ap_run(ljmd_handle* h, const float2* R_in, const float2* V_in, float2* R_ou
             float2* F_out, float* pe_out, const RunCtl& rc, float* vir_out);
 int  ap_check_error(ljmd_handle* h);
 int  ap_mode(ljmd_handle* h);
+// cap: pairs with r > cap are dropped too (+INFINITY: the plain histogram of ljmd_gr_hist)
 int  ap_gr_hist(ljmd_handle* h, const float2* R_hist, long long S, int nbins, const float* edges,
-                long long* counts);
+                float cap, long long* counts);
 
 // cells.cu
 int  cells_create(ljmd_handle* h);
@@ -108,6 +112,12 @@ int  cells_assign(ljmd_handle* h, const float2* R, int* cell_id, int* cell_count
 int  cells_neighbor_count(ljmd_handle* h, const float2* R, float radius, int* nbr_count);
 long long cells_last_rebuilds(ljmd_handle* h);
 int  cells_check_error(ljmd_handle* h);
+
+// gr.cu: g(r) through a periodic nc x nc cell grid of edge >= r_max (see ljmd_gr_hist_rmax)
+int  gr_grid_side(long long N, float box, float r_max);   // nc for this r_max (the grid is used when >= 3)
+int  gr_cells_hist(ljmd_handle* h, const float2* R_hist, long long S, int nbins, const float* edges,
+                   float r_max, int nc, long long* counts);
+void gr_destroy(ljmd_handle* h);
 
 // api.cu
 int  create_common(ljmd_t** out, const ljmd_params* p, int rank, int nranks, const void* nccl_uid);

@@ -9,7 +9,8 @@ reference's behaviour): ``--rc`` (cutoff, default none), ``--path`` (auto|allpai
 the default: like the reference's run it overflows fp32 within a few steps - SURVEY.md §0 - and
 finishes with non-finite positions; ``lattice`` is the physical lattice+jitter state that the
 parity tests and bench.py use), ``--energy_every``, ``--pressure`` (records the pair virial on the
-energy rows and reports the mean and spread of P over the production).  matplotlib is imported
+energy rows and reports the mean and spread of P over the production), ``--gr_rmax`` (largest r of
+g(r); default box/2 as the reference, a few sigma for millions of particles).  matplotlib is imported
 lazily (absent in this image): without it g(r) is written as ``.npy``/``.csv`` next to
 ``--output``.
 """
@@ -60,7 +61,7 @@ def main(args):
 
     print("\n--- Calculating g(r) ---")
     dr_g = 0.05                                                                # MD:157-159
-    r_max_g = box_size / np.float32(2.0)
+    r_max_g = box_size / np.float32(2.0) if args.gr_rmax is None else np.float32(args.gr_rmax)
     nbins_g = int(r_max_g / dr_g)
     start_time_g_r = time.time()
     r_bins_g, g_r = sim.calculate_g_r(R_history, N, box_size, nbins_g, r_max_g)   # MD:162
@@ -123,6 +124,9 @@ def build_parser():
     parser.add_argument("--pressure", action="store_true",
                         help="record the pair virial on the energy rows and report the pressure "
                              "(needs --energy_every > 0)")
+    parser.add_argument("--gr_rmax", type=float, default=None,
+                        help="largest r of g(r) (default: box/2, as the reference).  A few sigma makes "
+                             "g(r) work for millions of particles: only pairs within it are visited")
     return parser
 
 
@@ -131,6 +135,8 @@ def parse_args(argv=None):
     args = parser.parse_args(argv)
     if args.pressure and args.energy_every <= 0:
         parser.error("--pressure needs --energy_every > 0")
+    if args.gr_rmax is not None and not (args.gr_rmax > 0 and np.isfinite(args.gr_rmax)):
+        parser.error("--gr_rmax must be positive and finite")
     return args
 
 

@@ -328,9 +328,10 @@ class LJSimulation:
 
     # ------------------------------------------------------------------ MD:108-131
     def calculate_g_r(self, R_history, N_local=None, box_size_local=None, nbins=None, r_max=None):
-        """Radial distribution function (MD:108-129).  The O(S N^2) pair-distance histogram runs
-        on the GPU (ljmd_gr_hist); the nbins-long normalisation is host arithmetic in fp32 as in
-        the reference."""
+        """Radial distribution function (MD:108-129).  The pair-distance histogram runs on the GPU
+        (ljmd_gr_hist_rmax with the last edge as r_max: a cell grid visits only the pairs within r_max
+        when the box holds at least 3 cells of that edge per side, else all S N^2/2 pairs); the
+        nbins-long normalisation is host arithmetic in fp32 as in the reference."""
         N = self.N if N_local is None else int(N_local)
         if N != self.N:
             raise ValueError("calculate_g_r: N must match the simulation")
@@ -349,8 +350,8 @@ class LJSimulation:
         edges = torch.from_numpy(r_bins).to(self.device)
         counts = torch.empty((S, nbins), dtype=torch.int64, device=self.device)
         self._check_stream()
-        _lib.check(self.lib.ljmd_gr_hist(self._h, Rh.data_ptr(), S, nbins, edges.data_ptr(),
-                                         counts.data_ptr()), "ljmd_gr_hist")
+        _lib.check(self.lib.ljmd_gr_hist_rmax(self._h, Rh.data_ptr(), S, nbins, edges.data_ptr(),
+                                              float(r_bins[-1]), counts.data_ptr()), "ljmd_gr_hist_rmax")
         self._after()
         self.last_gr_counts = DeviceArray(counts)
         avg = counts.to(torch.float32).mean(dim=0) if S else torch.zeros(nbins, device=self.device)
