@@ -147,6 +147,26 @@ int ljmd_gr_hist(ljmd_t* h, const float* R_hist, int64_t S, int32_t nbins,
 int ljmd_gr_hist_rmax(ljmd_t* h, const float* R_hist, int64_t S, int32_t nbins,
                       const float* edges, float r_max, int64_t* counts);
 
+/* ---- density modes and the static structure factor (new; the reference has no S(k) - see DESIGN.md) ---- */
+/* Density modes rho_k(s) = sum_j exp(i 2pi (n_x x_j + n_y y_j) / box) of S snapshots for K integer wave vectors
+ * n = (n_x, n_y), k = (2pi / box) n; the structure factor is S(k) = <|rho_k|^2> / N.
+ * R_hist: device (S,N,2) float32, 8-byte aligned; nvec: device int32 (K,2), any integers, 8-byte aligned;
+ * rho: device float64 (S,K,2) = (Re, Im), 16-byte aligned.
+ *   - Fixed-point phase: each coordinate is converted once to the 32-bit phase word rint(x / box * 2^32) mod 2^32
+ *     and the phase of a term is n_x q_x + n_y q_y in uint32 arithmetic, exact modulo one revolution.  Positions
+ *     may lie anywhere: a coordinate outside [0, box] is taken periodically (x and x + box give the same bits).
+ *   - Accuracy, for each of Re and Im: |rho_k - exact| <= N eps_term + N 16.5 2^-24 + (N/32 + 1024) N 2^-53 with
+ *     eps_term = (|n_x| + |n_y|) pi 2^-32 + 1.074e-6 (phase words, fp32 angle, MUFU sin/cos; the second term is
+ *     the fp32 sum over chunks of 32 particles; derivation in csrc/sk.cu and DESIGN.md 4.5), for |x| <= 1024 box.
+ *   - NaN: a snapshot with a non-finite coordinate gets NaN in every rho_k of its row; other rows are unaffected.
+ *   - Deterministic: the same bits on every run, and rho_k of a (snapshot, vector) does not depend on the other
+ *     snapshots and vectors of the call (the particle split depends on N only).
+ *   - Any handle works, the multi-GPU ones included; there is no communication: each rank computes on the
+ *     snapshots it was given.  Two launches per batch; partial-sum scratch (<= 512 MiB, snapshots and vectors
+ *     batched to fit) is allocated on the first call and kept until ljmd_destroy.
+ * S < 0, K < 0 or a NULL array: LJMD_E_INVALID.  S == 0 or K == 0 does nothing, and the arrays may then be NULL. */
+int ljmd_density_modes(ljmd_t* h, const float* R_hist, int64_t S, const int32_t* nvec, int64_t K, double* rho);
+
 /* ---- the other dense pairwise kernels of the reference repo (SURVEY.md 8f) -------- */
 /* All-pairs acceleration with the pair law as a functor: gravity r^-3 in an open plane.
  *   LJMD_LAW_GRAVITY_NBODY  pairwise_forces(positions, masses) of nbody_bh_merger_sim (NBODY:54-67):

@@ -116,6 +116,7 @@ void ljmd_destroy(ljmd_t* h) {
     cells_destroy(h);
     dist_destroy(h);
     gr_destroy(h);
+    sk_destroy(h);
     for (int k = 0; k < 4; ++k) cudaFree(h->blk_full[k]);
     if (h->ev0) cudaEventDestroy(h->ev0);
     if (h->ev1) cudaEventDestroy(h->ev1);
@@ -251,6 +252,21 @@ int ljmd_gr_hist_rmax(ljmd_t* h, const float* R_hist, int64_t S, int32_t nbins, 
     const int nc = gr_grid_side(h->p.N, h->p.box, r_max);
     if (nc >= 3) return gr_cells_hist(h, R, S, nbins, edges, r_max, nc, c);
     return ap_gr_hist(h, R, S, nbins, edges, r_max, c);
+}
+
+int ljmd_density_modes(ljmd_t* h, const float* R_hist, int64_t S, const int32_t* nvec, int64_t K, double* rho) {
+    if (!h) { set_error("ljmd_density_modes: null handle"); return LJMD_E_INVALID; }
+    if (S < 0 || K < 0) { set_error("ljmd_density_modes: S and K must be >= 0"); return LJMD_E_INVALID; }
+    // with S == 0 or K == 0 there is nothing to read or write: the arrays may then be NULL (empty)
+    if (S == 0 || K == 0) return 0;
+    if (!R_hist || !nvec || !rho) { set_error("ljmd_density_modes: null argument"); return LJMD_E_INVALID; }
+    if ((uintptr_t)R_hist % 8 || (uintptr_t)nvec % 8 || (uintptr_t)rho % 16) {
+        set_error("ljmd_density_modes: R_hist and nvec must be 8-byte aligned, rho 16-byte aligned");
+        return LJMD_E_INVALID;
+    }
+    LJ_CUDA(cudaSetDevice(h->p.device));
+    return sk_density_modes(h, reinterpret_cast<const float2*>(R_hist), S, reinterpret_cast<const int2*>(nvec), K,
+                            reinterpret_cast<double2*>(rho));
 }
 
 int ljmd_cell_geometry(ljmd_t* h, int32_t* nrows, int32_t* nbins_x, int32_t* kbins,

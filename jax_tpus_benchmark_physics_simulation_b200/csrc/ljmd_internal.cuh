@@ -65,6 +65,7 @@ struct AllPairs;   // allpairs.cu
 struct Cells;      // cells.cu
 struct Dist;       // dist.cu
 struct Gr;         // gr.cu
+struct Sk;         // sk.cu
 
 }  // namespace ljmd
 
@@ -84,6 +85,7 @@ struct ljmd_handle {
     int              rank, nranks;
     long long        spin_limit;  // clocks a device-side spin wait may last (0 = unlimited)
     float2*          blk_full[4]; // all-pairs ljmd_run_blocked: replicated in / out arrays (allocated on first use)
+    ljmd::Sk*        sk;          // density-mode partial sums (allocated on the first ljmd_density_modes)
 };
 
 namespace ljmd {
@@ -118,6 +120,11 @@ int  gr_grid_side(long long N, float box, float r_max);   // nc for this r_max (
 int  gr_cells_hist(ljmd_handle* h, const float2* R_hist, long long S, int nbins, const float* edges,
                    float r_max, int nc, long long* counts);
 void gr_destroy(ljmd_handle* h);
+
+// sk.cu: density modes rho_k of S snapshots for K integer wave vectors (see ljmd_density_modes)
+int  sk_density_modes(ljmd_handle* h, const float2* R_hist, long long S, const int2* nvec, long long K,
+                      double2* rho);
+void sk_destroy(ljmd_handle* h);
 
 // api.cu
 int  create_common(ljmd_t** out, const ljmd_params* p, int rank, int nranks, const void* nccl_uid);

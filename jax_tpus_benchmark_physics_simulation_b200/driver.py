@@ -10,7 +10,9 @@ the default: like the reference's run it overflows fp32 within a few steps - SUR
 finishes with non-finite positions; ``lattice`` is the physical lattice+jitter state that the
 parity tests and bench.py use), ``--energy_every``, ``--pressure`` (records the pair virial on the
 energy rows and reports the mean and spread of P over the production), ``--gr_rmax`` (largest r of
-g(r); default box/2 as the reference, a few sigma for millions of particles).  matplotlib is imported
+g(r); default box/2 as the reference, a few sigma for millions of particles), ``--sk_kmax`` /
+``--sk_per_shell`` (the static structure factor S(k) of the production snapshots up to |k| = sk_kmax,
+default off; written as ``<stem>_sk.npy``/``.csv`` next to ``--output``).  matplotlib is imported
 lazily (absent in this image): without it g(r) is written as ``.npy``/``.csv`` next to
 ``--output``.
 """
@@ -69,11 +71,29 @@ def main(args):
     time_g_r = time.time() - start_time_g_r
     print(f"g(r) calculation complete in {time_g_r:.2f} s")
 
+    sk = None
+    if args.sk_kmax is not None:
+        print("\n--- Calculating S(k) ---")
+        start_time_sk = time.time()
+        k_sk, S_sk = sim.structure_factor(R_history, args.sk_kmax, args.sk_per_shell)
+        S_sk.block_until_ready()
+        time_sk = time.time() - start_time_sk
+        sk = (np.asarray(k_sk), np.asarray(S_sk))
+        print(f"S(k) calculation complete in {time_sk:.2f} s")
+
     print("\nSimulation Summary")
     print(f"  Equilibration  {time_eq:8.2f} s   {args.eq_steps:,} steps")
     print(f"  Production     {time_prod:8.2f} s   {args.prod_steps:,} steps")
     print(f"  g(r) Analysis  {time_g_r:8.2f} s   Collected {R_history.shape[0]} snapshots")
-    print(f"  Total          {time_eq + time_prod + time_g_r:8.2f} s")
+    if sk is not None:
+        print(f"  S(k) Analysis  {time_sk:8.2f} s   {sim.last_sk_nvec.shape[0]} wave vectors in {sk[0].size} shells")
+        if np.isfinite(sk[1]).any():
+            i = int(np.nanargmax(sk[1]))
+            print(f"  S(k) first peak: k = {sk[0][i]:.4f}  S = {sk[1][i]:.4f}")
+        else:
+            print("  S(k) first peak: none (S(k) is not finite)")
+    total = time_eq + time_prod + time_g_r + (time_sk if sk is not None else 0.0)
+    print(f"  Total          {total:8.2f} s")
     if sim.last_energies is not None:
         e = sim.last_energies.numpy()
         print(f"  Energy (KE+PE) first/last sample: {e[0].sum():.4f} / {e[-1].sum():.4f}")
@@ -100,6 +120,12 @@ def main(args):
         np.save(stem + ".npy", np.stack([r_np, g_np]))
         np.savetxt(stem + ".csv", np.stack([r_np, g_np], axis=1), delimiter=",", header="r,g_r")
         print(f"matplotlib unavailable: g(r) saved as '{stem}.npy' and '{stem}.csv'")
+    if sk is not None:
+        stem = args.output.rsplit(".", 1)[0] + "_sk"
+        np.save(stem + ".npy", np.stack(sk))
+        np.savetxt(stem + ".csv", np.stack(sk, axis=1), delimiter=",", header="k,S_k")
+        print(f"S(k) saved as '{stem}.npy' and '{stem}.csv'")
+        return state_final, R_history, (r_np, g_np), sk
     return state_final, R_history, (r_np, g_np)
 
 
@@ -127,6 +153,12 @@ def build_parser():
     parser.add_argument("--gr_rmax", type=float, default=None,
                         help="largest r of g(r) (default: box/2, as the reference).  A few sigma makes "
                              "g(r) work for millions of particles: only pairs within it are visited")
+    parser.add_argument("--sk_kmax", type=float, default=None,
+                        help="compute the static structure factor S(k) of the production snapshots for "
+                             "0 < |k| <= sk_kmax (default: off)")
+    parser.add_argument("--sk_per_shell", type=int, default=None,
+                        help="with --sk_kmax: at most this many wave vectors per shell floor(|n|), evenly "
+                             "spread in angle (default: all)")
     return parser
 
 
@@ -137,6 +169,10 @@ def parse_args(argv=None):
         parser.error("--pressure needs --energy_every > 0")
     if args.gr_rmax is not None and not (args.gr_rmax > 0 and np.isfinite(args.gr_rmax)):
         parser.error("--gr_rmax must be positive and finite")
+    if args.sk_kmax is not None and not (args.sk_kmax > 0 and np.isfinite(args.sk_kmax)):
+        parser.error("--sk_kmax must be positive and finite")
+    if args.sk_per_shell is not None and args.sk_per_shell < 1:
+        parser.error("--sk_per_shell must be >= 1")
     return args
 
 

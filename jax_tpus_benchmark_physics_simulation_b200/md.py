@@ -358,6 +358,48 @@ class LJSimulation:
         g = avg / torch.from_numpy(ideal.astype(np.float32)).to(self.device)      # MD:126-128
         return DeviceArray(torch.from_numpy(centers).to(self.device)), DeviceArray(g)
 
+    # ------------------------------------------------------------------ S(k) (new)
+    def density_modes(self, R_history, nvec) -> DeviceArray:
+        """rho_k(s) = sum_j exp(i 2 pi (n_x x_j + n_y y_j) / box) of the snapshots R_history (S, N, 2) (or one
+        (N, 2) state) for the integer wave vectors nvec (K, 2): a float64 (S, K, 2) = (Re, Im) device array
+        (ljmd_density_modes; fixed-point phase, accuracy bound and NaN rule in include/ljmd.h)."""
+        Rh = self._dev(R_history)
+        if Rh.dim() == 2:
+            Rh = Rh[None]
+        if Rh.dim() != 3 or tuple(Rh.shape[1:]) != (self.N, 2):
+            raise ValueError(f"expected snapshots of shape (S, {self.N}, 2), got {tuple(Rh.shape)}")
+        nv = torch.as_tensor(np.asarray(nvec, dtype=np.int32).reshape(-1, 2)).to(self.device).contiguous()
+        S, K = Rh.shape[0], nv.shape[0]
+        rho = torch.empty((S, K, 2), dtype=torch.float64, device=self.device)
+        self._check_stream()
+        _lib.check(self.lib.ljmd_density_modes(self._h, Rh.data_ptr() if S else None, S,
+                                               nv.data_ptr() if K else None, K, rho.data_ptr() if S * K else None),
+                   "ljmd_density_modes")
+        self._after()
+        return self._arr(rho)
+
+    def structure_factor(self, R_history, k_max: float, max_per_shell: Optional[int] = None):
+        """Static structure factor S(k) = <|rho_k|^2> / N over the snapshots R_history, in shells of the wave
+        vectors k = (2 pi / box) n with 0 < |k| <= k_max (``structure_factor_vectors``).  Returns (k, S_k)
+        float64 device arrays, one entry per non-empty shell: k the mean |k| of the shell's vectors, S_k the
+        mean of |rho_k|^2 / N over the snapshots and those vectors.  The vectors (``last_sk_nvec``, (K, 2)),
+        their shells (``last_sk_shell``, (K,)) and the per-snapshot |rho_k|^2 / N (``last_sk_power``, (S, K))
+        are kept."""
+        box = float(self.box_size)
+        nvec, shell = structure_factor_vectors(box, k_max, max_per_shell)
+        rho = self.density_modes(R_history, nvec).tensor
+        power = (rho[..., 0] ** 2 + rho[..., 1] ** 2) / self.N                   # (S, K) float64
+        self.last_sk_nvec, self.last_sk_shell = nvec, shell
+        self.last_sk_power = self._arr(power)
+        kmag = (2.0 * np.pi / box) * np.sqrt(np.sum(nvec.astype(np.float64) ** 2, axis=1))
+        starts = np.flatnonzero(np.r_[True, shell[1:] != shell[:-1]]) if shell.size else np.zeros(0, np.int64)
+        counts = np.diff(np.r_[starts, shell.size])
+        mean_v = power.mean(dim=0).cpu().numpy() if power.shape[0] else np.full(shell.size, np.nan)
+        k = np.add.reduceat(kmag, starts) / counts if shell.size else np.zeros(0)
+        S_k = np.add.reduceat(mean_v, starts) / counts if shell.size else np.zeros(0)
+        return (self._arr(torch.from_numpy(k).to(self.device)),
+                self._arr(torch.from_numpy(S_k).to(self.device)))
+
     # ------------------------------------------------------------------ cell-list introspection
     def cell_geometry(self):
         """(nrows, nbins_x, kbins, inv_row_height, inv_bin_width) of the strip-cell grid."""
@@ -410,6 +452,62 @@ class LJSimulation:
         v = ctypes.c_int64()
         _lib.check(self.lib.ljmd_launch_count(self._h, ctypes.byref(v)), "ljmd_launch_count")
         return v.value
+
+
+def _isqrt(n2: np.ndarray) -> np.ndarray:
+    """floor(sqrt(n2)) exactly for non-negative int64 n2 < 2^52: the float root is off by at most one."""
+    m = np.floor(np.sqrt(n2.astype(np.float64))).astype(np.int64)
+    m -= (m * m > n2)
+    m += ((m + 1) * (m + 1) <= n2)
+    return m
+
+
+def structure_factor_vectors(box: float, k_max: float, max_per_shell: Optional[int] = None):
+    """Integer wave vectors n of S(k) for a periodic box: k = (2 pi / box) n.
+
+    One vector of each +-k pair (rho_{-k} = conj(rho_k)): the half plane n_y > 0, or n_y = 0 and n_x > 0, with
+    0 < |k| <= k_max (decided as (2 pi / box) sqrt(n_x^2 + n_y^2) <= k_max in float64).  Vectors are grouped in
+    shells m = floor(|n|), computed exactly with an integer square root, and ordered by shell and then by angle
+    atan2(n_y, n_x) in [0, pi).  With ``max_per_shell`` = M, a shell of L > M vectors keeps the M at angle ranks
+    floor((i + 1/2) L / M), i = 0..M-1: evenly spread in angle, deterministic.
+    Returns (nvec (K, 2) int32, shell (K,) int64)."""
+    box, k_max = float(box), float(k_max)
+    if not (math.isfinite(k_max) and k_max > 0):
+        raise ValueError("k_max must be positive and finite")
+    if not (math.isfinite(box) and box > 0):
+        raise ValueError("box must be positive and finite")
+    if max_per_shell is not None and int(max_per_shell) < 1:
+        raise ValueError("max_per_shell must be >= 1")
+    dk = 2.0 * math.pi / box
+    nmax = int(math.floor(k_max / dk)) + 1
+    if nmax >= 1 << 15:
+        raise ValueError(f"k_max = {k_max} asks for |n| up to {nmax}: too many wave vectors")
+    ny = np.arange(0, nmax + 1, dtype=np.int64)
+    width = _isqrt(np.maximum(nmax * nmax - ny * ny, 0))                   # |n_x| <= width on row n_y
+    lo = np.where(ny > 0, -width, 1)                                       # row 0: n_x > 0 only
+    cnt = np.maximum(width - lo + 1, 0)
+    rows = np.repeat(ny, cnt)
+    first = np.cumsum(cnt) - cnt
+    nx = np.arange(rows.size, dtype=np.int64) - np.repeat(first, cnt) + np.repeat(lo, cnt)
+    n2 = nx * nx + rows * rows
+    keep = dk * np.sqrt(n2.astype(np.float64)) <= k_max
+    nx, rows, n2 = nx[keep], rows[keep], n2[keep]
+    m = _isqrt(n2)
+    # one float key orders by shell, then angle: two directions with |n| < 2^15 differ in angle by >= 1/|n|^2 > 2^-30,
+    # and the key (< 2^17) resolves 2^-35, so the keys are distinct and the order is unique
+    order = np.argsort(m.astype(np.float64) * 4.0 + np.arctan2(rows, nx))
+    nx, rows, m = nx[order], rows[order], m[order]
+    if max_per_shell is not None and m.size:
+        M = int(max_per_shell)
+        starts = np.flatnonzero(np.r_[True, m[1:] != m[:-1]])
+        L = np.diff(np.r_[starts, m.size])
+        big = L > M
+        sel = np.ones(m.size, dtype=bool)
+        for s0, ln in zip(starts[big], L[big]):
+            sel[s0:s0 + ln] = False
+            sel[s0 + (2 * np.arange(M) + 1) * ln // (2 * M)] = True
+        nx, rows, m = nx[sel], rows[sel], m[sel]
+    return np.stack([nx, rows], axis=1).astype(np.int32), m
 
 
 def slab_range(N: int, rank: int, nranks: int) -> Tuple[int, int]:
