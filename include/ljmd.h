@@ -167,6 +167,44 @@ int ljmd_gr_hist_rmax(ljmd_t* h, const float* R_hist, int64_t S, int32_t nbins,
  * S < 0, K < 0 or a NULL array: LJMD_E_INVALID.  S == 0 or K == 0 does nothing, and the arrays may then be NULL. */
 int ljmd_density_modes(ljmd_t* h, const float* R_hist, int64_t S, const int32_t* nvec, int64_t K, double* rho);
 
+/* ---- bond-orientational order (new; the reference has neither - see DESIGN.md) ----------------------------- */
+/* psi_m(i) = (1/n_i) sum_{j in nb(i)} exp(i m theta_ij) of every particle of S snapshots.
+ * R_hist: device (S,N,2) float32 in [0, box] (what production_fn returns; other input does not fault), 8-byte
+ * aligned; psi: device float64 (S,N,2) = (Re, Im) in ORIGINAL particle order, 16-byte aligned; nnb: device int32
+ * (S,N) = n_i, or NULL.  m in [1, 12]; r_nb finite and > 0.
+ *   - Neighbours: j != i with 0 < r_ij <= r_nb, r_ij exactly the fp32 minimum-image r that ljmd_gr_hist bins, so
+ *     sum_i n_i = 2 x the ljmd_gr_hist_rmax count with edges [0, r_nb] when no two particles coincide.
+ *   - Bond term: d = min_image(fl(x_j - x_i)) (from i to j) in double, u = d / |d| and w = u^m by m - 1 sequential
+ *     complex products, every double operation rounded once.
+ *   - Fixed point: each component of w is added as llrint(w 2^32) in int64 (exact, order-free), and
+ *     psi_i = (double)sum 2^-32 / n_i; psi_i = 0 when n_i = 0.  |psi_i - exact| <= 2^-33 + (9m + 3) 2^-53 per
+ *     component (derivation in csrc/bond.cu).
+ *   - NaN: a particle with a non-finite coordinate gets psi = NaN and n = 0 and is no particle's neighbour; other
+ *     particles are unaffected.
+ *   - Deterministic: the same bits on every run, whatever the other snapshots of the call or the batching.
+ *   - Through the periodic cell grid of ljmd_gr_hist_rmax (cells of edge >= r_nb, full 9-cell stencil; one cell,
+ *     i.e. all pairs, when r_nb > box / 3).  Four launches per batch of snapshots; the scratch is the grid's (16 B
+ *     per particle and snapshot, batches <= 512 MiB), allocated on first use and kept until ljmd_destroy.
+ *   - Any handle works, the multi-GPU ones included; there is no communication: each rank computes on the
+ *     snapshots it was given.
+ * S < 0, m or r_nb out of range, a NULL or misaligned array: LJMD_E_INVALID.  S == 0 does nothing, and the
+ * arrays may then be NULL.                                                                                       */
+int ljmd_bond_order(ljmd_t* h, const float* R_hist, int64_t S, int32_t m, float r_nb,
+                    double* psi, int32_t* nnb);
+
+/* Pair correlation of psi: the histogram of ljmd_gr_hist_rmax (same edges, r_max, pairs and selection of the
+ * cell grid or the all-pairs kernel) with a weight per pair.  For every pair it counts,
+ * w_ij = Re psi_i Re psi_j + Im psi_i Im psi_j (two products and the sum, each rounded once); a pair with a
+ * non-finite w_ij is skipped, any other adds 1 to counts[s*nbins + k] and llrint(w_ij 2^24) to wsum[s*nbins + k].
+ * g_m(r) = wsum / (2^24 counts).  psi: device float64 (S,N,2) as ljmd_bond_order writes it (|psi| <= 1),
+ * 16-byte aligned; counts, wsum: device int64 (S,nbins).  wsum is exact and order-free while every count is
+ * below 2^38 (|llrint(w 2^24)| <= 2^24 + 1), which a count can only reach for N > 741,455.  The counts equal
+ * ljmd_gr_hist_rmax's bit for bit when every psi is finite.  Scratch: the grid's (28 B per particle
+ * and snapshot, batches <= 512 MiB).
+ * Validation as ljmd_gr_hist_rmax, plus psi 16-byte aligned; S == 0 does nothing and accepts NULL arrays.        */
+int ljmd_bond_corr(ljmd_t* h, const float* R_hist, const double* psi, int64_t S, int32_t nbins,
+                   const float* edges, float r_max, int64_t* counts, int64_t* wsum);
+
 /* ---- the other dense pairwise kernels of the reference repo (SURVEY.md 8f) -------- */
 /* All-pairs acceleration with the pair law as a functor: gravity r^-3 in an open plane.
  *   LJMD_LAW_GRAVITY_NBODY  pairwise_forces(positions, masses) of nbody_bh_merger_sim (NBODY:54-67):

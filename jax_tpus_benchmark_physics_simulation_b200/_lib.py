@@ -23,7 +23,7 @@ EXPORTS = (
     "ljmd_neighbor_count", "ljmd_last_rebuilds", "ljmd_get_unique_id", "ljmd_create_dist",
     "ljmd_last_run_ms", "ljmd_launch_count", "ljmd_fp32_peak_probe", "ljmd_allpairs_mode",
     "ljmd_check", "ljmd_pair_accel", "ljmd_run_blocked", "ljmd_virial", "ljmd_run_virial",
-    "ljmd_gr_hist_rmax", "ljmd_density_modes",
+    "ljmd_gr_hist_rmax", "ljmd_density_modes", "ljmd_bond_order", "ljmd_bond_corr",
 )
 
 
@@ -81,6 +81,8 @@ def load() -> ctypes.CDLL:
     lib.ljmd_gr_hist.argtypes = [vp, vp, i64, i32, vp, vp]
     lib.ljmd_gr_hist_rmax.argtypes = [vp, vp, i64, i32, vp, f32, vp]
     lib.ljmd_density_modes.argtypes = [vp, vp, i64, vp, i64, vp]
+    lib.ljmd_bond_order.argtypes = [vp, vp, i64, i32, f32, vp, vp]
+    lib.ljmd_bond_corr.argtypes = [vp, vp, vp, i64, i32, vp, f32, vp, vp]
     lib.ljmd_cell_geometry.argtypes = [vp, ctypes.POINTER(i32), ctypes.POINTER(i32), ctypes.POINTER(i32),
                                        ctypes.POINTER(f32), ctypes.POINTER(f32)]
     lib.ljmd_cell_assign.argtypes = [vp, vp, vp, vp]

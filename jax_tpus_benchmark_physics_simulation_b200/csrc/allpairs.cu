@@ -931,10 +931,18 @@ constexpr int GR_THREADS = 256;
 constexpr int GR_TILE    = 256;
 constexpr int GR_MAXBINS = LJMD_GR_MAXBINS;
 
+// W: byte offset of the CTA's 64-bit weight sums, after gr_hist_kernel's other shared arrays (8-aligned)
+__host__ __device__ constexpr size_t gr_wsum_offset(int nbins) {
+    return (sizeof(float2) * GR_TILE + sizeof(float) * (2 * (size_t)nbins + 1) + 7) / 8 * 8;
+}
+
+// W (ljmd_bond_corr): a counted pair with a finite weight w_ij (bond_pair_weight) also adds llrint(w 2^24) to
+// wsum; a pair whose weight is not finite is neither counted nor summed.  psi (S,N) in particle order.
+template <bool W>
 __global__ void __launch_bounds__(GR_THREADS)
 gr_hist_kernel(const float2* __restrict__ Rh, int N, float box, float timg, int nbins,
                const float* __restrict__ edges, unsigned long long* __restrict__ counts,
-               int ntile, float cap) {
+               int ntile, float cap, const double2* __restrict__ psi, unsigned long long* __restrict__ wsum) {
     // blockIdx.x -> (tile_i <= tile_j) upper-triangular tile pair; blockIdx.y -> snapshot
     // cap: pairs with r > cap are dropped as well (ljmd_gr_hist_rmax); +INFINITY for ljmd_gr_hist
     extern __shared__ unsigned char smem_raw[];
@@ -946,6 +954,12 @@ gr_hist_kernel(const float2* __restrict__ Rh, int N, float box, float timg, int 
     while (t >= ntile - ti) { t -= ntile - ti; ++ti; }
     const int tj = ti + t;
     const float2* R = Rh + (size_t)blockIdx.y * N;
+    unsigned long long* swsum = nullptr;
+    if constexpr (W) {
+        swsum = reinterpret_cast<unsigned long long*>(smem_raw + gr_wsum_offset(nbins));   // nbins
+        psi += (size_t)blockIdx.y * N;
+        for (int k = tid; k < nbins; k += GR_THREADS) swsum[k] = 0ull;
+    }
     for (int k = tid; k <= nbins; k += GR_THREADS) sedges[k] = edges[k];
     for (int k = tid; k < nbins; k += GR_THREADS) shist[k] = 0u;
     {
@@ -956,6 +970,8 @@ gr_hist_kernel(const float2* __restrict__ Rh, int N, float box, float timg, int 
     const int i = ti * GR_TILE + tid;
     if (i < N) {
         const float2 ri = R[i];
+        double2 pi = make_double2(0.0, 0.0);
+        if constexpr (W) pi = psi[i];
         const float lo = sedges[0], hi = fminf(sedges[nbins], cap);
         const float scale = (float)nbins / (sedges[nbins] - lo);
         for (int q = 0; q < GR_TILE; ++q) {
@@ -966,6 +982,11 @@ gr_hist_kernel(const float2* __restrict__ Rh, int N, float box, float timg, int 
             const float r = __fsqrt_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)));
             const int b = gr_bin(r, sedges, nbins, lo, hi, scale);          // numpy drops outliers
             if (b < 0) continue;
+            if constexpr (W) {
+                long long wq;
+                if (!bond_pair_weight(pi, psi[j], wq)) continue;
+                atomicAdd(&swsum[b], (unsigned long long)wq);
+            }
             atomicAdd(&shist[b], 1u);
         }
     }
@@ -973,6 +994,11 @@ gr_hist_kernel(const float2* __restrict__ Rh, int N, float box, float timg, int 
     unsigned long long* out = counts + (size_t)blockIdx.y * nbins;
     for (int k = tid; k < nbins; k += GR_THREADS)
         if (shist[k]) atomicAdd(&out[k], (unsigned long long)shist[k]);
+    if constexpr (W) {
+        unsigned long long* wout = wsum + (size_t)blockIdx.y * nbins;
+        for (int k = tid; k < nbins; k += GR_THREADS)
+            if (swsum[k]) atomicAdd(&wout[k], swsum[k]);
+    }
 }
 
 }  // namespace
@@ -1410,22 +1436,28 @@ int ap_check_error(ljmd_handle* h) {
 }
 
 int ap_gr_hist(ljmd_handle* h, const float2* R_hist, long long S, int nbins, const float* edges,
-               float cap, long long* counts) {
+               float cap, long long* counts, const double2* psi, long long* wsum) {
     const int N = (int)h->p.N;
+    const bool W = psi != nullptr;
     if (nbins < 1 || nbins > GR_MAXBINS) { set_error("g(r): nbins must be in [1,%d]", GR_MAXBINS); return LJMD_E_INVALID; }
     cudaStream_t st = h->stream;
     LJ_CUDA(cudaMemsetAsync(counts, 0, sizeof(long long) * S * nbins, st));
+    if (W) LJ_CUDA(cudaMemsetAsync(wsum, 0, sizeof(long long) * S * nbins, st));
     if (S == 0) return 0;
     const int ntile = (N + GR_TILE - 1) / GR_TILE;
     const long long npairs = (long long)ntile * (ntile + 1) / 2;
-    const size_t smem = sizeof(float) * (nbins + 1) + sizeof(unsigned) * nbins + sizeof(float2) * GR_TILE;
-    LJ_CUDA(cudaFuncSetAttribute(gr_hist_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const size_t smem = W ? gr_wsum_offset(nbins) + sizeof(long long) * nbins
+                          : sizeof(float) * (nbins + 1) + sizeof(unsigned) * nbins + sizeof(float2) * GR_TILE;
+    auto kernel = W ? gr_hist_kernel<true> : gr_hist_kernel<false>;
+    LJ_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     // grid.y is limited to 65535 snapshots per launch
     for (long long s0 = 0; s0 < S; s0 += 65535) {
         const int ns = (int)std::min<long long>(65535, S - s0);
-        gr_hist_kernel<<<dim3((unsigned)npairs, ns), GR_THREADS, smem, st>>>(
+        kernel<<<dim3((unsigned)npairs, ns), GR_THREADS, smem, st>>>(
             R_hist + (size_t)s0 * N, N, h->pc.box, h->pc.timg, nbins, edges,
-            reinterpret_cast<unsigned long long*>(counts) + (size_t)s0 * nbins, ntile, cap);
+            reinterpret_cast<unsigned long long*>(counts) + (size_t)s0 * nbins, ntile, cap,
+            W ? psi + (size_t)s0 * N : nullptr,
+            W ? reinterpret_cast<unsigned long long*>(wsum) + (size_t)s0 * nbins : nullptr);
         LJ_CUDA(cudaGetLastError());
         h->launches++;
     }

@@ -269,6 +269,45 @@ int ljmd_density_modes(ljmd_t* h, const float* R_hist, int64_t S, const int32_t*
                             reinterpret_cast<double2*>(rho));
 }
 
+int ljmd_bond_order(ljmd_t* h, const float* R_hist, int64_t S, int32_t m, float r_nb, double* psi, int32_t* nnb) {
+    if (!h) { set_error("ljmd_bond_order: null handle"); return LJMD_E_INVALID; }
+    if (S < 0) { set_error("ljmd_bond_order: S must be >= 0"); return LJMD_E_INVALID; }
+    if (m < 1 || m > 12) { set_error("ljmd_bond_order: m must be in [1,12]"); return LJMD_E_INVALID; }
+    if (!(r_nb > 0.0f) || !std::isfinite(r_nb)) { set_error("ljmd_bond_order: r_nb must be positive and finite"); return LJMD_E_INVALID; }
+    // with S == 0 there is nothing to read or write: the arrays may then be NULL (empty)
+    if (S == 0) return 0;
+    if (!R_hist || !psi) { set_error("ljmd_bond_order: null argument"); return LJMD_E_INVALID; }
+    if ((uintptr_t)R_hist % 8 || (uintptr_t)psi % 16 || (uintptr_t)nnb % 4) {
+        set_error("ljmd_bond_order: R_hist must be 8-byte aligned, psi 16-byte aligned, nnb 4-byte aligned");
+        return LJMD_E_INVALID;
+    }
+    LJ_CUDA(cudaSetDevice(h->p.device));
+    return bond_order(h, reinterpret_cast<const float2*>(R_hist), S, m, r_nb, reinterpret_cast<double2*>(psi), nnb);
+}
+
+int ljmd_bond_corr(ljmd_t* h, const float* R_hist, const double* psi, int64_t S, int32_t nbins,
+                   const float* edges, float r_max, int64_t* counts, int64_t* wsum) {
+    if (!h) { set_error("ljmd_bond_corr: null handle"); return LJMD_E_INVALID; }
+    if (S < 0) { set_error("ljmd_bond_corr: S must be >= 0"); return LJMD_E_INVALID; }
+    if (nbins < 1 || nbins > LJMD_GR_MAXBINS) { set_error("ljmd_bond_corr: nbins must be in [1,%d]", LJMD_GR_MAXBINS); return LJMD_E_INVALID; }
+    if (!(r_max > 0.0f) || !std::isfinite(r_max)) { set_error("ljmd_bond_corr: r_max must be positive and finite"); return LJMD_E_INVALID; }
+    if (S == 0) return 0;
+    if (!R_hist || !psi || !edges || !counts || !wsum) { set_error("ljmd_bond_corr: null argument"); return LJMD_E_INVALID; }
+    if ((uintptr_t)R_hist % 8 || (uintptr_t)psi % 16 || (uintptr_t)counts % 8 || (uintptr_t)wsum % 8) {
+        set_error("ljmd_bond_corr: R_hist, counts and wsum must be 8-byte aligned, psi 16-byte aligned");
+        return LJMD_E_INVALID;
+    }
+    LJ_CUDA(cudaSetDevice(h->p.device));
+    const float2* R = reinterpret_cast<const float2*>(R_hist);
+    const double2* p = reinterpret_cast<const double2*>(psi);
+    long long* c = reinterpret_cast<long long*>(counts);
+    long long* w = reinterpret_cast<long long*>(wsum);
+    // the same selection as ljmd_gr_hist_rmax, so the counts are its counts wherever every weight is finite
+    const int nc = gr_grid_side(h->p.N, h->p.box, r_max);
+    if (nc >= 3) return gr_cells_hist(h, R, S, nbins, edges, r_max, nc, c, p, w);
+    return ap_gr_hist(h, R, S, nbins, edges, r_max, c, p, w);
+}
+
 int ljmd_cell_geometry(ljmd_t* h, int32_t* nrows, int32_t* nbins_x, int32_t* kbins,
                        float* inv_row_height, float* inv_bin_width) {
     if (!h) { set_error("null handle"); return LJMD_E_INVALID; }

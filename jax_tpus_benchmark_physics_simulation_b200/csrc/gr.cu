@@ -11,6 +11,11 @@
 //   gr_cells_kernel    the half stencil of every cell into a per-CTA shared histogram
 // Snapshots are batched up to GR_BATCH_BYTES of scratch: at N = 4096 all 100 snapshots of the driver take
 // one batch (four launches per call); at N = 16 M a batch holds two.
+//
+// The same grid serves the bond order (bond.cu: the first three launches, then its own kernel) and the
+// weighted histogram g_m(r) of ljmd_bond_corr (the W instantiations).  The scatter's W instantiation also
+// records each particle's original index (bond order: 16 B of scratch per particle instead of 12) or its psi
+// in cell order (g_m(r): 28 B).
 #include "ljmd_device.cuh"
 
 #include <algorithm>
@@ -19,7 +24,7 @@
 namespace ljmd {
 
 struct Gr {
-    void*  buf = nullptr;   // cell starts | positions in cell order | ranks, for one batch of snapshots
+    void*  buf = nullptr;   // one batch of snapshots binned into the grid (GrGrid, gr_grid_alloc)
     size_t bytes = 0;
 };
 
@@ -35,15 +40,6 @@ constexpr int      GRC_CELLS       = 64;            // home cells per CTA
 // conservatively, 32 per staged target); beyond that (a clumped state) it adds to the global counts
 // directly, so the CTA's counters stay below GRC_WARPS * (2^28 + 1024) < 2^32.
 constexpr long long GRC_WARP_BUDGET = 1ll << 28;
-
-// Cell of a position in [0, box]: one fp32 multiply and truncation per axis.  The clamps keep any other
-// input (outside [0, box], non-finite) inside the grid; such pairs are then dropped by the binning or
-// counted as gr_hist_kernel would count them, as long as they are adjacent.
-__device__ __forceinline__ int gr_cell(float2 p, float inv_cell, int nc) {
-    const int cx = min(max((int)__fmul_rn(p.x, inv_cell), 0), nc - 1);
-    const int cy = min(max((int)__fmul_rn(p.y, inv_cell), 0), nc - 1);
-    return cy * nc + cx;
-}
 
 __global__ void __launch_bounds__(GRB_THREADS)
 gr_count_kernel(const float2* __restrict__ R, int N, float inv_cell, int nc, int* __restrict__ cstart,
@@ -102,15 +98,23 @@ gr_scan_kernel(int* __restrict__ cstart, long long stride, int L) {
     }
 }
 
+// W: also, where the pointers are given, the original index of every particle in cell order (idx) and its psi (Ppsi)
+template <bool W>
 __global__ void __launch_bounds__(GRB_THREADS)
 gr_scatter_kernel(const float2* __restrict__ R, int N, float inv_cell, int nc, const int* __restrict__ cstart,
-                  long long stride, const int* __restrict__ rank, float2* __restrict__ P) {
+                  long long stride, const int* __restrict__ rank, float2* __restrict__ P,
+                  int* __restrict__ idx, const double2* __restrict__ psi, double2* __restrict__ Ppsi) {
     const int i = blockIdx.x * GRB_THREADS + threadIdx.x;
     if (i >= N) return;
     const size_t s = blockIdx.y;
     const float2 r = R[s * N + i];
     const int c = gr_cell(r, inv_cell, nc);
-    P[s * N + cstart[s * stride + c] + rank[s * N + i]] = r;
+    const size_t o = s * N + cstart[s * stride + c] + rank[s * N + i];
+    P[o] = r;
+    if constexpr (W) {
+        if (idx) idx[o] = i;
+        if (psi) Ppsi[o] = psi[s * N + i];
+    }
 }
 
 struct GrCellsArgs {
@@ -121,12 +125,22 @@ struct GrCellsArgs {
     float box, timg, cap;
     const float* edges;           // nbins + 1
     unsigned long long* counts;   // (ns, nbins)
+    const double2* psi;           // W: (ns, N) psi in cell order
+    unsigned long long* wsum;     // W: (ns, nbins) sums of llrint(w 2^24) (two's complement)
 };
+
+// W: byte offset of the CTA's 64-bit weight sums, after the pair kernel's other shared arrays (8-aligned)
+__host__ __device__ constexpr size_t grc_wsum_offset(int nbins) {
+    return (sizeof(float2) * GRC_WARPS * 32 + sizeof(float) * (2 * (size_t)nbins + 1) + 7) / 8 * 8;
+}
 
 // One warp per home cell c: its particles, 32 at a time one per lane, against the targets of the half
 // stencil - c itself (j > i), E, NE, N and NW, periodic - staged 32 at a time in the warp's shared slots.
 // Cells of any occupancy are walked in these chunks.  For nc >= 3 the five cells are distinct and every
 // unordered pair of particles in adjacent cells is visited exactly once.
+// W (ljmd_bond_corr): a counted pair with a finite weight w_ij (bond_pair_weight) also adds llrint(w 2^24) to
+// wsum; a pair whose weight is not finite is neither counted nor summed.
+template <bool W>
 __global__ void __launch_bounds__(GRC_THREADS)
 gr_cells_kernel(const GrCellsArgs a) {
     extern __shared__ unsigned char smem_raw[];
@@ -139,6 +153,15 @@ gr_cells_kernel(const GrCellsArgs a) {
     const float2* P = a.P + s * a.N;
     const int* cs = a.cstart + s * a.stride;
     unsigned long long* out = a.counts + s * nbins;
+    unsigned long long* swsum = nullptr;
+    unsigned long long* wout = nullptr;
+    const double2* psi = nullptr;
+    if constexpr (W) {
+        swsum = reinterpret_cast<unsigned long long*>(smem_raw + grc_wsum_offset(nbins));   // nbins
+        wout = a.wsum + s * nbins;
+        psi = a.psi + s * a.N;
+        for (int k = tid; k < nbins; k += GRC_THREADS) swsum[k] = 0ull;
+    }
     for (int k = tid; k <= nbins; k += GRC_THREADS) sedges[k] = a.edges[k];
     for (int k = tid; k < nbins; k += GRC_THREADS) shist[k] = 0u;
     __syncthreads();
@@ -156,6 +179,8 @@ gr_cells_kernel(const GrCellsArgs a) {
             const int i = ib + lane;
             const bool has_i = i < a1;
             const float2 ri = has_i ? P[i] : make_float2(0.0f, 0.0f);
+            double2 pi = make_double2(0.0, 0.0);
+            if constexpr (W) pi = has_i ? psi[i] : pi;
             for (int t = 0; t < 5; ++t) {
                 int b0 = ib, b1 = a1;                                       // t == 0: own cell, j > i
                 if (t > 0) {
@@ -179,6 +204,12 @@ gr_cells_kernel(const GrCellsArgs a) {
                         const float r = __fsqrt_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)));
                         const int b = gr_bin(r, sedges, nbins, lo, hi, scale);
                         if (b < 0) continue;
+                        if constexpr (W) {
+                            long long wq;
+                            if (!bond_pair_weight(pi, psi[jb + q], wq)) continue;
+                            if (direct) atomicAdd(&wout[b], (unsigned long long)wq);
+                            else        atomicAdd(&swsum[b], (unsigned long long)wq);
+                        }
                         if (direct) atomicAdd(&out[b], 1ull);
                         else        atomicAdd(&shist[b], 1u);
                     }
@@ -189,6 +220,10 @@ gr_cells_kernel(const GrCellsArgs a) {
     __syncthreads();
     for (int k = tid; k < nbins; k += GRC_THREADS)
         if (shist[k]) atomicAdd(&out[k], (unsigned long long)shist[k]);
+    if constexpr (W) {
+        for (int k = tid; k < nbins; k += GRC_THREADS)
+            if (swsum[k]) atomicAdd(&wout[k], swsum[k]);
+    }
 }
 
 }  // namespace
@@ -215,55 +250,89 @@ int gr_grid_side(long long N, float box, float r_max) {
     return (int)std::max<long long>(0, std::min(nc, cap));
 }
 
-int gr_cells_hist(ljmd_handle* h, const float2* R_hist, long long S, int nbins, const float* edges,
-                  float r_max, int nc, long long* counts) {
+int gr_grid_alloc(ljmd_handle* h, long long S, int nc, bool with_idx, bool with_psi, GrGrid* g) {
     const long long N = h->p.N;
-    cudaStream_t st = h->stream;
-    LJ_CUDA(cudaMemsetAsync(counts, 0, sizeof(long long) * S * nbins, st));
-    if (S == 0) return 0;
     const long long ncell = (long long)nc * nc;
     const long long stride = (ncell + 1 + 3) / 4 * 4;                       // int4-aligned rows of cell starts
-    const size_t per = sizeof(int) * stride + (sizeof(float2) + sizeof(int)) * (size_t)N;
+    const size_t extra = (with_psi ? sizeof(double2) : 0) + (with_idx ? sizeof(int) : 0);
+    const size_t per = sizeof(int) * stride + (sizeof(float2) + sizeof(int) + extra) * (size_t)N;
     const long long nb = std::max<long long>(1, std::min<long long>(std::min<long long>(S, 65535),
                                                                     (long long)(GR_BATCH_BYTES / per)));
     const size_t need = per * (size_t)nb;
     if (!h->gr) h->gr = new Gr();
-    Gr* g = h->gr;
-    if (g->bytes < need) {
-        LJ_CUDA(cudaFree(g->buf));
-        g->buf = nullptr;
-        g->bytes = 0;
-        LJ_CUDA(cudaMalloc(&g->buf, need));
-        g->bytes = need;
+    Gr* b = h->gr;
+    if (b->bytes < need) {
+        LJ_CUDA(cudaFree(b->buf));
+        b->buf = nullptr;
+        b->bytes = 0;
+        LJ_CUDA(cudaMalloc(&b->buf, need));
+        b->bytes = need;
     }
-    int* cs = reinterpret_cast<int*>(g->buf);
-    float2* P = reinterpret_cast<float2*>(cs + nb * stride);
-    int* rank = reinterpret_cast<int*>(P + nb * N);
+    // cell starts (rows of 16 B) | psi (with_psi) | positions | ranks | original indices (with_idx)
+    g->cs = reinterpret_cast<int*>(b->buf);
+    double2* after_cs = reinterpret_cast<double2*>(g->cs + nb * stride);
+    g->psi = with_psi ? after_cs : nullptr;
+    g->P = reinterpret_cast<float2*>(with_psi ? after_cs + nb * N : after_cs);
+    g->rank = reinterpret_cast<int*>(g->P + nb * N);
+    g->idx = with_idx ? g->rank + nb * N : nullptr;
+    g->stride = stride;
+    g->nb = nb;
+    g->nc = nc;
+    g->inv_cell = (float)nc / h->p.box;
+    return 0;
+}
+
+int gr_grid_bin(ljmd_handle* h, const GrGrid& g, const float2* R, const double2* psi, unsigned ns) {
+    const long long N = h->p.N;
+    cudaStream_t st = h->stream;
+    const long long ncell = (long long)g.nc * g.nc;
+    const unsigned pblocks = (unsigned)((N + GRB_THREADS - 1) / GRB_THREADS);
+    LJ_CUDA(cudaMemsetAsync(g.cs, 0, sizeof(int) * g.stride * ns, st));
+    gr_count_kernel<<<dim3(pblocks, ns), GRB_THREADS, 0, st>>>(R, (int)N, g.inv_cell, g.nc, g.cs, g.stride, g.rank);
+    LJ_CUDA(cudaGetLastError());
+    gr_scan_kernel<<<dim3(1, ns), GRS_THREADS, 0, st>>>(g.cs, g.stride, (int)(ncell + 1));
+    LJ_CUDA(cudaGetLastError());
+    if (g.idx || g.psi)
+        gr_scatter_kernel<true><<<dim3(pblocks, ns), GRB_THREADS, 0, st>>>(R, (int)N, g.inv_cell, g.nc, g.cs, g.stride,
+                                                                          g.rank, g.P, g.idx, psi, g.psi);
+    else
+        gr_scatter_kernel<false><<<dim3(pblocks, ns), GRB_THREADS, 0, st>>>(R, (int)N, g.inv_cell, g.nc, g.cs, g.stride,
+                                                                           g.rank, g.P, nullptr, nullptr, nullptr);
+    LJ_CUDA(cudaGetLastError());
+    h->launches += 3;
+    return 0;
+}
+
+int gr_cells_hist(ljmd_handle* h, const float2* R_hist, long long S, int nbins, const float* edges,
+                  float r_max, int nc, long long* counts, const double2* psi, long long* wsum) {
+    const long long N = h->p.N;
+    const bool W = psi != nullptr;
+    cudaStream_t st = h->stream;
+    LJ_CUDA(cudaMemsetAsync(counts, 0, sizeof(long long) * S * nbins, st));
+    if (W) LJ_CUDA(cudaMemsetAsync(wsum, 0, sizeof(long long) * S * nbins, st));
+    if (S == 0) return 0;
+    GrGrid g;
+    if (int e = gr_grid_alloc(h, S, nc, false, W, &g)) return e;
 
     GrCellsArgs a{};
-    a.P = P; a.cstart = cs; a.stride = stride;
+    a.P = g.P; a.cstart = g.cs; a.stride = g.stride;
     a.N = (int)N; a.nc = nc; a.nbins = nbins;
     a.box = h->pc.box; a.timg = h->pc.timg; a.cap = r_max;
     a.edges = edges;
-    const float inv_cell = (float)nc / h->p.box;
-    const size_t smem = sizeof(float2) * GRC_WARPS * 32 + sizeof(float) * (nbins + 1) + sizeof(unsigned) * nbins;
-    LJ_CUDA(cudaFuncSetAttribute(gr_cells_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    const unsigned pblocks = (unsigned)((N + GRB_THREADS - 1) / GRB_THREADS);
-    const unsigned cblocks = (unsigned)((ncell + GRC_CELLS - 1) / GRC_CELLS);
-    for (long long s0 = 0; s0 < S; s0 += nb) {
-        const unsigned ns = (unsigned)std::min(nb, S - s0);
-        const float2* R = R_hist + (size_t)s0 * N;
-        LJ_CUDA(cudaMemsetAsync(cs, 0, sizeof(int) * stride * ns, st));
-        gr_count_kernel<<<dim3(pblocks, ns), GRB_THREADS, 0, st>>>(R, (int)N, inv_cell, nc, cs, stride, rank);
-        LJ_CUDA(cudaGetLastError());
-        gr_scan_kernel<<<dim3(1, ns), GRS_THREADS, 0, st>>>(cs, stride, (int)(ncell + 1));
-        LJ_CUDA(cudaGetLastError());
-        gr_scatter_kernel<<<dim3(pblocks, ns), GRB_THREADS, 0, st>>>(R, (int)N, inv_cell, nc, cs, stride, rank, P);
-        LJ_CUDA(cudaGetLastError());
+    a.psi = g.psi;
+    const size_t smem = W ? grc_wsum_offset(nbins) + sizeof(long long) * nbins
+                          : sizeof(float2) * GRC_WARPS * 32 + sizeof(float) * (nbins + 1) + sizeof(unsigned) * nbins;
+    void (*kernel)(const GrCellsArgs) = W ? gr_cells_kernel<true> : gr_cells_kernel<false>;
+    LJ_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const unsigned cblocks = (unsigned)(((long long)nc * nc + GRC_CELLS - 1) / GRC_CELLS);
+    for (long long s0 = 0; s0 < S; s0 += g.nb) {
+        const unsigned ns = (unsigned)std::min(g.nb, S - s0);
+        if (int e = gr_grid_bin(h, g, R_hist + (size_t)s0 * N, W ? psi + (size_t)s0 * N : nullptr, ns)) return e;
         a.counts = reinterpret_cast<unsigned long long*>(counts) + (size_t)s0 * nbins;
-        gr_cells_kernel<<<dim3(cblocks, ns), GRC_THREADS, smem, st>>>(a);
+        if (W) a.wsum = reinterpret_cast<unsigned long long*>(wsum) + (size_t)s0 * nbins;
+        kernel<<<dim3(cblocks, ns), GRC_THREADS, smem, st>>>(a);
         LJ_CUDA(cudaGetLastError());
-        h->launches += 4;
+        h->launches += 1;
     }
     return 0;
 }

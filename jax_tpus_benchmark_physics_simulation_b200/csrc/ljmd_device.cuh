@@ -42,6 +42,26 @@ __device__ __forceinline__ int gr_bin(float r, const float* e, int nbins, float 
     return b;
 }
 
+// Cell of a position in [0, box] on the periodic nc x nc grid of g(r) and the bond order (gr.cu, bond.cu): one
+// fp32 multiply and truncation per axis.  The clamps keep any other input (outside [0, box], non-finite)
+// inside the grid; such pairs are then dropped by the binning or counted as gr_hist_kernel would count
+// them, as long as they are adjacent.
+__device__ __forceinline__ int gr_cell(float2 p, float inv_cell, int nc) {
+    const int cx = min(max((int)__fmul_rn(p.x, inv_cell), 0), nc - 1);
+    const int cy = min(max((int)__fmul_rn(p.y, inv_cell), 0), nc - 1);
+    return cy * nc + cx;
+}
+
+// Weight of a pair in the g_m(r) histogram (ljmd_bond_corr): w = Re psi_i Re psi_j + Im psi_i Im psi_j, each
+// operation rounded once, added as the integer llrint(w 2^24) (exact and order-free).  false: w is not
+// finite and the pair is skipped.
+__device__ __forceinline__ bool bond_pair_weight(double2 pi, double2 pj, long long& q) {
+    const double w = __dadd_rn(__dmul_rn(pi.x, pj.x), __dmul_rn(pi.y, pj.y));
+    if (!isfinite(w)) return false;
+    q = llrint(__dmul_rn(w, 16777216.0));
+    return true;
+}
+
 // One ordered pair (i <- j) of total_energy_fn / force_fn (MD:50-64):
 //   r2 = dx^2 + dy^2 with each operation rounded once (no FMA contraction), so the pair set
 //   {r2 < rc2} is decided on the same fp32 r2 as the CPU restatement;

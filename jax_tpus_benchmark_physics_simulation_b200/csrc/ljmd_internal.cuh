@@ -78,7 +78,7 @@ struct ljmd_handle {
     ljmd::AllPairs*  ap;
     ljmd::Cells*     cells;
     ljmd::Dist*      dist;
-    ljmd::Gr*        gr;          // cell-grid g(r) scratch (allocated on the first ljmd_gr_hist_rmax that uses it)
+    ljmd::Gr*        gr;          // cell-grid scratch of g(r), psi_m and g_m(r) (allocated on the first call that uses it)
     cudaEvent_t      ev0, ev1;
     bool             timed;
     long long        launches;
@@ -101,8 +101,9 @@ int  ap_run(ljmd_handle* h, const float2* R_in, const float2* V_in, float2* R_ou
 int  ap_check_error(ljmd_handle* h);
 int  ap_mode(ljmd_handle* h);
 // cap: pairs with r > cap are dropped too (+INFINITY: the plain histogram of ljmd_gr_hist)
+// psi != nullptr: the weighted histogram of ljmd_bond_corr (psi (S,N) in particle order, wsum (S,nbins))
 int  ap_gr_hist(ljmd_handle* h, const float2* R_hist, long long S, int nbins, const float* edges,
-                float cap, long long* counts);
+                float cap, long long* counts, const double2* psi = nullptr, long long* wsum = nullptr);
 
 // cells.cu
 int  cells_create(ljmd_handle* h);
@@ -117,9 +118,29 @@ int  cells_check_error(ljmd_handle* h);
 
 // gr.cu: g(r) through a periodic nc x nc cell grid of edge >= r_max (see ljmd_gr_hist_rmax)
 int  gr_grid_side(long long N, float box, float r_max);   // nc for this r_max (the grid is used when >= 3)
+// psi != nullptr: the weighted histogram of ljmd_bond_corr (psi (S,N) in particle order, wsum (S,nbins))
 int  gr_cells_hist(ljmd_handle* h, const float2* R_hist, long long S, int nbins, const float* edges,
-                   float r_max, int nc, long long* counts);
+                   float r_max, int nc, long long* counts, const double2* psi = nullptr, long long* wsum = nullptr);
+// One batch of snapshots binned into the nc x nc grid, in the handle's Gr scratch (rows of the batch: nb).
+// with_idx: also idx (original index of each particle in cell order, for the bond order);
+// with_psi: also psi (its psi in cell order, for the weighted histogram of ljmd_bond_corr).
+struct GrGrid {
+    int*      cs;        // (nb, stride) cell starts; cs[c + 1] - cs[c] particles in cell c
+    float2*   P;         // (nb, N) positions in cell order
+    int*      rank;      // (nb, N) rank of each particle in its cell
+    int*      idx;       // with_idx: (nb, N) original index in cell order, else nullptr
+    double2*  psi;       // with_psi: (nb, N) psi in cell order, else nullptr
+    long long stride, nb;
+    int       nc;
+    float     inv_cell;  // fl(nc / box), the multiplier of gr_cell
+};
+int  gr_grid_alloc(ljmd_handle* h, long long S, int nc, bool with_idx, bool with_psi, GrGrid* g);
+// count / scan / scatter of ns <= nb snapshots R (ns, N); psi (ns, N) is permuted too when given (with_psi)
+int  gr_grid_bin(ljmd_handle* h, const GrGrid& g, const float2* R, const double2* psi, unsigned ns);
 void gr_destroy(ljmd_handle* h);
+
+// bond.cu: bond-orientational order psi_m of every particle (see ljmd_bond_order)
+int  bond_order(ljmd_handle* h, const float2* R_hist, long long S, int m, float r_nb, double2* psi, int* nnb);
 
 // sk.cu: density modes rho_k of S snapshots for K integer wave vectors (see ljmd_density_modes)
 int  sk_density_modes(ljmd_handle* h, const float2* R_hist, long long S, const int2* nvec, long long K,

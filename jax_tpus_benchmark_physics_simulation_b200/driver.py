@@ -12,7 +12,9 @@ parity tests and bench.py use), ``--energy_every``, ``--pressure`` (records the 
 energy rows and reports the mean and spread of P over the production), ``--gr_rmax`` (largest r of
 g(r); default box/2 as the reference, a few sigma for millions of particles), ``--sk_kmax`` /
 ``--sk_per_shell`` (the static structure factor S(k) of the production snapshots up to |k| = sk_kmax,
-default off; written as ``<stem>_sk.npy``/``.csv`` next to ``--output``).  matplotlib is imported
+default off; written as ``<stem>_sk.npy``/``.csv`` next to ``--output``), ``--bond_m`` / ``--bond_rnb``
+(the bond-orientational order psi_M of the production snapshots and its pair correlation g_M(r) on g(r)'s
+bins, default off; written as ``<stem>_psi{M}.npy`` and ``<stem>_g{M}.npy``/``.csv``).  matplotlib is imported
 lazily (absent in this image): without it g(r) is written as ``.npy``/``.csv`` next to
 ``--output``.
 """
@@ -81,6 +83,18 @@ def main(args):
         sk = (np.asarray(k_sk), np.asarray(S_sk))
         print(f"S(k) calculation complete in {time_sk:.2f} s")
 
+    bond = None
+    if args.bond_m is not None:
+        M = args.bond_m
+        print(f"\n--- Calculating psi_{M} ---")
+        start_time_bond = time.time()
+        r_b, g_b = sim.bond_correlation(R_history, r_max_g, nbins_g, M, args.bond_rnb)
+        g_b.block_until_ready()
+        Psi = sim.last_bond_global.numpy()                                     # (S, 2): Psi_M of each snapshot
+        time_bond = time.time() - start_time_bond
+        bond = (np.asarray(r_b), np.asarray(g_b), Psi)
+        print(f"psi_{M} calculation complete in {time_bond:.2f} s")
+
     print("\nSimulation Summary")
     print(f"  Equilibration  {time_eq:8.2f} s   {args.eq_steps:,} steps")
     print(f"  Production     {time_prod:8.2f} s   {args.prod_steps:,} steps")
@@ -92,7 +106,14 @@ def main(args):
             print(f"  S(k) first peak: k = {sk[0][i]:.4f}  S = {sk[1][i]:.4f}")
         else:
             print("  S(k) first peak: none (S(k) is not finite)")
-    total = time_eq + time_prod + time_g_r + (time_sk if sk is not None else 0.0)
+    if bond is not None:
+        mag = np.hypot(bond[2][:, 0], bond[2][:, 1])
+        print(f"  psi_{M} Analysis {time_bond:7.2f} s   r_nb = {args.bond_rnb}, g_{M}(r) on {bond[0].size} bins")
+        if mag.size:
+            chi = N * (np.mean(mag ** 2) - np.mean(mag) ** 2)
+            print(f"  <|Psi_{M}|> = {np.mean(mag):.6f}  chi_{M} = {chi:.6f}  over {mag.size} snapshots")
+    total = (time_eq + time_prod + time_g_r + (time_sk if sk is not None else 0.0)
+             + (time_bond if bond is not None else 0.0))
     print(f"  Total          {total:8.2f} s")
     if sim.last_energies is not None:
         e = sim.last_energies.numpy()
@@ -120,6 +141,12 @@ def main(args):
         np.save(stem + ".npy", np.stack([r_np, g_np]))
         np.savetxt(stem + ".csv", np.stack([r_np, g_np], axis=1), delimiter=",", header="r,g_r")
         print(f"matplotlib unavailable: g(r) saved as '{stem}.npy' and '{stem}.csv'")
+    if bond is not None:
+        stem = args.output.rsplit(".", 1)[0]
+        np.save(f"{stem}_psi{M}.npy", bond[2])
+        np.save(f"{stem}_g{M}.npy", np.stack(bond[:2]))
+        np.savetxt(f"{stem}_g{M}.csv", np.stack(bond[:2], axis=1), delimiter=",", header=f"r,g_{M}")
+        print(f"psi_{M} saved as '{stem}_psi{M}.npy', g_{M}(r) as '{stem}_g{M}.npy' and '{stem}_g{M}.csv'")
     if sk is not None:
         stem = args.output.rsplit(".", 1)[0] + "_sk"
         np.save(stem + ".npy", np.stack(sk))
@@ -159,6 +186,13 @@ def build_parser():
     parser.add_argument("--sk_per_shell", type=int, default=None,
                         help="with --sk_kmax: at most this many wave vectors per shell floor(|n|), evenly "
                              "spread in angle (default: all)")
+    parser.add_argument("--bond_m", type=int, default=None,
+                        help="compute the bond-orientational order psi_M (M in [1, 12]; 6 for 2-D melting, 4 for the "
+                             "square lattice) of the production snapshots and its pair correlation g_M(r) on "
+                             "g(r)'s bins (default: off)")
+    parser.add_argument("--bond_rnb", type=float, default=1.5,
+                        help="with --bond_m: neighbour radius of psi_M (default: 1.5, the conventional first "
+                             "minimum of g(r))")
     return parser
 
 
@@ -173,6 +207,10 @@ def parse_args(argv=None):
         parser.error("--sk_kmax must be positive and finite")
     if args.sk_per_shell is not None and args.sk_per_shell < 1:
         parser.error("--sk_per_shell must be >= 1")
+    if args.bond_m is not None and not 1 <= args.bond_m <= 12:
+        parser.error("--bond_m must be in [1, 12]")
+    if not (args.bond_rnb > 0 and np.isfinite(args.bond_rnb)):
+        parser.error("--bond_rnb must be positive and finite")
     return args
 
 

@@ -400,6 +400,63 @@ class LJSimulation:
         return (self._arr(torch.from_numpy(k).to(self.device)),
                 self._arr(torch.from_numpy(S_k).to(self.device)))
 
+    # ------------------------------------------------------------------ bond order psi_m (new)
+    def _snapshots(self, R_history) -> torch.Tensor:
+        Rh = self._dev(R_history)
+        if Rh.dim() == 2:
+            Rh = Rh[None]
+        if Rh.dim() != 3 or tuple(Rh.shape[1:]) != (self.N, 2):
+            raise ValueError(f"expected snapshots of shape (S, {self.N}, 2), got {tuple(Rh.shape)}")
+        return Rh
+
+    def bond_order(self, R_history, m: int = 6, r_nb: float = 1.5):
+        """Bond-orientational order psi_m(i) = (1/n_i) sum_{j: 0 < r_ij <= r_nb} exp(i m theta_ij) of every particle
+        of the snapshots R_history (S, N, 2) (or one (N, 2) state): (psi (S, N, 2) float64 = (Re, Im), n (S, N)
+        int32) device arrays (ljmd_bond_order; neighbour rule, fixed-point bound and NaN rule in include/ljmd.h).
+        r_nb = 1.5 sigma is the conventional first minimum of g(r) of this fluid (a default, not a measured
+        value).  The per-snapshot mean Psi_m = (1/N) sum_i psi_i is kept as ``last_bond_global`` (S, 2)."""
+        Rh = self._snapshots(R_history)
+        S = Rh.shape[0]
+        psi = torch.empty((S, self.N, 2), dtype=torch.float64, device=self.device)
+        nnb = torch.empty((S, self.N), dtype=torch.int32, device=self.device)
+        self._check_stream()
+        _lib.check(self.lib.ljmd_bond_order(self._h, Rh.data_ptr() if S else None, S, int(m), float(r_nb),
+                                            psi.data_ptr() if S else None, nnb.data_ptr() if S else None),
+                   "ljmd_bond_order")
+        self._after()
+        self.last_bond_global = self._arr(psi.mean(dim=1))
+        return self._arr(psi), self._arr(nnb)
+
+    def bond_correlation(self, R_history, r_max, nbins: Optional[int] = None, m: int = 6, r_nb: float = 1.5):
+        """Pair correlation of the bond order g_m(r) = <psi_m(i) psi_m(j)*> over the pairs at distance r, on
+        calculate_g_r's fp32 bins linspace(0, r_max, nbins + 1) (nbins defaults to int(r_max / 0.05)).  Returns
+        (centers, g_m) device arrays; g_m = sum_s wsum / (2^24 sum_s counts) (ljmd_bond_corr), NaN in an empty bin.
+        The per-snapshot ``last_bond_counts`` / ``last_bond_wsum`` (S, nbins) int64 are kept, and psi_m as
+        ``bond_order`` keeps it.  Raises LjmdError if a count reaches 2^38, where wsum would stop being exact."""
+        r_max = np.float32(r_max)
+        nbins = int(r_max / 0.05) if nbins is None else int(nbins)
+        Rh = self._snapshots(R_history)
+        S = Rh.shape[0]
+        psi = self.bond_order(Rh, m, r_nb)[0].tensor
+        r_bins = np.linspace(0, r_max, nbins + 1, dtype=np.float32)              # as calculate_g_r
+        centers = (r_bins[:-1] + r_bins[1:]) / np.float32(2.0)
+        edges = torch.from_numpy(r_bins).to(self.device)
+        counts = torch.empty((S, nbins), dtype=torch.int64, device=self.device)
+        wsum = torch.empty((S, nbins), dtype=torch.int64, device=self.device)
+        self._check_stream()
+        _lib.check(self.lib.ljmd_bond_corr(self._h, Rh.data_ptr() if S else None, psi.data_ptr() if S else None, S,
+                                           nbins, edges.data_ptr(), float(r_bins[-1]),
+                                           counts.data_ptr() if S else None, wsum.data_ptr() if S else None),
+                   "ljmd_bond_corr")
+        self._after()
+        self.last_bond_counts, self.last_bond_wsum = self._arr(counts), self._arr(wsum)
+        if S and int(counts.max()) >= 1 << 38:
+            raise _lib.LjmdError("ljmd_bond_corr: a bin count reached 2^38, beyond which wsum is not exact")
+        c = counts.to(torch.float64).sum(dim=0)
+        g = wsum.to(torch.float64).sum(dim=0) / (c * float(1 << 24))
+        g = torch.where(c > 0, g, torch.full_like(g, float("nan")))
+        return self._arr(torch.from_numpy(centers).to(self.device)), self._arr(g)
+
     # ------------------------------------------------------------------ cell-list introspection
     def cell_geometry(self):
         """(nrows, nbins_x, kbins, inv_row_height, inv_bin_width) of the strip-cell grid."""
