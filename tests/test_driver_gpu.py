@@ -59,10 +59,14 @@ def test_reference_defaults_match_parser():
 
 
 @pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs")
-def test_sharded_allpairs_matches_single_gpu():
+@pytest.mark.parametrize("N,port", [(16384, 29541), (3364, 29545), (4356, 29547)])
+def test_sharded_allpairs_matches_single_gpu(N, port):
+    """N = 16384: the tile mode on 8192 particles per rank.  N = 3364 = 58^2: 1682 < 2048 per rank, so the ordered
+    ipt 2 kernel with a partly filled i-block.  N = 4356 = 66^2: 2178 per rank, the tile mode with a partly filled
+    last 64-particle block."""
     cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", "2",
-           "--master-addr", "127.0.0.1", "--master-port", "29541",
-           os.path.join(ROOT, "scripts", "dist_check.py"), "16384", "30"]
+           "--master-addr", "127.0.0.1", "--master-port", str(port),
+           os.path.join(ROOT, "scripts", "dist_check.py"), str(N), "30"]
     r = subprocess.run(cmd, capture_output=True, text=True, timeout=600, cwd=ROOT)
     assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-3000:]
     assert r.stdout.count("-> OK") == 2
