@@ -205,6 +205,35 @@ int ljmd_bond_order(ljmd_t* h, const float* R_hist, int64_t S, int32_t m, float 
 int ljmd_bond_corr(ljmd_t* h, const float* R_hist, const double* psi, int64_t S, int32_t nbins,
                    const float* edges, float r_max, int64_t* counts, int64_t* wsum);
 
+/* ---- cluster analysis (new; the reference has none - see DESIGN.md) ------------------------------------------ */
+/* Connected components ("clusters") of the link graph of every snapshot of S.
+ * R_hist: device (S,N,2) float32 in [0, box], 8-byte aligned; mask: device uint8 (S,N) or NULL (every particle);
+ * labels: device int32 (S,N), 4-byte aligned; sizes: device int32 (S,N), 4-byte aligned, or NULL.  r_link finite
+ * and > 0.
+ *   - Active: particle i of snapshot s is active when both its coordinates are finite and, if mask is given,
+ *     mask[s*N + i] != 0.
+ *   - Link: two distinct active particles i != j are linked when r_ij <= r_link, r_ij exactly the fp32
+ *     minimum-image r that ljmd_gr_hist bins and ljmd_bond_order uses (min_image of fl(x_j - x_i), fl(dx^2),
+ *     fl(dy^2), their rounded sum, rounded sqrt).  Coincident particles (r = 0) are linked.  With every particle
+ *     active, the number of links is the ljmd_gr_hist_rmax count on edges [0, r_link].
+ *   - Clusters: the connected components of that graph, periodic through the minimum image.
+ *   - labels[s*N + i] (ORIGINAL particle order) = the smallest original index in i's cluster; -1 for an inactive
+ *     particle; an isolated active particle is its own cluster.  sizes[s*N + k] = the number of particles labelled
+ *     k: non-zero exactly at the cluster roots (labels[s*N + k] == k).
+ *   - Deterministic: the canonical label does not depend on the order of any atomic operation, so the output is
+ *     bit-identical on every run, whatever the other snapshots of the call, the batching or the handle.
+ *   - Through the periodic cell grid of ljmd_gr_hist_rmax (cells of edge >= r_link, full 9-cell stencil; one cell,
+ *     i.e. all pairs, when r_link > box / 3) and a lock-free union-find whose forest lives in labels (derivation in
+ *     csrc/cluster.cu).  Six launches per batch of snapshots (three of the grid, init, hook, flatten).  The only
+ *     scratch is the grid's (16 B per particle and snapshot, batches <= 512 MiB), allocated on first use and kept
+ *     until ljmd_destroy.
+ *   - Any handle works, the multi-GPU ones included; there is no communication: each rank computes on the
+ *     snapshots it was given.
+ * S < 0, r_link out of range, a NULL R_hist or labels, or a misaligned array: LJMD_E_INVALID.  S == 0 does nothing,
+ * and the arrays may then be NULL.                                                                               */
+int ljmd_clusters(ljmd_t* h, const float* R_hist, int64_t S, float r_link, const uint8_t* mask,
+                  int32_t* labels, int32_t* sizes);
+
 /* ---- the other dense pairwise kernels of the reference repo (SURVEY.md 8f) -------- */
 /* All-pairs acceleration with the pair law as a functor: gravity r^-3 in an open plane.
  *   LJMD_LAW_GRAVITY_NBODY  pairwise_forces(positions, masses) of nbody_bh_merger_sim (NBODY:54-67):

@@ -308,6 +308,22 @@ int ljmd_bond_corr(ljmd_t* h, const float* R_hist, const double* psi, int64_t S,
     return ap_gr_hist(h, R, S, nbins, edges, r_max, c, p, w);
 }
 
+int ljmd_clusters(ljmd_t* h, const float* R_hist, int64_t S, float r_link, const uint8_t* mask, int32_t* labels,
+                  int32_t* sizes) {
+    if (!h) { set_error("ljmd_clusters: null handle"); return LJMD_E_INVALID; }
+    if (S < 0) { set_error("ljmd_clusters: S must be >= 0"); return LJMD_E_INVALID; }
+    if (!(r_link > 0.0f) || !std::isfinite(r_link)) { set_error("ljmd_clusters: r_link must be positive and finite"); return LJMD_E_INVALID; }
+    // with S == 0 there is nothing to read or write: the arrays may then be NULL (empty)
+    if (S == 0) return 0;
+    if (!R_hist || !labels) { set_error("ljmd_clusters: null argument"); return LJMD_E_INVALID; }
+    if ((uintptr_t)R_hist % 8 || (uintptr_t)labels % 4 || (uintptr_t)sizes % 4) {
+        set_error("ljmd_clusters: R_hist must be 8-byte aligned, labels and sizes 4-byte aligned");
+        return LJMD_E_INVALID;
+    }
+    LJ_CUDA(cudaSetDevice(h->p.device));
+    return clusters(h, reinterpret_cast<const float2*>(R_hist), S, r_link, mask, labels, sizes);
+}
+
 int ljmd_cell_geometry(ljmd_t* h, int32_t* nrows, int32_t* nbins_x, int32_t* kbins,
                        float* inv_row_height, float* inv_bin_width) {
     if (!h) { set_error("null handle"); return LJMD_E_INVALID; }

@@ -63,25 +63,12 @@ bond_order_kernel(const float2* __restrict__ P, const int* __restrict__ idx, con
     long long sx = 0, sy = 0;
     int n = 0;
     if (ok) {
-        const int c = gr_cell(ri, inv_cell, nc);
-        const int cx = c % nc, cy = c / nc;
-        const int o = nc >= 3 ? 1 : 0;                 // nc < 3 only as nc == 1: one cell, all pairs
-        for (int oy = -o; oy <= o; ++oy) {
-            const int y = (cy + oy + nc) % nc;
-            for (int ox = -o; ox <= o; ++ox) {
-                const int cc = y * nc + (cx + ox + nc) % nc;
-                const int j1 = cs[cc + 1];
-                for (int j = cs[cc]; j < j1; ++j) {
-                    const float2 rj = Ps[j];
-                    const float dx = min_image(__fsub_rn(rj.x, ri.x), box, timg);
-                    const float dy = min_image(__fsub_rn(rj.y, ri.y), box, timg);
-                    const float r = __fsqrt_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)));
-                    if (!(r > 0.0f && r <= r_nb)) continue;   // also drops j == i and non-finite j
-                    bond_term(dx, dy, m, sx, sy);
-                    ++n;
-                }
-            }
-        }
+        gr_stencil_walk(Ps, cs, ri, inv_cell, nc, box, timg,
+                        [=](int, float dx, float dy, float r, long long& sx, long long& sy, int& n) {
+                            if (!(r > 0.0f && r <= r_nb)) return;      // also drops j == i and non-finite j
+                            bond_term(dx, dy, m, sx, sy);
+                            ++n;
+                        }, sx, sy, n);
     }
     double2 v = make_double2(0.0, 0.0);
     if (!ok) {

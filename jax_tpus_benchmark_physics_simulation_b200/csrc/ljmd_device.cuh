@@ -52,6 +52,34 @@ __device__ __forceinline__ int gr_cell(float2 p, float inv_cell, int nc) {
     return cy * nc + cx;
 }
 
+// The full 9-cell stencil of ri's cell on that grid (one cell, every particle, when nc < 3), for the bond order and
+// the cluster hook (bond.cu, cluster.cu): f(j, dx, dy, r, acc...) for every j in those cells (i itself included),
+// j in cell order, with d = min_image(fl(x_j - x_i)) and r = fl(sqrt(fl(fl(dx^2) + fl(dy^2)))), the r that g(r)
+// bins.  Ps: the snapshot's positions in cell order; cs: its cell starts.  The caller's per-thread accumulators
+// travel as the reference arguments acc rather than as captures of f: so bond_order_kernel compiles to the same
+// instructions as its hand-written loop did.
+template <class F, class... A>
+__device__ __forceinline__ void gr_stencil_walk(const float2* Ps, const int* cs, float2 ri, float inv_cell, int nc,
+                                                float box, float timg, F f, A&... acc) {
+    const int c = gr_cell(ri, inv_cell, nc);
+    const int cx = c % nc, cy = c / nc;
+    const int o = nc >= 3 ? 1 : 0;                 // nc < 3 only as nc == 1: one cell, all pairs
+    for (int oy = -o; oy <= o; ++oy) {
+        const int y = (cy + oy + nc) % nc;
+        for (int ox = -o; ox <= o; ++ox) {
+            const int cc = y * nc + (cx + ox + nc) % nc;
+            const int j1 = cs[cc + 1];
+            for (int j = cs[cc]; j < j1; ++j) {
+                const float2 rj = Ps[j];
+                const float dx = min_image(__fsub_rn(rj.x, ri.x), box, timg);
+                const float dy = min_image(__fsub_rn(rj.y, ri.y), box, timg);
+                const float r = __fsqrt_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)));
+                f(j, dx, dy, r, acc...);
+            }
+        }
+    }
+}
+
 // Weight of a pair in the g_m(r) histogram (ljmd_bond_corr): w = Re psi_i Re psi_j + Im psi_i Im psi_j, each
 // operation rounded once, added as the integer llrint(w 2^24) (exact and order-free).  false: w is not
 // finite and the pair is skipped.

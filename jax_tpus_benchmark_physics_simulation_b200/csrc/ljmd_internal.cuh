@@ -78,7 +78,7 @@ struct ljmd_handle {
     ljmd::AllPairs*  ap;
     ljmd::Cells*     cells;
     ljmd::Dist*      dist;
-    ljmd::Gr*        gr;          // cell-grid scratch of g(r), psi_m and g_m(r) (allocated on the first call that uses it)
+    ljmd::Gr*        gr;          // cell-grid scratch of g(r), psi_m, g_m(r) and clusters (allocated on the first call that uses it)
     cudaEvent_t      ev0, ev1;
     bool             timed;
     long long        launches;
@@ -141,6 +141,10 @@ void gr_destroy(ljmd_handle* h);
 
 // bond.cu: bond-orientational order psi_m of every particle (see ljmd_bond_order)
 int  bond_order(ljmd_handle* h, const float2* R_hist, long long S, int m, float r_nb, double2* psi, int* nnb);
+
+// cluster.cu: connected components within r_link of every snapshot (see ljmd_clusters); mask and sizes may be null
+int  clusters(ljmd_handle* h, const float2* R_hist, long long S, float r_link, const unsigned char* mask,
+              int* labels, int* sizes);
 
 // sk.cu: density modes rho_k of S snapshots for K integer wave vectors (see ljmd_density_modes)
 int  sk_density_modes(ljmd_handle* h, const float2* R_hist, long long S, const int2* nvec, long long K,

@@ -14,7 +14,10 @@ g(r); default box/2 as the reference, a few sigma for millions of particles), ``
 ``--sk_per_shell`` (the static structure factor S(k) of the production snapshots up to |k| = sk_kmax,
 default off; written as ``<stem>_sk.npy``/``.csv`` next to ``--output``), ``--bond_m`` / ``--bond_rnb``
 (the bond-orientational order psi_M of the production snapshots and its pair correlation g_M(r) on g(r)'s
-bins, default off; written as ``<stem>_psi{M}.npy`` and ``<stem>_g{M}.npy``/``.csv``).  matplotlib is imported
+bins, default off; written as ``<stem>_psi{M}.npy`` and ``<stem>_g{M}.npy``/``.csv``), ``--cluster_rlink`` /
+``--cluster_psi_min`` (the clusters of particles within r_link of the production snapshots, optionally only of
+the particles with |psi_M| >= psi_min, default off; the cluster-size distribution is written as
+``<stem>_clusters.npy``/``.csv``).  matplotlib is imported
 lazily (absent in this image): without it g(r) is written as ``.npy``/``.csv`` next to
 ``--output``.
 """
@@ -95,6 +98,23 @@ def main(args):
         bond = (np.asarray(r_b), np.asarray(g_b), Psi)
         print(f"psi_{M} calculation complete in {time_bond:.2f} s")
 
+    clus = None
+    if args.cluster_rlink is not None:
+        print("\n--- Calculating clusters ---")
+        start_time_clus = time.time()
+        mask = None
+        if args.cluster_psi_min is not None:                                    # solid-like particles only
+            psi = sim.last_bond_psi.tensor
+            mask = torch.hypot(psi[..., 0], psi[..., 1]) >= args.cluster_psi_min
+        _, sizes = sim.clusters(R_history, args.cluster_rlink, mask)
+        s_c, n_s = sim.cluster_distribution(sizes)
+        n_s.block_until_ready()
+        count, largest = sim.last_cluster_count.numpy(), sim.last_cluster_largest.numpy()
+        active = sizes.tensor.sum(dim=1, dtype=torch.int64).cpu().numpy()
+        time_clus = time.time() - start_time_clus
+        clus = (np.asarray(s_c), np.asarray(n_s))
+        print(f"Cluster analysis complete in {time_clus:.2f} s")
+
     print("\nSimulation Summary")
     print(f"  Equilibration  {time_eq:8.2f} s   {args.eq_steps:,} steps")
     print(f"  Production     {time_prod:8.2f} s   {args.prod_steps:,} steps")
@@ -112,8 +132,16 @@ def main(args):
         if mag.size:
             chi = N * (np.mean(mag ** 2) - np.mean(mag) ** 2)
             print(f"  <|Psi_{M}|> = {np.mean(mag):.6f}  chi_{M} = {chi:.6f}  over {mag.size} snapshots")
+    if clus is not None:
+        print(f"  Cluster Analysis {time_clus:6.2f} s   r_link = {args.cluster_rlink}"
+              + (f", |psi_{M}| >= {args.cluster_psi_min}" if args.cluster_psi_min is not None else "")
+              + f", {count.size} snapshots")
+        if count.size:
+            frac = largest / np.maximum(active, 1)
+            print(f"  <clusters> = {count.mean():.3f}  <largest> = {largest.mean():.3f}"
+                  f" ({frac.mean():.6f} of the active particles)")
     total = (time_eq + time_prod + time_g_r + (time_sk if sk is not None else 0.0)
-             + (time_bond if bond is not None else 0.0))
+             + (time_bond if bond is not None else 0.0) + (time_clus if clus is not None else 0.0))
     print(f"  Total          {total:8.2f} s")
     if sim.last_energies is not None:
         e = sim.last_energies.numpy()
@@ -147,6 +175,11 @@ def main(args):
         np.save(f"{stem}_g{M}.npy", np.stack(bond[:2]))
         np.savetxt(f"{stem}_g{M}.csv", np.stack(bond[:2], axis=1), delimiter=",", header=f"r,g_{M}")
         print(f"psi_{M} saved as '{stem}_psi{M}.npy', g_{M}(r) as '{stem}_g{M}.npy' and '{stem}_g{M}.csv'")
+    if clus is not None:
+        stem = args.output.rsplit(".", 1)[0] + "_clusters"
+        np.save(stem + ".npy", np.stack([clus[0].astype(np.float64), clus[1]]))
+        np.savetxt(stem + ".csv", np.stack(clus, axis=1), delimiter=",", header="s,n_s")
+        print(f"cluster sizes saved as '{stem}.npy' and '{stem}.csv'")
     if sk is not None:
         stem = args.output.rsplit(".", 1)[0] + "_sk"
         np.save(stem + ".npy", np.stack(sk))
@@ -193,6 +226,13 @@ def build_parser():
     parser.add_argument("--bond_rnb", type=float, default=1.5,
                         help="with --bond_m: neighbour radius of psi_M (default: 1.5, the conventional first "
                              "minimum of g(r))")
+    parser.add_argument("--cluster_rlink", type=float, default=None,
+                        help="find the clusters of the production snapshots: particles linked when they are "
+                             "within this distance (default: off)")
+    parser.add_argument("--cluster_psi_min", type=float, default=None,
+                        help="with --cluster_rlink and --bond_m M: only particles with |psi_M| >= this value "
+                             "(in [0, 1]) take part, e.g. the crystalline clusters of a melting or nucleating "
+                             "state (default: every particle)")
     return parser
 
 
@@ -211,6 +251,13 @@ def parse_args(argv=None):
         parser.error("--bond_m must be in [1, 12]")
     if not (args.bond_rnb > 0 and np.isfinite(args.bond_rnb)):
         parser.error("--bond_rnb must be positive and finite")
+    if args.cluster_rlink is not None and not (args.cluster_rlink > 0 and np.isfinite(args.cluster_rlink)):
+        parser.error("--cluster_rlink must be positive and finite")
+    if args.cluster_psi_min is not None:
+        if args.bond_m is None or args.cluster_rlink is None:
+            parser.error("--cluster_psi_min needs --cluster_rlink and --bond_m")
+        if not 0 <= args.cluster_psi_min <= 1:
+            parser.error("--cluster_psi_min must be in [0, 1]")
     return args
 
 

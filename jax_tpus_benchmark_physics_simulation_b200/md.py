@@ -431,13 +431,15 @@ class LJSimulation:
         """Pair correlation of the bond order g_m(r) = <psi_m(i) psi_m(j)*> over the pairs at distance r, on
         calculate_g_r's fp32 bins linspace(0, r_max, nbins + 1) (nbins defaults to int(r_max / 0.05)).  Returns
         (centers, g_m) device arrays; g_m = sum_s wsum / (2^24 sum_s counts) (ljmd_bond_corr), NaN in an empty bin.
-        The per-snapshot ``last_bond_counts`` / ``last_bond_wsum`` (S, nbins) int64 are kept, and psi_m as
-        ``bond_order`` keeps it.  Raises LjmdError if a count reaches 2^38, where wsum would stop being exact."""
+        The per-snapshot ``last_bond_counts`` / ``last_bond_wsum`` (S, nbins) int64 are kept, psi_m as
+        ``bond_order`` keeps it, and psi (S, N, 2) itself as ``last_bond_psi``.  Raises LjmdError if a count
+        reaches 2^38, where wsum would stop being exact."""
         r_max = np.float32(r_max)
         nbins = int(r_max / 0.05) if nbins is None else int(nbins)
         Rh = self._snapshots(R_history)
         S = Rh.shape[0]
         psi = self.bond_order(Rh, m, r_nb)[0].tensor
+        self.last_bond_psi = self._arr(psi)
         r_bins = np.linspace(0, r_max, nbins + 1, dtype=np.float32)              # as calculate_g_r
         centers = (r_bins[:-1] + r_bins[1:]) / np.float32(2.0)
         edges = torch.from_numpy(r_bins).to(self.device)
@@ -456,6 +458,52 @@ class LJSimulation:
         g = wsum.to(torch.float64).sum(dim=0) / (c * float(1 << 24))
         g = torch.where(c > 0, g, torch.full_like(g, float("nan")))
         return self._arr(torch.from_numpy(centers).to(self.device)), self._arr(g)
+
+    # ------------------------------------------------------------------ cluster analysis (new)
+    def clusters(self, R_history, r_link: float, mask=None):
+        """Clusters (connected components) of the snapshots R_history (S, N, 2) (or one (N, 2) state), two active
+        particles being linked when r_ij <= r_link (ljmd_clusters; link rule, active rule and labels in
+        include/ljmd.h).  mask: bool / uint8 (S, N) or (N,) (broadcast over the snapshots), or None (every particle
+        with finite coordinates is active).  Returns (labels, sizes) (S, N) int32 device arrays: labels[s, i] is the
+        smallest index in i's cluster (-1 for an inactive particle), sizes[s, k] the number of particles labelled k.
+        The number of clusters and the size of the largest one per snapshot are kept as ``last_cluster_count`` and
+        ``last_cluster_largest`` (S,) int64."""
+        Rh = self._snapshots(R_history)
+        S = Rh.shape[0]
+        m = None
+        if mask is not None:
+            if isinstance(mask, DeviceArray):
+                m = mask.tensor
+            elif isinstance(mask, torch.Tensor):
+                m = mask
+            else:
+                m = torch.from_numpy(np.ascontiguousarray(mask))
+            if m.dtype != torch.bool and m.dtype != torch.uint8:
+                raise ValueError(f"mask must be bool or uint8, got {m.dtype}")
+            if tuple(m.shape) not in ((self.N,), (S, self.N)):
+                raise ValueError(f"expected a mask of shape ({self.N},) or ({S}, {self.N}), got {tuple(m.shape)}")
+            m = m.to(self.device).to(torch.uint8).expand(S, self.N).contiguous()
+        labels = torch.empty((S, self.N), dtype=torch.int32, device=self.device)
+        sizes = torch.empty((S, self.N), dtype=torch.int32, device=self.device)
+        self._check_stream()
+        _lib.check(self.lib.ljmd_clusters(self._h, Rh.data_ptr() if S else None, S, float(r_link),
+                                          m.data_ptr() if m is not None and S else None,
+                                          labels.data_ptr() if S else None, sizes.data_ptr() if S else None),
+                   "ljmd_clusters")
+        self._after()
+        self.last_cluster_count = self._arr((sizes > 0).sum(dim=1, dtype=torch.int64))
+        self.last_cluster_largest = self._arr(sizes.max(dim=1).values.to(torch.int64))
+        return self._arr(labels), self._arr(sizes)
+
+    def cluster_distribution(self, sizes):
+        """Cluster-size distribution of the sizes (S, N) that ``clusters`` returns: (s, n_s) device arrays over the
+        sizes s that occur (int64, ascending), n_s the mean number of clusters of size s per snapshot (float64)."""
+        t = sizes.tensor if isinstance(sizes, DeviceArray) else torch.as_tensor(sizes)
+        t = t.to(self.device)
+        S = t.shape[0] if t.dim() == 2 else 1
+        counts = torch.bincount(t[t > 0].to(torch.int64).flatten())
+        s = torch.nonzero(counts).flatten()
+        return self._arr(s), self._arr(counts[s].to(torch.float64) / max(S, 1))
 
     # ------------------------------------------------------------------ cell-list introspection
     def cell_geometry(self):
