@@ -234,6 +234,44 @@ int ljmd_bond_corr(ljmd_t* h, const float* R_hist, const double* psi, int64_t S,
 int ljmd_clusters(ljmd_t* h, const float* R_hist, int64_t S, float r_link, const uint8_t* mask,
                   int32_t* labels, int32_t* sizes);
 
+/* ---- Voronoi tessellation (new; the reference has none - see DESIGN.md 4.8) ---------------------------------- */
+#define LJMD_VORONOI_MAX_VERTICES 64   /* polygon vertices a cell may need while it is built */
+/* The Voronoi cell of every particle of S snapshots on the periodic box.
+ * R_hist: device (S,N,2) float32 in [0, box], 8-byte aligned.  nvor: device int32 (S,N), required; area: device
+ * float64 (S,N), 8-byte aligned, or NULL; adj: device int32 (S,N,adj_cap), or NULL; psi: device float64 (S,N,2),
+ * 16-byte aligned, or NULL.  Integer arrays 4-byte aligned.  adj_cap in [1, 64] when adj is given; m in [1, 12]
+ * when psi is given (read only then).
+ *   - Sites: every particle with finite coordinates.  d_ij is the minimum-image difference of the fp32
+ *     coordinates computed in double (x_j - x_i, then -box if > box/2, +box if < -box/2): exact unless a
+ *     coordinate is a non-zero value below about 2^-29 box, and within 2^-53 box even then.  So d_ji = -d_ij.
+ *   - Cell: V_i = { p : p.d_ij <= |d_ij|^2 / 2 for every site j with d_ij != 0 }, relative to site i, in double.
+ *     Coincident sites (d_ij = 0) are ignored: two coincident particles get the same cell.
+ *   - Complete: with R_i the largest distance from i to a vertex of V_i, the cell is exact on the torus once
+ *     2 R_i < box / 2 (only minimum images can then cut it).  A particle whose cell does not meet that, or would
+ *     need more than LJMD_VORONOI_MAX_VERTICES vertices while it is clipped, is INCOMPLETE; so is a particle with a
+ *     non-finite coordinate, which is also nobody's neighbour.  Such a particle gets nvor = -1, area = psi = NaN
+ *     and an adjacency row of -1; the other particles are unaffected, and ljmd_check stays clean.
+ *   - Neighbours: j is a Voronoi neighbour of i when its half-plane gives V_i an edge of length l_ij > 2^-30 R_i
+ *     (rounding at a degenerate vertex - four co-circular sites, e.g. the exact square lattice - leaves edges of
+ *     ~1e-16 R_i, so the square lattice has 4 neighbours).  nvor[s*N + i] = their number.
+ *   - area[s*N + i]: the shoelace area of the final polygon, in double.
+ *   - adj[(s*N + i)*adj_cap + t]: the neighbours' original indices ordered by the angle of d_ij ascending in
+ *     (-pi, pi], padded with -1; with nvor > adj_cap the first adj_cap of them (nvor still counts all).
+ *   - psi[s*N + i]: sum_j (l_ij / L_i) (d_ij / |d_ij|)^m over the neighbours in adjacency order, L_i = sum_j l_ij;
+ *     the power by m - 1 sequential complex products as ljmd_bond_order, each operation rounded once.
+ *   - Deterministic: one thread per particle clips the cell by the sites in the order (double r^2, original index)
+ *     ascending, so the output is bit-identical on every run, whatever the other snapshots of the call, the
+ *     batching or the handle.
+ *   - Through the periodic cell grid of ljmd_gr_hist_rmax (cells of about two mean spacings; the rings around a
+ *     particle's cell grow until they cover its security radius 2 R_i; derivation in csrc/voronoi.cu).  Four
+ *     launches per batch of snapshots; the scratch is the grid's (16 B per particle and snapshot, batches <= 512
+ *     MiB), allocated on first use and kept until ljmd_destroy.
+ *   - Any handle works, the multi-GPU ones included; there is no communication.
+ * S < 0, a NULL R_hist or nvor, adj_cap or m out of range for a requested output, or a misaligned array:
+ * LJMD_E_INVALID.  S == 0 does nothing, and the arrays may then be NULL.                                         */
+int ljmd_voronoi(ljmd_t* h, const float* R_hist, int64_t S, int32_t* nvor, double* area,
+                 int32_t* adj, int32_t adj_cap, int32_t m, double* psi);
+
 /* ---- the other dense pairwise kernels of the reference repo (SURVEY.md 8f) -------- */
 /* All-pairs acceleration with the pair law as a functor: gravity r^-3 in an open plane.
  *   LJMD_LAW_GRAVITY_NBODY  pairwise_forces(positions, masses) of nbody_bh_merger_sim (NBODY:54-67):

@@ -324,6 +324,25 @@ int ljmd_clusters(ljmd_t* h, const float* R_hist, int64_t S, float r_link, const
     return clusters(h, reinterpret_cast<const float2*>(R_hist), S, r_link, mask, labels, sizes);
 }
 
+int ljmd_voronoi(ljmd_t* h, const float* R_hist, int64_t S, int32_t* nvor, double* area, int32_t* adj,
+                 int32_t adj_cap, int32_t m, double* psi) {
+    if (!h) { set_error("ljmd_voronoi: null handle"); return LJMD_E_INVALID; }
+    if (S < 0) { set_error("ljmd_voronoi: S must be >= 0"); return LJMD_E_INVALID; }
+    if (adj && (adj_cap < 1 || adj_cap > 64)) { set_error("ljmd_voronoi: adj_cap must be in [1,64]"); return LJMD_E_INVALID; }
+    if (psi && (m < 1 || m > 12)) { set_error("ljmd_voronoi: m must be in [1,12]"); return LJMD_E_INVALID; }
+    // with S == 0 there is nothing to read or write: the arrays may then be NULL (empty)
+    if (S == 0) return 0;
+    if (!R_hist || !nvor) { set_error("ljmd_voronoi: null argument"); return LJMD_E_INVALID; }
+    if ((uintptr_t)R_hist % 8 || (uintptr_t)nvor % 4 || (uintptr_t)area % 8 || (uintptr_t)adj % 4 ||
+        (uintptr_t)psi % 16) {
+        set_error("ljmd_voronoi: R_hist and area must be 8-byte aligned, psi 16-byte aligned, nvor and adj 4-byte aligned");
+        return LJMD_E_INVALID;
+    }
+    LJ_CUDA(cudaSetDevice(h->p.device));
+    return voronoi(h, reinterpret_cast<const float2*>(R_hist), S, nvor, area, adj, adj_cap, m,
+                   reinterpret_cast<double2*>(psi));
+}
+
 int ljmd_cell_geometry(ljmd_t* h, int32_t* nrows, int32_t* nbins_x, int32_t* kbins,
                        float* inv_row_height, float* inv_bin_width) {
     if (!h) { set_error("null handle"); return LJMD_E_INVALID; }

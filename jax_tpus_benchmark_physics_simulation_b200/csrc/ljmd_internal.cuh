@@ -78,7 +78,7 @@ struct ljmd_handle {
     ljmd::AllPairs*  ap;
     ljmd::Cells*     cells;
     ljmd::Dist*      dist;
-    ljmd::Gr*        gr;          // cell-grid scratch of g(r), psi_m, g_m(r) and clusters (allocated on the first call that uses it)
+    ljmd::Gr*        gr;          // cell-grid scratch of g(r), psi_m, g_m(r), clusters and Voronoi (allocated on the first call that uses it)
     cudaEvent_t      ev0, ev1;
     bool             timed;
     long long        launches;
@@ -145,6 +145,10 @@ int  bond_order(ljmd_handle* h, const float2* R_hist, long long S, int m, float 
 // cluster.cu: connected components within r_link of every snapshot (see ljmd_clusters); mask and sizes may be null
 int  clusters(ljmd_handle* h, const float2* R_hist, long long S, float r_link, const unsigned char* mask,
               int* labels, int* sizes);
+
+// voronoi.cu: Voronoi cell of every particle (see ljmd_voronoi); area, adj and psi may be null
+int  voronoi(ljmd_handle* h, const float2* R_hist, long long S, int* nvor, double* area, int* adj, int adj_cap,
+             int m, double2* psi);
 
 // sk.cu: density modes rho_k of S snapshots for K integer wave vectors (see ljmd_density_modes)
 int  sk_density_modes(ljmd_handle* h, const float2* R_hist, long long S, const int2* nvec, long long K,

@@ -17,7 +17,9 @@ default off; written as ``<stem>_sk.npy``/``.csv`` next to ``--output``), ``--bo
 bins, default off; written as ``<stem>_psi{M}.npy`` and ``<stem>_g{M}.npy``/``.csv``), ``--cluster_rlink`` /
 ``--cluster_psi_min`` (the clusters of particles within r_link of the production snapshots, optionally only of
 the particles with |psi_M| >= psi_min, default off; the cluster-size distribution is written as
-``<stem>_clusters.npy``/``.csv``).  matplotlib is imported
+``<stem>_clusters.npy``/``.csv``), ``--voronoi`` (the Voronoi tessellation of the production snapshots:
+neighbour counts and topological defects, with ``--bond_m`` also the edge-weighted psi_M, default off; the
+per-snapshot counts are written as ``<stem>_voronoi.npy``/``.csv``).  matplotlib is imported
 lazily (absent in this image): without it g(r) is written as ``.npy``/``.csv`` next to
 ``--output``.
 """
@@ -115,6 +117,23 @@ def main(args):
         clus = (np.asarray(s_c), np.asarray(n_s))
         print(f"Cluster analysis complete in {time_clus:.2f} s")
 
+    vor = None
+    if args.voronoi:
+        from .md import topological_defects
+        print("\n--- Calculating Voronoi tessellation ---")
+        start_time_vor = time.time()
+        nvor, _ = sim.voronoi(R_history, m=args.bond_m, adj_cap=16)
+        d = topological_defects(nvor, sim.last_voronoi_adj)
+        nv = nvor.tensor
+        ok = nv >= 0
+        cols = ["n5", "n7", "other", "charge", "incomplete", "disclinations", "dislocations", "defect_clusters"]
+        vor = np.stack([d[c].cpu().numpy() for c in cols], axis=1).astype(np.int64)
+        n_mean = float(torch.where(ok, nv, torch.zeros_like(nv)).sum()) / max(int(ok.sum()), 1)
+        defect_frac = float((ok & (nv != 6)).sum()) / max(int(ok.sum()), 1)
+        vpsi = sim.last_voronoi_global.numpy() if args.bond_m is not None else None
+        time_vor = time.time() - start_time_vor
+        print(f"Voronoi tessellation complete in {time_vor:.2f} s")
+
     print("\nSimulation Summary")
     print(f"  Equilibration  {time_eq:8.2f} s   {args.eq_steps:,} steps")
     print(f"  Production     {time_prod:8.2f} s   {args.prod_steps:,} steps")
@@ -140,8 +159,19 @@ def main(args):
             frac = largest / np.maximum(active, 1)
             print(f"  <clusters> = {count.mean():.3f}  <largest> = {largest.mean():.3f}"
                   f" ({frac.mean():.6f} of the active particles)")
+    if vor is not None:
+        print(f"  Voronoi Analysis {time_vor:6.2f} s   {vor.shape[0]} snapshots, {int(vor[:, 4].sum())} incomplete cells")
+        if vor.shape[0]:
+            print(f"  <n> = {n_mean:.6f}  defect fraction = {defect_frac:.6f}  <disclinations> = "
+                  f"{vor[:, 5].mean():.3f}  <dislocations> = {vor[:, 6].mean():.3f} per snapshot")
+            if vpsi is not None:
+                line = f"  <|Psi_{M}|> Voronoi-weighted = {np.mean(np.hypot(vpsi[:, 0], vpsi[:, 1])):.6f}"
+                if bond is not None and bond[2].size:
+                    line += f"  (r_nb = {args.bond_rnb}: {np.mean(np.hypot(bond[2][:, 0], bond[2][:, 1])):.6f})"
+                print(line)
     total = (time_eq + time_prod + time_g_r + (time_sk if sk is not None else 0.0)
-             + (time_bond if bond is not None else 0.0) + (time_clus if clus is not None else 0.0))
+             + (time_bond if bond is not None else 0.0) + (time_clus if clus is not None else 0.0)
+             + (time_vor if vor is not None else 0.0))
     print(f"  Total          {total:8.2f} s")
     if sim.last_energies is not None:
         e = sim.last_energies.numpy()
@@ -180,6 +210,12 @@ def main(args):
         np.save(stem + ".npy", np.stack([clus[0].astype(np.float64), clus[1]]))
         np.savetxt(stem + ".csv", np.stack(clus, axis=1), delimiter=",", header="s,n_s")
         print(f"cluster sizes saved as '{stem}.npy' and '{stem}.csv'")
+    if vor is not None:
+        stem = args.output.rsplit(".", 1)[0] + "_voronoi"
+        np.save(stem + ".npy", vor)
+        np.savetxt(stem + ".csv", vor, delimiter=",", fmt="%d",
+                   header="n5,n7,other,charge,incomplete,disclinations,dislocations,defect_clusters")
+        print(f"Voronoi defect counts saved as '{stem}.npy' and '{stem}.csv'")
     if sk is not None:
         stem = args.output.rsplit(".", 1)[0] + "_sk"
         np.save(stem + ".npy", np.stack(sk))
@@ -233,6 +269,9 @@ def build_parser():
                         help="with --cluster_rlink and --bond_m M: only particles with |psi_M| >= this value "
                              "(in [0, 1]) take part, e.g. the crystalline clusters of a melting or nucleating "
                              "state (default: every particle)")
+    parser.add_argument("--voronoi", action="store_true",
+                        help="compute the Voronoi tessellation of the production snapshots: neighbour counts, "
+                             "topological defects and, with --bond_m M, the edge-weighted psi_M (default: off)")
     return parser
 
 

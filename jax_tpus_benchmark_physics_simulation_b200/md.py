@@ -505,6 +505,40 @@ class LJSimulation:
         s = torch.nonzero(counts).flatten()
         return self._arr(s), self._arr(counts[s].to(torch.float64) / max(S, 1))
 
+    # ------------------------------------------------------------------ Voronoi tessellation (new)
+    def voronoi(self, R_history, m: Optional[int] = None, adj_cap: int = 16):
+        """Voronoi cell of every particle of the snapshots R_history (S, N, 2) (or one (N, 2) state) on the periodic
+        box (ljmd_voronoi; cell, completeness and neighbour rules in include/ljmd.h).  Returns (nvor (S, N) int32,
+        area (S, N) float64) device arrays; nvor = -1 and area = NaN for an incomplete or non-finite particle.
+        With adj_cap > 0 the neighbours' original indices ordered by angle, (S, N, adj_cap) int32 padded with -1,
+        are kept as ``last_voronoi_adj``.  With m given, the edge-weighted psi_m (S, N, 2) float64 is kept as
+        ``last_voronoi_psi`` and its per-snapshot mean over the complete particles as ``last_voronoi_global``
+        (S, 2)."""
+        Rh = self._snapshots(R_history)
+        S = Rh.shape[0]
+        adj_cap = int(adj_cap)
+        if not 0 <= adj_cap <= 64:
+            raise ValueError(f"adj_cap must be in [0, 64], got {adj_cap}")
+        if m is not None and not 1 <= int(m) <= 12:
+            raise ValueError(f"m must be in [1, 12], got {m}")
+        nvor = torch.empty((S, self.N), dtype=torch.int32, device=self.device)
+        area = torch.empty((S, self.N), dtype=torch.float64, device=self.device)
+        adj = torch.empty((S, self.N, adj_cap), dtype=torch.int32, device=self.device) if adj_cap else None
+        psi = torch.empty((S, self.N, 2), dtype=torch.float64, device=self.device) if m is not None else None
+        ptr = (lambda t: t.data_ptr() if t is not None and S else None)
+        self._check_stream()
+        _lib.check(self.lib.ljmd_voronoi(self._h, ptr(Rh), S, ptr(nvor), ptr(area), ptr(adj), max(adj_cap, 1),
+                                         int(m) if m is not None else 0, ptr(psi)), "ljmd_voronoi")
+        self._after()
+        self.last_voronoi_adj = self._arr(adj) if adj is not None else None
+        self.last_voronoi_psi = self._arr(psi) if psi is not None else None
+        self.last_voronoi_global = None
+        if psi is not None:
+            ok = (nvor >= 0).unsqueeze(-1)
+            tot = torch.where(ok, psi, torch.zeros_like(psi)).sum(dim=1)
+            self.last_voronoi_global = self._arr(tot / ok.sum(dim=1).clamp(min=1).to(torch.float64))
+        return self._arr(nvor), self._arr(area)
+
     # ------------------------------------------------------------------ cell-list introspection
     def cell_geometry(self):
         """(nrows, nbins_x, kbins, inv_row_height, inv_bin_width) of the strip-cell grid."""
@@ -557,6 +591,69 @@ class LJSimulation:
         v = ctypes.c_int64()
         _lib.check(self.lib.ljmd_launch_count(self._h, ctypes.byref(v)), "ljmd_launch_count")
         return v.value
+
+
+def topological_defects(nvor, adj) -> dict:
+    """Topological defects of Voronoi tessellations (LJSimulation.voronoi): nvor (S, N) and adj (S, N, adj_cap)
+    integer tensors (or DeviceArrays, or one (N,) / (N, adj_cap) snapshot), on any device.  Per snapshot, (S,)
+    int64 tensors on that device:
+        n5, n7       complete particles with 5 and 7 neighbours
+        other        complete particles with n not in {5, 6, 7}
+        charge       sum of 6 - n over the complete particles (0 for a tessellation of the whole torus)
+        incomplete   particles with nvor = -1
+    and the components of the defect subgraph - the complete particles with n != 6, linked by Voronoi adjacency -
+    found by min-label propagation (deterministic):
+        disclinations    components of one particle
+        dislocations     components of exactly one 5 and one 7
+        defect_clusters  every other component
+    Raises ValueError if a defective particle has more neighbours than adj holds (its row would be truncated)."""
+    nv = nvor.tensor if isinstance(nvor, DeviceArray) else torch.as_tensor(nvor)
+    ad = adj.tensor if isinstance(adj, DeviceArray) else torch.as_tensor(adj)
+    if nv.dim() == 1:
+        nv, ad = nv[None], ad[None]
+    if nv.dim() != 2 or ad.dim() != 3 or ad.shape[:2] != nv.shape:
+        raise ValueError(f"expected nvor (S, N) and adj (S, N, cap), got {tuple(nv.shape)} and {tuple(ad.shape)}")
+    S, N = nv.shape
+    cap = ad.shape[2]
+    nv = nv.to(torch.int64)
+    ad = ad.to(device=nv.device, dtype=torch.int64)
+    complete = nv >= 0
+    defect = complete & (nv != 6)
+    if bool((defect & (nv > cap)).any()):
+        raise ValueError(f"a defective particle has more than adj_cap = {cap} neighbours: raise adj_cap")
+    out = {
+        "n5": (nv == 5).sum(dim=1), "n7": (nv == 7).sum(dim=1),
+        "other": (complete & (nv != 5) & (nv != 6) & (nv != 7)).sum(dim=1),
+        "charge": torch.where(complete, 6 - nv, torch.zeros_like(nv)).sum(dim=1),
+        "incomplete": (~complete).sum(dim=1),
+    }
+    base = (torch.arange(S, device=nv.device) * N)[:, None]
+    src = (base + torch.arange(N, device=nv.device)[None, :])[:, :, None].expand(S, N, cap)
+    dst = base[:, :, None] + ad
+    flat_def = defect.flatten()
+    keep = (ad >= 0) & defect[:, :, None]
+    keep &= flat_def[torch.where(keep, dst, torch.zeros_like(dst))]
+    a, b = src[keep], dst[keep]
+    a, b = torch.cat([a, b]), torch.cat([b, a])
+    big = S * N
+    label = torch.where(flat_def, torch.arange(big, device=nv.device), torch.full_like(flat_def, big, dtype=torch.int64))
+    while True:
+        new = label.scatter_reduce(0, b, label[a], reduce="amin")
+        if torch.equal(new, label):
+            break
+        label = new
+    roots = label[flat_def]
+    size = torch.bincount(roots, minlength=big)
+    c5 = torch.bincount(roots, weights=(nv.flatten()[flat_def] == 5).to(torch.float64), minlength=big)
+    c7 = torch.bincount(roots, weights=(nv.flatten()[flat_def] == 7).to(torch.float64), minlength=big)
+    is_root = size > 0
+    snap = torch.arange(big, device=nv.device) // N
+    one = is_root & (size == 1)
+    pair57 = is_root & (size == 2) & (c5 == 1) & (c7 == 1)
+    rest = is_root & ~one & ~pair57
+    for name, sel in (("disclinations", one), ("dislocations", pair57), ("defect_clusters", rest)):
+        out[name] = torch.bincount(snap[sel], minlength=S)
+    return out
 
 
 def _isqrt(n2: np.ndarray) -> np.ndarray:
