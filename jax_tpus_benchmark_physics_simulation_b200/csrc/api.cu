@@ -232,9 +232,10 @@ int ljmd_run_blocked(ljmd_t* h, const float* R_blk, const float* V_blk, float* R
 int ljmd_gr_hist(ljmd_t* h, const float* R_hist, int64_t S, int32_t nbins, const float* edges,
                  int64_t* counts) {
     if (!h || !counts || !edges || (S > 0 && !R_hist) || S < 0) { set_error("bad argument"); return LJMD_E_INVALID; }
+    if (nbins < 1 || nbins > LJMD_GR_MAXBINS) { set_error("g(r): nbins must be in [1,%d]", LJMD_GR_MAXBINS); return LJMD_E_INVALID; }
     LJ_CUDA(cudaSetDevice(h->p.device));
-    return ap_gr_hist(h, reinterpret_cast<const float2*>(R_hist), S, nbins, edges,
-                      std::numeric_limits<float>::infinity(), reinterpret_cast<long long*>(counts));
+    return gr_allpairs_hist(h, reinterpret_cast<const float2*>(R_hist), S, nbins, edges,
+                            std::numeric_limits<float>::infinity(), reinterpret_cast<long long*>(counts));
 }
 
 int ljmd_gr_hist_rmax(ljmd_t* h, const float* R_hist, int64_t S, int32_t nbins, const float* edges,
@@ -246,12 +247,8 @@ int ljmd_gr_hist_rmax(ljmd_t* h, const float* R_hist, int64_t S, int32_t nbins, 
     if (!(r_max > 0.0f) || !std::isfinite(r_max)) { set_error("ljmd_gr_hist_rmax: r_max must be positive and finite"); return LJMD_E_INVALID; }
     if (S == 0) return 0;
     LJ_CUDA(cudaSetDevice(h->p.device));
-    const float2* R = reinterpret_cast<const float2*>(R_hist);
-    long long* c = reinterpret_cast<long long*>(counts);
-    // the cell grid needs 3 cells per side for its half stencil to visit every pair once
-    const int nc = gr_grid_side(h->p.N, h->p.box, r_max);
-    if (nc >= 3) return gr_cells_hist(h, R, S, nbins, edges, r_max, nc, c);
-    return ap_gr_hist(h, R, S, nbins, edges, r_max, c);
+    return gr_pair_hist(h, reinterpret_cast<const float2*>(R_hist), S, nbins, edges, r_max,
+                        reinterpret_cast<long long*>(counts));
 }
 
 int ljmd_density_modes(ljmd_t* h, const float* R_hist, int64_t S, const int32_t* nvec, int64_t K, double* rho) {
@@ -298,14 +295,9 @@ int ljmd_bond_corr(ljmd_t* h, const float* R_hist, const double* psi, int64_t S,
         return LJMD_E_INVALID;
     }
     LJ_CUDA(cudaSetDevice(h->p.device));
-    const float2* R = reinterpret_cast<const float2*>(R_hist);
-    const double2* p = reinterpret_cast<const double2*>(psi);
-    long long* c = reinterpret_cast<long long*>(counts);
-    long long* w = reinterpret_cast<long long*>(wsum);
-    // the same selection as ljmd_gr_hist_rmax, so the counts are its counts wherever every weight is finite
-    const int nc = gr_grid_side(h->p.N, h->p.box, r_max);
-    if (nc >= 3) return gr_cells_hist(h, R, S, nbins, edges, r_max, nc, c, p, w);
-    return ap_gr_hist(h, R, S, nbins, edges, r_max, c, p, w);
+    return gr_pair_hist(h, reinterpret_cast<const float2*>(R_hist), S, nbins, edges, r_max,
+                        reinterpret_cast<long long*>(counts), reinterpret_cast<const double2*>(psi),
+                        reinterpret_cast<long long*>(wsum));
 }
 
 int ljmd_clusters(ljmd_t* h, const float* R_hist, int64_t S, float r_link, const uint8_t* mask, int32_t* labels,

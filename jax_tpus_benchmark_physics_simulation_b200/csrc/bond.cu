@@ -8,7 +8,7 @@
 //
 // Bond term.  d = min_image(fl(x_j - x_i)) from i to j (the sign matters for odd m), converted to double (exact);
 // then in double, every operation rounded once (no contraction): r_d = sqrt(d_x^2 + d_y^2), u = d / r_d, and
-// w = u^m by m - 1 sequential complex products w <- w u = (ac - bd, ad + bc).
+// w = u^m by m - 1 sequential complex products w <- w u = (ac - bd, ad + bc) (unit_pow, ljmd_device.cuh).
 //
 // Fixed-point sum.  q = llrint(w 2^32) per component, summed in int64: exact (N < 2^31 terms of |q| <= 2^32 + 1)
 // and independent of the order of the terms, hence of the cell order that the atomic ranks of gr_count_kernel
@@ -36,17 +36,9 @@ namespace {
 constexpr int BO_THREADS = 256;
 
 __device__ __forceinline__ void bond_term(float dxf, float dyf, int m, long long& sx, long long& sy) {
-    const double dx = (double)dxf, dy = (double)dyf;
-    const double r = __dsqrt_rn(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)));
-    const double ux = __ddiv_rn(dx, r), uy = __ddiv_rn(dy, r);
-    double wx = ux, wy = uy;
-    for (int k = 1; k < m; ++k) {
-        const double a = wx, b = wy;
-        wx = __dsub_rn(__dmul_rn(a, ux), __dmul_rn(b, uy));
-        wy = __dadd_rn(__dmul_rn(a, uy), __dmul_rn(b, ux));
-    }
-    sx += llrint(__dmul_rn(wx, 4294967296.0));
-    sy += llrint(__dmul_rn(wy, 4294967296.0));
+    const double2 w = unit_pow((double)dxf, (double)dyf, m);
+    sx += llrint(__dmul_rn(w.x, 4294967296.0));
+    sy += llrint(__dmul_rn(w.y, 4294967296.0));
 }
 
 __global__ void __launch_bounds__(BO_THREADS)

@@ -1,10 +1,11 @@
-// gr.cu — the pair-distance histogram of calculate_g_r (get_histogram, MD:117-124) through a cell grid:
-// only pairs in neighbouring cells of a periodic nc x nc grid of edge >= r_max are visited, so a histogram
-// that ends at r_max costs O(S N rho pi r_max^2) instead of the O(S N^2) of gr_hist_kernel (allpairs.cu).
-// The counts are those of gr_hist_kernel bit for bit: the same fp32 r of every pair, the same binning
-// (gr_bin), exact integer counts.  ljmd_gr_hist_rmax (api.cu) decides which of the two kernels runs.
+// gr.cu — the pair-distance histogram of calculate_g_r (get_histogram, MD:117-124), by two kernels with the same
+// counts bit for bit: the same fp32 r of every pair, the same binning (gr_bin), exact integer counts.
+//   gr_hist_kernel   every pair, O(S N^2): ljmd_gr_hist, and the fallback for small boxes
+//   gr_cells_kernel  only pairs in neighbouring cells of a periodic nc x nc grid of edge >= r_max, so a histogram
+//                    that ends at r_max costs O(S N rho pi r_max^2)
+// gr_pair_hist decides which of the two runs for ljmd_gr_hist_rmax and ljmd_bond_corr.
 //
-// Per batch of snapshots (blockIdx.y = snapshot in the batch), four launches:
+// Cell grid, per batch of snapshots (blockIdx.y = snapshot in the batch), four launches:
 //   gr_count_kernel    cell of every particle, atomic per-cell count; the returned slot is its rank in the cell
 //   gr_scan_kernel     in-place exclusive scan of the counts -> cell_start[nc^2 + 1] (one CTA per snapshot)
 //   gr_scatter_kernel  positions in cell order
@@ -226,6 +227,80 @@ gr_cells_kernel(const GrCellsArgs a) {
     }
 }
 
+// ---- all pairs: the upper triangle of (GR_TILE x GR_TILE) tiles ------------------------------------------------
+constexpr int GR_THREADS = 256;
+constexpr int GR_TILE    = 256;
+
+// W: byte offset of the CTA's 64-bit weight sums, after gr_hist_kernel's other shared arrays (8-aligned)
+__host__ __device__ constexpr size_t gr_wsum_offset(int nbins) {
+    return (sizeof(float2) * GR_TILE + sizeof(float) * (2 * (size_t)nbins + 1) + 7) / 8 * 8;
+}
+
+// W (ljmd_bond_corr): a counted pair with a finite weight w_ij (bond_pair_weight) also adds llrint(w 2^24) to
+// wsum; a pair whose weight is not finite is neither counted nor summed.  psi (S,N) in particle order.
+template <bool W>
+__global__ void __launch_bounds__(GR_THREADS)
+gr_hist_kernel(const float2* __restrict__ Rh, int N, float box, float timg, int nbins,
+               const float* __restrict__ edges, unsigned long long* __restrict__ counts,
+               int ntile, float cap, const double2* __restrict__ psi, unsigned long long* __restrict__ wsum) {
+    // blockIdx.x -> (tile_i <= tile_j) upper-triangular tile pair; blockIdx.y -> snapshot
+    // cap: pairs with r > cap are dropped as well (ljmd_gr_hist_rmax); +INFINITY for ljmd_gr_hist
+    extern __shared__ unsigned char smem_raw[];
+    float2*   sj     = reinterpret_cast<float2*>(smem_raw);                 // GR_TILE (8-byte aligned)
+    float*    sedges = reinterpret_cast<float*>(sj + GR_TILE);              // nbins+1
+    unsigned* shist  = reinterpret_cast<unsigned*>(sedges + nbins + 1);     // nbins
+    const int tid = threadIdx.x;
+    int t = blockIdx.x, ti = 0;
+    while (t >= ntile - ti) { t -= ntile - ti; ++ti; }
+    const int tj = ti + t;
+    const float2* R = Rh + (size_t)blockIdx.y * N;
+    unsigned long long* swsum = nullptr;
+    if constexpr (W) {
+        swsum = reinterpret_cast<unsigned long long*>(smem_raw + gr_wsum_offset(nbins));   // nbins
+        psi += (size_t)blockIdx.y * N;
+        for (int k = tid; k < nbins; k += GR_THREADS) swsum[k] = 0ull;
+    }
+    for (int k = tid; k <= nbins; k += GR_THREADS) sedges[k] = edges[k];
+    for (int k = tid; k < nbins; k += GR_THREADS) shist[k] = 0u;
+    {
+        const int j = tj * GR_TILE + tid;
+        if (tid < GR_TILE) sj[tid] = (j < N) ? R[j] : make_float2(SENT_J, SENT_J);
+    }
+    __syncthreads();
+    const int i = ti * GR_TILE + tid;
+    if (i < N) {
+        const float2 ri = R[i];
+        double2 pi = make_double2(0.0, 0.0);
+        if constexpr (W) pi = psi[i];
+        const float lo = sedges[0], hi = fminf(sedges[nbins], cap);
+        const float scale = (float)nbins / (sedges[nbins] - lo);
+        for (int q = 0; q < GR_TILE; ++q) {
+            const int j = tj * GR_TILE + q;
+            if (j <= i || j >= N) continue;                                  // triu, k=1
+            const float dx = min_image(__fsub_rn(ri.x, sj[q].x), box, timg);
+            const float dy = min_image(__fsub_rn(ri.y, sj[q].y), box, timg);
+            const float r = __fsqrt_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)));
+            const int b = gr_bin(r, sedges, nbins, lo, hi, scale);          // numpy drops outliers
+            if (b < 0) continue;
+            if constexpr (W) {
+                long long wq;
+                if (!bond_pair_weight(pi, psi[j], wq)) continue;
+                atomicAdd(&swsum[b], (unsigned long long)wq);
+            }
+            atomicAdd(&shist[b], 1u);
+        }
+    }
+    __syncthreads();
+    unsigned long long* out = counts + (size_t)blockIdx.y * nbins;
+    for (int k = tid; k < nbins; k += GR_THREADS)
+        if (shist[k]) atomicAdd(&out[k], (unsigned long long)shist[k]);
+    if constexpr (W) {
+        unsigned long long* wout = wsum + (size_t)blockIdx.y * nbins;
+        for (int k = tid; k < nbins; k += GR_THREADS)
+            if (swsum[k]) atomicAdd(&wout[k], swsum[k]);
+    }
+}
+
 }  // namespace
 
 // Cells per side of the g(r) grid for pairs up to r_max.  Every pair with fp32 r <= r_max must lie in
@@ -303,8 +378,11 @@ int gr_grid_bin(ljmd_handle* h, const GrGrid& g, const float2* R, const double2*
     return 0;
 }
 
-int gr_cells_hist(ljmd_handle* h, const float2* R_hist, long long S, int nbins, const float* edges,
-                  float r_max, int nc, long long* counts, const double2* psi, long long* wsum) {
+int gr_pair_hist(ljmd_handle* h, const float2* R_hist, long long S, int nbins, const float* edges, float r_max,
+                 long long* counts, const double2* psi, long long* wsum) {
+    // the cell grid needs 3 cells per side for its half stencil to visit every pair once
+    const int nc = gr_grid_side(h->p.N, h->p.box, r_max);
+    if (nc < 3) return gr_allpairs_hist(h, R_hist, S, nbins, edges, r_max, counts, psi, wsum);
     const long long N = h->p.N;
     const bool W = psi != nullptr;
     cudaStream_t st = h->stream;
@@ -333,6 +411,34 @@ int gr_cells_hist(ljmd_handle* h, const float2* R_hist, long long S, int nbins, 
         kernel<<<dim3(cblocks, ns), GRC_THREADS, smem, st>>>(a);
         LJ_CUDA(cudaGetLastError());
         h->launches += 1;
+    }
+    return 0;
+}
+
+int gr_allpairs_hist(ljmd_handle* h, const float2* R_hist, long long S, int nbins, const float* edges,
+                     float cap, long long* counts, const double2* psi, long long* wsum) {
+    const int N = (int)h->p.N;
+    const bool W = psi != nullptr;
+    cudaStream_t st = h->stream;
+    LJ_CUDA(cudaMemsetAsync(counts, 0, sizeof(long long) * S * nbins, st));
+    if (W) LJ_CUDA(cudaMemsetAsync(wsum, 0, sizeof(long long) * S * nbins, st));
+    if (S == 0) return 0;
+    const int ntile = (N + GR_TILE - 1) / GR_TILE;
+    const long long npairs = (long long)ntile * (ntile + 1) / 2;
+    const size_t smem = W ? gr_wsum_offset(nbins) + sizeof(long long) * nbins
+                          : sizeof(float) * (nbins + 1) + sizeof(unsigned) * nbins + sizeof(float2) * GR_TILE;
+    auto kernel = W ? gr_hist_kernel<true> : gr_hist_kernel<false>;
+    LJ_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    // grid.y is limited to 65535 snapshots per launch
+    for (long long s0 = 0; s0 < S; s0 += 65535) {
+        const int ns = (int)std::min<long long>(65535, S - s0);
+        kernel<<<dim3((unsigned)npairs, ns), GR_THREADS, smem, st>>>(
+            R_hist + (size_t)s0 * N, N, h->pc.box, h->pc.timg, nbins, edges,
+            reinterpret_cast<unsigned long long*>(counts) + (size_t)s0 * nbins, ntile, cap,
+            W ? psi + (size_t)s0 * N : nullptr,
+            W ? reinterpret_cast<unsigned long long*>(wsum) + (size_t)s0 * nbins : nullptr);
+        LJ_CUDA(cudaGetLastError());
+        h->launches++;
     }
     return 0;
 }

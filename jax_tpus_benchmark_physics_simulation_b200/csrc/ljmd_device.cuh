@@ -4,6 +4,8 @@
 
 namespace ljmd {
 
+constexpr float SENT_J = 1.0e18f;   // padding particles: far away, contribute exactly 0
+
 __device__ __forceinline__ float rcp_approx(float x) {
     float r;
     asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));   // MUFU.RCP, <= 1 ulp
@@ -44,8 +46,8 @@ __device__ __forceinline__ int gr_bin(float r, const float* e, int nbins, float 
 
 // Cell of a position in [0, box] on the periodic nc x nc grid of g(r) and the bond order (gr.cu, bond.cu): one
 // fp32 multiply and truncation per axis.  The clamps keep any other input (outside [0, box], non-finite)
-// inside the grid; such pairs are then dropped by the binning or counted as gr_hist_kernel would count
-// them, as long as they are adjacent.
+// inside the grid; such pairs are then dropped by the binning or counted as gr_hist_kernel (gr.cu) would
+// count them, as long as they are adjacent.
 __device__ __forceinline__ int gr_cell(float2 p, float inv_cell, int nc) {
     const int cx = min(max((int)__fmul_rn(p.x, inv_cell), 0), nc - 1);
     const int cy = min(max((int)__fmul_rn(p.y, inv_cell), 0), nc - 1);
@@ -78,6 +80,21 @@ __device__ __forceinline__ void gr_stencil_walk(const float2* Ps, const int* cs,
             }
         }
     }
+}
+
+// (d / |d|)^m of a bond vector d in double, every operation rounded once: r = sqrt(dx^2 + dy^2), u = d / r, then
+// m - 1 sequential complex products w <- w u = (ac - bd, ad + bc).  The psi_m of bond.cu and voronoi.cu agree
+// because both take u^m from here.
+__device__ __forceinline__ double2 unit_pow(double dx, double dy, int m) {
+    const double r = __dsqrt_rn(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)));
+    const double ux = __ddiv_rn(dx, r), uy = __ddiv_rn(dy, r);
+    double wx = ux, wy = uy;
+    for (int k = 1; k < m; ++k) {
+        const double a = wx, b = wy;
+        wx = __dsub_rn(__dmul_rn(a, ux), __dmul_rn(b, uy));
+        wy = __dadd_rn(__dmul_rn(a, uy), __dmul_rn(b, ux));
+    }
+    return make_double2(wx, wy);
 }
 
 // Weight of a pair in the g_m(r) histogram (ljmd_bond_corr): w = Re psi_i Re psi_j + Im psi_i Im psi_j, each

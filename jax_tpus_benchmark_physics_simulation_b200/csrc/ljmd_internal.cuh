@@ -100,10 +100,6 @@ int  ap_run(ljmd_handle* h, const float2* R_in, const float2* V_in, float2* R_ou
             float2* F_out, float* pe_out, const RunCtl& rc, float* vir_out);
 int  ap_check_error(ljmd_handle* h);
 int  ap_mode(ljmd_handle* h);
-// cap: pairs with r > cap are dropped too (+INFINITY: the plain histogram of ljmd_gr_hist)
-// psi != nullptr: the weighted histogram of ljmd_bond_corr (psi (S,N) in particle order, wsum (S,nbins))
-int  ap_gr_hist(ljmd_handle* h, const float2* R_hist, long long S, int nbins, const float* edges,
-                float cap, long long* counts, const double2* psi = nullptr, long long* wsum = nullptr);
 
 // cells.cu
 int  cells_create(ljmd_handle* h);
@@ -116,11 +112,15 @@ int  cells_neighbor_count(ljmd_handle* h, const float2* R, float radius, int* nb
 long long cells_last_rebuilds(ljmd_handle* h);
 int  cells_check_error(ljmd_handle* h);
 
-// gr.cu: g(r) through a periodic nc x nc cell grid of edge >= r_max (see ljmd_gr_hist_rmax)
-int  gr_grid_side(long long N, float box, float r_max);   // nc for this r_max (the grid is used when >= 3)
-// psi != nullptr: the weighted histogram of ljmd_bond_corr (psi (S,N) in particle order, wsum (S,nbins))
-int  gr_cells_hist(ljmd_handle* h, const float2* R_hist, long long S, int nbins, const float* edges,
-                   float r_max, int nc, long long* counts, const double2* psi = nullptr, long long* wsum = nullptr);
+// gr.cu: the g(r) pair-distance histogram, over all pairs or through a periodic nc x nc cell grid of edge >= r_max.
+// psi != nullptr: the weighted histogram of ljmd_bond_corr (psi (S,N) in particle order, wsum (S,nbins)).
+// Every pair; cap: pairs with r > cap are dropped too (+INFINITY: the plain histogram of ljmd_gr_hist)
+int  gr_allpairs_hist(ljmd_handle* h, const float2* R_hist, long long S, int nbins, const float* edges,
+                      float cap, long long* counts, const double2* psi = nullptr, long long* wsum = nullptr);
+// The pairs with r <= r_max, through the grid when it has >= 3 cells per side, else gr_allpairs_hist
+int  gr_pair_hist(ljmd_handle* h, const float2* R_hist, long long S, int nbins, const float* edges,
+                  float r_max, long long* counts, const double2* psi = nullptr, long long* wsum = nullptr);
+int  gr_grid_side(long long N, float box, float r_max);   // nc for this r_max
 // One batch of snapshots binned into the nc x nc grid, in the handle's Gr scratch (rows of the batch: nb).
 // with_idx: also idx (original index of each particle in cell order, for the bond order);
 // with_psi: also psi (its psi in cell order, for the weighted histogram of ljmd_bond_corr).

@@ -42,7 +42,7 @@
 // the shoelace formula over all vertices; adjacency = the counted neighbours' original indices ordered by the angle
 // of d_ij ascending in (-pi, pi] (the polygon is counter-clockwise, so its edge normals already are in angular
 // order up to the start), first adj_cap of them, -1 padded; psi = sum_j (l_j / L) (d_j / |d_j|)^m in that order,
-// L = sum of the counted l_j, u^m as bond_term (m - 1 sequential complex products), every operation rounded once.
+// L = sum of the counted l_j, u^m by unit_pow (m - 1 sequential complex products), every operation rounded once.
 #include "ljmd_device.cuh"
 
 #include <algorithm>
@@ -305,17 +305,10 @@ voronoi_kernel(const VorArgs a) {
             if (!(l > lmin)) continue;
             const float2 rj = Ps[P.g[k]];
             const double dx = vor_disp(rj.x, ri.x, box, half), dy = vor_disp(rj.y, ri.y, box, half);
-            const double r = __dsqrt_rn(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)));
-            const double ux = __ddiv_rn(dx, r), uy = __ddiv_rn(dy, r);
-            double wx = ux, wy = uy;
-            for (int q = 1; q < a.m; ++q) {
-                const double u = wx, v = wy;
-                wx = __dsub_rn(__dmul_rn(u, ux), __dmul_rn(v, uy));
-                wy = __dadd_rn(__dmul_rn(u, uy), __dmul_rn(v, ux));
-            }
+            const double2 w = unit_pow(dx, dy, a.m);
             const double c_l = __ddiv_rn(l, L);
-            sx = __dadd_rn(sx, __dmul_rn(c_l, wx));
-            sy = __dadd_rn(sy, __dmul_rn(c_l, wy));
+            sx = __dadd_rn(sx, __dmul_rn(c_l, w.x));
+            sy = __dadd_rn(sy, __dmul_rn(c_l, w.y));
         }
         a.psi[o] = make_double2(sx, sy);
     }

@@ -27,6 +27,12 @@ _PATHS = {"auto": _lib.LJMD_PATH_AUTO, "allpairs": _lib.LJMD_PATH_ALLPAIRS,
           "cells": _lib.LJMD_PATH_CELLS}
 
 
+def _ptr(t: Optional[torch.Tensor]) -> Optional[int]:
+    """Device address of t for the C ABI, or None (NULL) when t is None or empty: the library reads and writes
+    nothing of an empty array, and accepts NULL for it."""
+    return t.data_ptr() if t is not None and t.numel() else None
+
+
 class DeviceArray:
     """Minimal jax.Array look-alike over a CUDA torch tensor: ``.block_until_ready()``
     (MD:145,152,163), ``.shape`` (MD:174), ``__array__`` for numpy/matplotlib (MD:181)."""
@@ -176,15 +182,15 @@ class LJSimulation:
             raise ValueError(f"expected shape {tuple(shape)}, got {tuple(t.shape)}")
         return t
 
-    def _check_stream(self):
+    def _call(self, name: str, *args) -> None:
+        """self.lib.<name>(handle, *args), checked, ordered after torch's current stream and before its later work
+        (the handle enqueues on the stream captured at construction)."""
         cur = torch.cuda.current_stream(self.device)
-        if cur.cuda_stream != self._stream.cuda_stream:
-            # the handle enqueues on the stream captured at construction: order the two streams
+        other = cur.cuda_stream != self._stream.cuda_stream
+        if other:
             self._stream.wait_stream(cur)
-
-    def _after(self):
-        cur = torch.cuda.current_stream(self.device)
-        if cur.cuda_stream != self._stream.cuda_stream:
+        _lib.check(getattr(self.lib, name)(self._h, *args), name)
+        if other:
             cur.wait_stream(self._stream)
 
     # ------------------------------------------------------------------ MD:46-48
@@ -200,28 +206,21 @@ class LJSimulation:
     def total_energy_fn(self, R) -> DeviceArray:
         R = self._dev(R, (self.N, 2))
         out = torch.empty(1, dtype=torch.float32, device=self.device)
-        self._check_stream()
-        _lib.check(self.lib.ljmd_energy(self._h, R.data_ptr(), out.data_ptr()), "ljmd_energy")
-        self._after()
+        self._call("ljmd_energy", R.data_ptr(), out.data_ptr())
         return self._arr(out[0])
 
     # ------------------------------------------------------------------ MD:64
     def force_fn(self, R) -> DeviceArray:
         R = self._dev(R, (self.N, 2))
         F = torch.empty_like(R)
-        self._check_stream()
-        _lib.check(self.lib.ljmd_forces(self._h, R.data_ptr(), F.data_ptr(), None), "ljmd_forces")
-        self._after()
+        self._call("ljmd_forces", R.data_ptr(), F.data_ptr(), None)
         return self._arr(F)
 
     def force_and_energy(self, R) -> Tuple[DeviceArray, DeviceArray]:
         R = self._dev(R, (self.N, 2))
         F = torch.empty_like(R)
         pe = torch.empty(1, dtype=torch.float32, device=self.device)
-        self._check_stream()
-        _lib.check(self.lib.ljmd_forces(self._h, R.data_ptr(), F.data_ptr(), pe.data_ptr()),
-                   "ljmd_forces")
-        self._after()
+        self._call("ljmd_forces", R.data_ptr(), F.data_ptr(), pe.data_ptr())
         return self._arr(F), self._arr(pe[0])
 
     # ------------------------------------------------------------------ virial / pressure (new)
@@ -230,9 +229,7 @@ class LJSimulation:
         same pair set, minimum image and fp32 arithmetic as the force; no tail correction."""
         R = self._dev(R, (self.N, 2))
         out = torch.empty(1, dtype=torch.float32, device=self.device)
-        self._check_stream()
-        _lib.check(self.lib.ljmd_virial(self._h, R.data_ptr(), out.data_ptr()), "ljmd_virial")
-        self._after()
+        self._call("ljmd_virial", R.data_ptr(), out.data_ptr())
         return self._arr(out[0])
 
     def _pressure(self, ke: torch.Tensor, w: torch.Tensor) -> torch.Tensor:
@@ -262,20 +259,14 @@ class LJSimulation:
         ne = -(-nsteps // energy_every) if energy_every > 0 else 0
         ke_pe = torch.zeros((ne, 2), dtype=torch.float32, device=self.device) if ne else None
         w = torch.zeros(ne, dtype=torch.float32, device=self.device) if (virial and ne) else None
-        self._check_stream()
         if w is None:
-            _lib.check(self.lib.ljmd_run(
-                self._h, R.data_ptr(), V.data_ptr(), R_out.data_ptr(), V_out.data_ptr(), nsteps,
-                sample_every if S > 0 else 0, traj.data_ptr() if S > 0 else None,
-                energy_every if ne else 0, ke_pe.data_ptr() if ne else None,
-                self.thermostat_kT, self.thermostat_every), "ljmd_run")
+            self._call("ljmd_run", R.data_ptr(), V.data_ptr(), R_out.data_ptr(), V_out.data_ptr(), nsteps,
+                       sample_every if S > 0 else 0, _ptr(traj), energy_every if ne else 0, _ptr(ke_pe),
+                       self.thermostat_kT, self.thermostat_every)
         else:
-            _lib.check(self.lib.ljmd_run_virial(
-                self._h, R.data_ptr(), V.data_ptr(), R_out.data_ptr(), V_out.data_ptr(), nsteps,
-                sample_every if S > 0 else 0, traj.data_ptr() if S > 0 else None,
-                energy_every, ke_pe.data_ptr(), self.thermostat_kT, self.thermostat_every,
-                w.data_ptr()), "ljmd_run_virial")
-        self._after()
+            self._call("ljmd_run_virial", R.data_ptr(), V.data_ptr(), R_out.data_ptr(), V_out.data_ptr(), nsteps,
+                       sample_every if S > 0 else 0, _ptr(traj), energy_every, ke_pe.data_ptr(),
+                       self.thermostat_kT, self.thermostat_every, w.data_ptr())
         self.last_energies = self._arr(ke_pe) if ne else None
         self.last_virial = self._arr(w) if w is not None else None
         self.last_pressure = self._arr(self._pressure(ke_pe[:, 0], w)) if w is not None else None
@@ -307,11 +298,8 @@ class LJSimulation:
         R_out, V_out = torch.empty_like(R), torch.empty_like(V)
         ne = -(-nsteps // energy_every) if energy_every > 0 else 0
         ke_pe = torch.zeros((ne, 2), dtype=torch.float32, device=self.device) if ne else None
-        self._check_stream()
-        _lib.check(self.lib.ljmd_run_blocked(
-            self._h, R.data_ptr(), V.data_ptr(), R_out.data_ptr(), V_out.data_ptr(), int(nsteps),
-            energy_every if ne else 0, ke_pe.data_ptr() if ne else None), "ljmd_run_blocked")
-        self._after()
+        self._call("ljmd_run_blocked", R.data_ptr(), V.data_ptr(), R_out.data_ptr(), V_out.data_ptr(), int(nsteps),
+                   energy_every if ne else 0, _ptr(ke_pe))
         self.last_energies = self._arr(ke_pe) if ne else None
         return self._arr(R_out), self._arr(V_out)
 
@@ -349,10 +337,8 @@ class LJSimulation:
         ideal = rho_pairs * shell                                                 # MD:115
         edges = torch.from_numpy(r_bins).to(self.device)
         counts = torch.empty((S, nbins), dtype=torch.int64, device=self.device)
-        self._check_stream()
-        _lib.check(self.lib.ljmd_gr_hist_rmax(self._h, Rh.data_ptr(), S, nbins, edges.data_ptr(),
-                                              float(r_bins[-1]), counts.data_ptr()), "ljmd_gr_hist_rmax")
-        self._after()
+        self._call("ljmd_gr_hist_rmax", Rh.data_ptr(), S, nbins, edges.data_ptr(), float(r_bins[-1]),
+                   counts.data_ptr())
         self.last_gr_counts = DeviceArray(counts)
         avg = counts.to(torch.float32).mean(dim=0) if S else torch.zeros(nbins, device=self.device)
         g = avg / torch.from_numpy(ideal.astype(np.float32)).to(self.device)      # MD:126-128
@@ -363,19 +349,11 @@ class LJSimulation:
         """rho_k(s) = sum_j exp(i 2 pi (n_x x_j + n_y y_j) / box) of the snapshots R_history (S, N, 2) (or one
         (N, 2) state) for the integer wave vectors nvec (K, 2): a float64 (S, K, 2) = (Re, Im) device array
         (ljmd_density_modes; fixed-point phase, accuracy bound and NaN rule in include/ljmd.h)."""
-        Rh = self._dev(R_history)
-        if Rh.dim() == 2:
-            Rh = Rh[None]
-        if Rh.dim() != 3 or tuple(Rh.shape[1:]) != (self.N, 2):
-            raise ValueError(f"expected snapshots of shape (S, {self.N}, 2), got {tuple(Rh.shape)}")
+        Rh = self._snapshots(R_history)
         nv = torch.as_tensor(np.asarray(nvec, dtype=np.int32).reshape(-1, 2)).to(self.device).contiguous()
         S, K = Rh.shape[0], nv.shape[0]
         rho = torch.empty((S, K, 2), dtype=torch.float64, device=self.device)
-        self._check_stream()
-        _lib.check(self.lib.ljmd_density_modes(self._h, Rh.data_ptr() if S else None, S,
-                                               nv.data_ptr() if K else None, K, rho.data_ptr() if S * K else None),
-                   "ljmd_density_modes")
-        self._after()
+        self._call("ljmd_density_modes", _ptr(Rh), S, _ptr(nv), K, _ptr(rho))
         return self._arr(rho)
 
     def structure_factor(self, R_history, k_max: float, max_per_shell: Optional[int] = None):
@@ -419,11 +397,7 @@ class LJSimulation:
         S = Rh.shape[0]
         psi = torch.empty((S, self.N, 2), dtype=torch.float64, device=self.device)
         nnb = torch.empty((S, self.N), dtype=torch.int32, device=self.device)
-        self._check_stream()
-        _lib.check(self.lib.ljmd_bond_order(self._h, Rh.data_ptr() if S else None, S, int(m), float(r_nb),
-                                            psi.data_ptr() if S else None, nnb.data_ptr() if S else None),
-                   "ljmd_bond_order")
-        self._after()
+        self._call("ljmd_bond_order", _ptr(Rh), S, int(m), float(r_nb), _ptr(psi), _ptr(nnb))
         self.last_bond_global = self._arr(psi.mean(dim=1))
         return self._arr(psi), self._arr(nnb)
 
@@ -445,12 +419,8 @@ class LJSimulation:
         edges = torch.from_numpy(r_bins).to(self.device)
         counts = torch.empty((S, nbins), dtype=torch.int64, device=self.device)
         wsum = torch.empty((S, nbins), dtype=torch.int64, device=self.device)
-        self._check_stream()
-        _lib.check(self.lib.ljmd_bond_corr(self._h, Rh.data_ptr() if S else None, psi.data_ptr() if S else None, S,
-                                           nbins, edges.data_ptr(), float(r_bins[-1]),
-                                           counts.data_ptr() if S else None, wsum.data_ptr() if S else None),
-                   "ljmd_bond_corr")
-        self._after()
+        self._call("ljmd_bond_corr", _ptr(Rh), _ptr(psi), S, nbins, edges.data_ptr(), float(r_bins[-1]),
+                   _ptr(counts), _ptr(wsum))
         self.last_bond_counts, self.last_bond_wsum = self._arr(counts), self._arr(wsum)
         if S and int(counts.max()) >= 1 << 38:
             raise _lib.LjmdError("ljmd_bond_corr: a bin count reached 2^38, beyond which wsum is not exact")
@@ -485,12 +455,7 @@ class LJSimulation:
             m = m.to(self.device).to(torch.uint8).expand(S, self.N).contiguous()
         labels = torch.empty((S, self.N), dtype=torch.int32, device=self.device)
         sizes = torch.empty((S, self.N), dtype=torch.int32, device=self.device)
-        self._check_stream()
-        _lib.check(self.lib.ljmd_clusters(self._h, Rh.data_ptr() if S else None, S, float(r_link),
-                                          m.data_ptr() if m is not None and S else None,
-                                          labels.data_ptr() if S else None, sizes.data_ptr() if S else None),
-                   "ljmd_clusters")
-        self._after()
+        self._call("ljmd_clusters", _ptr(Rh), S, float(r_link), _ptr(m), _ptr(labels), _ptr(sizes))
         self.last_cluster_count = self._arr((sizes > 0).sum(dim=1, dtype=torch.int64))
         self.last_cluster_largest = self._arr(sizes.max(dim=1).values.to(torch.int64))
         return self._arr(labels), self._arr(sizes)
@@ -525,11 +490,8 @@ class LJSimulation:
         area = torch.empty((S, self.N), dtype=torch.float64, device=self.device)
         adj = torch.empty((S, self.N, adj_cap), dtype=torch.int32, device=self.device) if adj_cap else None
         psi = torch.empty((S, self.N, 2), dtype=torch.float64, device=self.device) if m is not None else None
-        ptr = (lambda t: t.data_ptr() if t is not None and S else None)
-        self._check_stream()
-        _lib.check(self.lib.ljmd_voronoi(self._h, ptr(Rh), S, ptr(nvor), ptr(area), ptr(adj), max(adj_cap, 1),
-                                         int(m) if m is not None else 0, ptr(psi)), "ljmd_voronoi")
-        self._after()
+        self._call("ljmd_voronoi", _ptr(Rh), S, _ptr(nvor), _ptr(area), _ptr(adj), max(adj_cap, 1),
+                   int(m) if m is not None else 0, _ptr(psi))
         self.last_voronoi_adj = self._arr(adj) if adj is not None else None
         self.last_voronoi_psi = self._arr(psi) if psi is not None else None
         self.last_voronoi_global = None
@@ -554,19 +516,13 @@ class LJSimulation:
         nr, nb, _, _, _ = self.cell_geometry()
         cid = torch.empty(self.N, dtype=torch.int32, device=self.device)
         cnt = torch.empty(nr * nb, dtype=torch.int32, device=self.device)
-        self._check_stream()
-        _lib.check(self.lib.ljmd_cell_assign(self._h, R.data_ptr(), cid.data_ptr(), cnt.data_ptr()),
-                   "ljmd_cell_assign")
-        self._after()
+        self._call("ljmd_cell_assign", R.data_ptr(), cid.data_ptr(), cnt.data_ptr())
         return cid, cnt
 
     def neighbor_count(self, R, radius: float):
         R = self._dev(R, (self.N, 2))
         out = torch.empty(self.N, dtype=torch.int32, device=self.device)
-        self._check_stream()
-        _lib.check(self.lib.ljmd_neighbor_count(self._h, R.data_ptr(), float(radius),
-                                                out.data_ptr()), "ljmd_neighbor_count")
-        self._after()
+        self._call("ljmd_neighbor_count", R.data_ptr(), float(radius), out.data_ptr())
         return out
 
     def last_rebuilds(self) -> int:

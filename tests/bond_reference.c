@@ -9,69 +9,13 @@
  *   corr         for the pairs i < j of gr_reference.c's histogram: w = a.x b.x + a.y b.y, skipped when not
  *                finite, else counts += 1 and wsum += llrint(w 2^24)
  * Neighbour search: every pair for N <= 65536 (bref_bond_order) or with fewer than 5 cells per side, otherwise
- * an OpenMP grid of cells of edge >= the radius (in double) with a +-2-cell stencil, so the result does not rely
- * on the margin proof of the library's grid.  Compiled by tests/bond_reference.py with -O2 -ffp-contract=off
- * -fno-fast-math (every operation rounds once).  The product never loads it.
+ * the grid of ref_grid.h (cells of edge >= the radius, +-2-cell stencil, OpenMP over i), so the result does not
+ * rely on the margin proof of the library's grid.  Compiled by tests/cref.py.  The product never loads it.
  */
-#include <math.h>
-#include <stdint.h>
-#include <stdlib.h>
-#include <string.h>
+#include "ref_grid.h"
 #ifdef _OPENMP
 #include <omp.h>
 #endif
-
-static inline float minimg(float d, float box) {
-    return d - box * rintf(d / box);
-}
-
-static inline int finite2(const float* R, int64_t i) {
-    return isfinite(R[2 * i]) && isfinite(R[2 * i + 1]);
-}
-
-/* cells of edge >= radius with a +-2-cell stencil; NULL (every pair) when that grid has fewer than 5 per side */
-typedef struct { int32_t nc; int32_t* head; int32_t* cid; int32_t* order; } Grid;
-
-static int grid_build(Grid* g, int64_t N, const float* R, float box, float radius) {
-    int32_t nc = (int32_t)floor((double)box / (double)radius);
-    if (nc > 4096) nc = 4096;
-    if (nc < 5) return 0;
-    double cell = (double)box / nc;
-    size_t ncc = (size_t)nc * nc;
-    g->nc = nc;
-    g->head = (int32_t*)calloc(ncc + 1, sizeof(int32_t));
-    g->cid = (int32_t*)malloc(sizeof(int32_t) * N);
-    g->order = (int32_t*)malloc(sizeof(int32_t) * N);
-    for (int64_t i = 0; i < N; ++i) {
-        int32_t cx = 0, cy = 0;
-        if (finite2(R, i)) {                       /* non-finite particles pair with nobody: any cell will do */
-            cx = (int32_t)floor((double)R[2 * i] / cell);
-            cy = (int32_t)floor((double)R[2 * i + 1] / cell);
-            if (cx >= nc) cx = nc - 1;
-            if (cy >= nc) cy = nc - 1;
-            if (cx < 0) cx = 0;
-            if (cy < 0) cy = 0;
-        }
-        g->cid[i] = cy * nc + cx;
-        g->head[g->cid[i] + 1]++;
-    }
-    for (size_t c = 0; c < ncc; ++c) g->head[c + 1] += g->head[c];
-    int32_t* fill = (int32_t*)malloc(sizeof(int32_t) * ncc);
-    memcpy(fill, g->head, sizeof(int32_t) * ncc);
-    for (int64_t i = 0; i < N; ++i) g->order[fill[g->cid[i]]++] = (int32_t)i;
-    free(fill);
-    return 1;
-}
-
-static void grid_free(Grid* g) {
-    free(g->head); free(g->cid); free(g->order);
-}
-
-static inline float pair_r(const float* R, int64_t i, int64_t j, float box, float* dx, float* dy) {
-    *dx = minimg(R[2 * j] - R[2 * i], box);
-    *dy = minimg(R[2 * j + 1] - R[2 * i + 1], box);
-    return sqrtf(*dx * *dx + *dy * *dy);
-}
 
 static inline void bond_add(const float* R, int64_t i, int64_t j, float box, int32_t m, float r_nb,
                             int64_t* sx, int64_t* sy, int32_t* n) {

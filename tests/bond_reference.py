@@ -1,47 +1,22 @@
 """TEST INFRASTRUCTURE ONLY — fp64 CPU restatement of the bond-orientational order psi_m (ljmd_bond_order) and of
 its pair-correlation histogram (ljmd_bond_corr), with the library's neighbour and fixed-point rules.
 
-``bond_order`` and ``bond_corr`` call tests/bond_reference.c, compiled on first use into a temporary directory
-(the source tree may be read-only).  The product package never imports this module.
+``bond_order`` and ``bond_corr`` call tests/bond_reference.c, compiled on first use (tests/cref.py).  The product
+package never imports this module.
 """
 from __future__ import annotations
 
 import ctypes
-import os
-import shutil
-import subprocess
-import tempfile
 
 import numpy as np
 
+import cref
 from gr_reference import edges_for
 
-_HERE = os.path.dirname(os.path.abspath(__file__))
-_lib = None
-
-
-def _build() -> ctypes.CDLL:
-    global _lib
-    if _lib is not None:
-        return _lib
-    cc = shutil.which("/usr/bin/gcc") or shutil.which("gcc") or shutil.which("cc")
-    if cc is None:
-        raise RuntimeError("no C compiler found for tests/bond_reference.c")
-    out = os.path.join(tempfile.mkdtemp(prefix="bond_reference_"), "libbond_reference.so")
-    src = os.path.join(_HERE, "bond_reference.c")
-    flags = ["-O2", "-fPIC", "-shared", "-std=c11", "-ffp-contract=off", "-fno-fast-math"]
-    try:
-        subprocess.check_call([cc, *flags, "-fopenmp", "-o", out, src, "-lm"], stderr=subprocess.DEVNULL)
-    except subprocess.CalledProcessError:             # no OpenMP runtime: serial build
-        subprocess.check_call([cc, *flags, "-Wno-unknown-pragmas", "-o", out, src, "-lm"])
-    lib = ctypes.CDLL(out)
+def _lib():
     vp, i64, i32, f32 = ctypes.c_void_p, ctypes.c_int64, ctypes.c_int32, ctypes.c_float
-    lib.bref_bond_order.argtypes = [i64, vp, f32, i32, f32, vp, vp]
-    lib.bref_bond_order.restype = None
-    lib.bref_bond_corr.argtypes = [i64, vp, vp, f32, i32, vp, f32, vp, vp]
-    lib.bref_bond_corr.restype = None
-    _lib = lib
-    return lib
+    return cref.load("bond_reference", {"bref_bond_order": ([i64, vp, f32, i32, f32, vp, vp], None),
+                                        "bref_bond_corr": ([i64, vp, vp, f32, i32, vp, f32, vp, vp], None)})
 
 
 def bond_order(R, box, m, r_nb):
@@ -50,8 +25,8 @@ def bond_order(R, box, m, r_nb):
     N = R.shape[0]
     psi = np.zeros((N, 2), np.float64)
     nnb = np.zeros(N, np.int32)
-    _build().bref_bond_order(N, R.ctypes.data, float(np.float32(box)), int(m), float(np.float32(r_nb)),
-                             psi.ctypes.data, nnb.ctypes.data)
+    _lib().bref_bond_order(N, R.ctypes.data, float(np.float32(box)), int(m), float(np.float32(r_nb)),
+                           psi.ctypes.data, nnb.ctypes.data)
     return psi, nnb
 
 
@@ -64,8 +39,8 @@ def bond_corr(R, psi, box, nbins, r_max, r_cap=None):
     cap = float(edges[-1]) if r_cap is None else float(np.float32(r_cap))
     counts = np.zeros(nbins, np.int64)
     wsum = np.zeros(nbins, np.int64)
-    _build().bref_bond_corr(R.shape[0], R.ctypes.data, psi.ctypes.data, float(np.float32(box)), nbins,
-                            edges.ctypes.data, cap, counts.ctypes.data, wsum.ctypes.data)
+    _lib().bref_bond_corr(R.shape[0], R.ctypes.data, psi.ctypes.data, float(np.float32(box)), nbins,
+                          edges.ctypes.data, cap, counts.ctypes.data, wsum.ctypes.data)
     return counts, wsum
 
 

@@ -5,10 +5,10 @@
  *   links    the pairs i < j of active particles with r <= r_link, r = sqrtf(dx*dx + dy*dy), dx = minimg(x_j - x_i)
  *            in fp32; coincident particles (r = 0) are linked
  * Every pair when the grid of cells of edge >= r_link has fewer than 5 per side, otherwise that grid with its
- * +-2-cell stencil.  tests/cluster_reference.py compiles it with bond_reference.c's flags and turns the links into
- * components.  The product never loads it.
+ * +-2-cell stencil.  tests/cluster_reference.py compiles it (tests/cref.py) and turns the links into components.
+ * The product never loads it.
  */
-#include "bond_reference.c"
+#include "ref_grid.h"
 
 static inline int active(const float* R, const uint8_t* mask, int64_t i) {
     return finite2(R, i) && (!mask || mask[i]);

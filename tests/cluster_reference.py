@@ -3,46 +3,17 @@ tests/cluster_reference.c (the fp32 pair rule of the library), their connected c
 scipy.sparse.csgraph, and the library's labels (smallest index of the cluster, -1 for an inactive particle) and
 sizes.
 
-The C file is compiled on first use into a temporary directory (the source tree may be read-only).  The product
-package never imports this module.
+The C file is compiled on first use (tests/cref.py).  The product package never imports this module.
 """
 from __future__ import annotations
 
 import ctypes
-import os
-import shutil
-import subprocess
-import tempfile
 
 import numpy as np
 from scipy.sparse import coo_matrix
 from scipy.sparse.csgraph import connected_components
 
-_HERE = os.path.dirname(os.path.abspath(__file__))
-_lib = None
-
-
-def _build() -> ctypes.CDLL:
-    global _lib
-    if _lib is not None:
-        return _lib
-    cc = shutil.which("/usr/bin/gcc") or shutil.which("gcc") or shutil.which("cc")
-    if cc is None:
-        raise RuntimeError("no C compiler found for tests/cluster_reference.c")
-    out = os.path.join(tempfile.mkdtemp(prefix="cluster_reference_"), "libcluster_reference.so")
-    src = os.path.join(_HERE, "cluster_reference.c")
-    flags = ["-O2", "-fPIC", "-shared", "-std=c11", "-ffp-contract=off", "-fno-fast-math", "-I", _HERE]
-    try:
-        subprocess.check_call([cc, *flags, "-fopenmp", "-o", out, src, "-lm"], stderr=subprocess.DEVNULL)
-    except subprocess.CalledProcessError:             # no OpenMP runtime: serial build
-        subprocess.check_call([cc, *flags, "-Wno-unknown-pragmas", "-o", out, src, "-lm"])
-    lib = ctypes.CDLL(out)
-    vp, i64, f32 = ctypes.c_void_p, ctypes.c_int64, ctypes.c_float
-    lib.bref_links.argtypes = [i64, vp, f32, f32, vp, vp]
-    lib.bref_links.restype = i64
-    _lib = lib
-    return lib
-
+import cref
 
 def _mask(mask, N):
     return None if mask is None else np.ascontiguousarray(np.broadcast_to(np.asarray(mask) != 0, (N,)), np.uint8)
@@ -54,7 +25,9 @@ def links(R, box, r_link, mask=None):
     N = R.shape[0]
     m = _mask(mask, N)
     mp = None if m is None else m.ctypes.data
-    lib = _build()
+    lib = cref.load("cluster_reference", {"bref_links": ([ctypes.c_int64, ctypes.c_void_p, ctypes.c_float,
+                                                          ctypes.c_float, ctypes.c_void_p, ctypes.c_void_p],
+                                                         ctypes.c_int64)})
     args = (N, R.ctypes.data, float(np.float32(box)), float(np.float32(r_link)), mp)
     n = lib.bref_links(*args, None)
     pairs = np.zeros((max(n, 1), 2), np.int32)

@@ -2,44 +2,21 @@
 
 ``c_gr_hist_cells`` is tests/gr_reference.c: oracle/lj_oracle.c's orc_gr_hist (the same fp32 r and binary
 search against the fp32 edges) through an OpenMP cell grid with a +-2-cell stencil, optionally dropping
-pairs with r > r_cap.  The C file is compiled on first use into a temporary directory (the source tree may
-be read-only).  The product package never imports this module.
+pairs with r > r_cap.  The C file is compiled on first use (tests/cref.py).  The product package never imports
+this module.
 """
 from __future__ import annotations
 
 import ctypes
-import os
-import shutil
-import subprocess
-import tempfile
 
 import numpy as np
 
-_HERE = os.path.dirname(os.path.abspath(__file__))
-_lib = None
+import cref
 
-
-def _build() -> ctypes.CDLL:
-    global _lib
-    if _lib is not None:
-        return _lib
-    cc = shutil.which("/usr/bin/gcc") or shutil.which("gcc") or shutil.which("cc")
-    if cc is None:
-        raise RuntimeError("no C compiler found for tests/gr_reference.c")
-    out = os.path.join(tempfile.mkdtemp(prefix="gr_reference_"), "libgr_reference.so")
-    src = os.path.join(_HERE, "gr_reference.c")
-    flags = ["-O2", "-fPIC", "-shared", "-std=c11", "-ffp-contract=off", "-fno-fast-math"]
-    try:
-        subprocess.check_call([cc, *flags, "-fopenmp", "-o", out, src, "-lm"], stderr=subprocess.DEVNULL)
-    except subprocess.CalledProcessError:             # no OpenMP runtime: serial build
-        subprocess.check_call([cc, *flags, "-Wno-unknown-pragmas", "-o", out, src, "-lm"])
-    lib = ctypes.CDLL(out)
+def _lib():
     f32p = ctypes.POINTER(ctypes.c_float)
-    lib.gref_gr_hist.argtypes = [ctypes.c_int64, f32p, ctypes.c_float, ctypes.c_int32, f32p, ctypes.c_float,
-                                 ctypes.POINTER(ctypes.c_int64)]
-    lib.gref_gr_hist.restype = None
-    _lib = lib
-    return lib
+    return cref.load("gr_reference", {"gref_gr_hist": ([ctypes.c_int64, f32p, ctypes.c_float, ctypes.c_int32, f32p,
+                                                        ctypes.c_float, ctypes.POINTER(ctypes.c_int64)], None)})
 
 
 def edges_for(r_max, nbins):
@@ -54,9 +31,9 @@ def c_gr_hist_cells(R, box, nbins, r_max, r_cap=None):
     edges = edges_for(r_max, nbins)
     cap = float(edges[-1]) if r_cap is None else float(np.float32(r_cap))
     counts = np.zeros(nbins, dtype=np.int64)
-    _build().gref_gr_hist(R.shape[0], R.ctypes.data_as(ctypes.POINTER(ctypes.c_float)), float(np.float32(box)),
-                          nbins, edges.ctypes.data_as(ctypes.POINTER(ctypes.c_float)), cap,
-                          counts.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)))
+    _lib().gref_gr_hist(R.shape[0], R.ctypes.data_as(ctypes.POINTER(ctypes.c_float)), float(np.float32(box)),
+                        nbins, edges.ctypes.data_as(ctypes.POINTER(ctypes.c_float)), cap,
+                        counts.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)))
     return counts
 
 

@@ -8,24 +8,13 @@ import pytest
 import torch
 
 import bond_reference as ref
+from analysis_helpers import E_INVALID, hist_rmax, make_sim, md_snapshots, same_bits
 from gr_reference import adversarial, edges_for
 from jax_tpus_benchmark_physics_simulation_b200 import lattice_jitter
-from jax_tpus_benchmark_physics_simulation_b200.md import LJSimulation
 
 pytestmark = pytest.mark.gpu
 
 CELLS, ALLPAIRS = 4, 1
-E_INVALID = -1
-
-
-def _sim(N, path="auto"):
-    return LJSimulation(N, rc=2.5, dt=0.005, path=path, device=0)
-
-
-def _snapshots(sim, N, nsteps=30, every=10, seed=0):
-    R, V, box = lattice_jitter(N, seed=seed)
-    (_, _), traj = sim.run((R, V), nsteps, sample_every=every)
-    return traj.numpy(), float(box)
 
 
 def order(sim, Rs, m, r_nb):
@@ -51,26 +40,10 @@ def corr(sim, Rs, psi, nbins, r_max):
     return c.cpu().numpy(), w.cpu().numpy(), sim.launch_count() - l0
 
 
-def gr_counts(sim, Rs, nbins, r_max):
-    Rs = np.ascontiguousarray(Rs, np.float32).reshape(-1, sim.N, 2)
-    Rh = torch.from_numpy(Rs).cuda()
-    e = torch.from_numpy(edges_for(r_max, nbins)).cuda()
-    c = torch.full((Rs.shape[0], nbins), -1, dtype=torch.int64, device="cuda")
-    rc = sim.lib.ljmd_gr_hist_rmax(sim._h, Rh.data_ptr(), Rs.shape[0], nbins, e.data_ptr(),
-                                   float(edges_for(r_max, nbins)[-1]), c.data_ptr())
-    assert rc == 0, sim.lib.ljmd_last_error()
-    torch.cuda.synchronize()
-    return c.cpu().numpy()
-
-
-def _same_bits(a, b):
-    return np.array_equal(np.asarray(a).view(np.int64), np.asarray(b).view(np.int64))
-
-
 @pytest.mark.parametrize("N", [400, 4096, 65536])
 def test_psi_matches_reference(N):
-    sim = _sim(N)
-    th, box = _snapshots(sim, N)
+    sim = make_sim(N)
+    th, box = md_snapshots(sim, N)
     if N == 65536:
         th = th[:1]                                       # the reference visits all N^2 pairs below 65,536 + 1
     for m in (4, 6):
@@ -80,40 +53,40 @@ def test_psi_matches_reference(N):
             for s in range(th.shape[0]):
                 p_ref, n_ref = ref.bond_order(th[s], box, m, r_nb)
                 assert np.array_equal(n[s], n_ref), (m, r_nb, s)
-                assert _same_bits(psi[s], p_ref), (m, r_nb, s)
+                assert same_bits(psi[s], p_ref), (m, r_nb, s)
 
 
 def test_psi_matches_reference_4m():
     N = 4194304
-    sim = _sim(N, path="cells")
+    sim = make_sim(N, path="cells")
     R, _, box = lattice_jitter(N, seed=3)
     psi, n, _ = order(sim, R, 6, 1.5)
     p_ref, n_ref = ref.bond_order(R, box, 6, 1.5)
-    assert np.array_equal(n[0], n_ref) and _same_bits(psi[0], p_ref)
+    assert np.array_equal(n[0], n_ref) and same_bits(psi[0], p_ref)
 
 
 @pytest.mark.parametrize("N", [400, 4096])
 def test_adversarial_placements(N):
-    sim = _sim(N)
+    sim = make_sim(N)
     box = float(lattice_jitter(N)[2])
     for r_nb in (1.2, 1.5, 2.5, 5.0, 8.0):               # 8.0 at N = 400: one cell, all pairs
         X = adversarial(N, box, r_nb, seed=5)
         for m in (3, 6):
             psi, n, _ = order(sim, X, m, r_nb)
             p_ref, n_ref = ref.bond_order(X, box, m, r_nb)
-            assert np.array_equal(n[0], n_ref) and _same_bits(psi[0], p_ref), (r_nb, m)
+            assert np.array_equal(n[0], n_ref) and same_bits(psi[0], p_ref), (r_nb, m)
 
 
 @pytest.mark.parametrize("N,r_max,path", [(4096, 5.0, CELLS), (400, None, ALLPAIRS), (4096, None, ALLPAIRS)])
 def test_corr_counts_and_wsum(N, r_max, path):
-    sim = _sim(N)
-    th, box = _snapshots(sim, N)
+    sim = make_sim(N)
+    th, box = md_snapshots(sim, N)
     r_max = float(np.float32(box) / np.float32(2)) if r_max is None else r_max
     nbins = int(np.float32(r_max) / 0.05)
     psi, _, _ = order(sim, th, 6, 1.5)
     counts, wsum, launches = corr(sim, th, psi, nbins, r_max)
     assert launches == path
-    assert np.array_equal(counts, gr_counts(sim, th, nbins, r_max))
+    assert np.array_equal(counts, hist_rmax(sim, th, nbins, r_max)[0])
     for s in range(th.shape[0]):
         c_ref, w_ref = ref.bond_corr(th[s], psi[s], box, nbins, r_max)
         assert np.array_equal(counts[s], c_ref) and np.array_equal(wsum[s], w_ref), s
@@ -121,20 +94,19 @@ def test_corr_counts_and_wsum(N, r_max, path):
 
 @pytest.mark.parametrize("N", [400, 4096])
 def test_neighbour_count_is_twice_the_gr_count(N):
-    sim = _sim(N)
-    th, box = _snapshots(sim, N)
+    sim = make_sim(N)
+    th, box = md_snapshots(sim, N)
     # 8.0 at N = 400: fewer than 3 cells per side, so psi_m uses one cell and g(r) the all-pairs kernel
     for r_nb in (1.2, 1.5, 2.5, 8.0):
         _, n, _ = order(sim, th, 6, r_nb)
-        l0 = sim.launch_count()
-        counts = gr_counts(sim, th, 1, r_nb)
-        assert sim.launch_count() - l0 == (ALLPAIRS if N == 400 and r_nb == 8.0 else CELLS)
+        counts, launches = hist_rmax(sim, th, 1, r_nb)
+        assert launches == (ALLPAIRS if N == 400 and r_nb == 8.0 else CELLS)
         assert np.array_equal(n.sum(axis=1, dtype=np.int64), 2 * counts[:, 0]), r_nb
 
 
 def test_bond_correlation_api_and_lattice_physics():
     N = 4096
-    sim = _sim(N)
+    sim = make_sim(N)
     R, V, box = lattice_jitter(N, seed=1)
     a = float(box) / 64
     r_nb = 1.2 * a                                        # between a and the diagonal a sqrt(2)
@@ -149,7 +121,7 @@ def test_bond_correlation_api_and_lattice_physics():
     th = traj.numpy()
     centers, g = sim.bond_correlation(th, 5.0, 100, 6, 1.5)
     counts, wsum = sim.last_bond_counts.numpy(), sim.last_bond_wsum.numpy()
-    assert np.array_equal(counts, gr_counts(sim, th, 100, 5.0))
+    assert np.array_equal(counts, hist_rmax(sim, th, 100, 5.0)[0])
     assert np.array_equal(centers.numpy(), (edges_for(5.0, 100)[:-1] + edges_for(5.0, 100)[1:]) / np.float32(2))
     g_ref = ref.g_m(counts.sum(axis=0), wsum.astype(np.float64).sum(axis=0))
     assert np.array_equal(np.isnan(g.numpy()), np.isnan(g_ref))
@@ -158,14 +130,14 @@ def test_bond_correlation_api_and_lattice_physics():
 
 def test_determinism_and_batches():
     N = 4096
-    sim = _sim(N)
-    th, box = _snapshots(sim, N, nsteps=60, every=10)
+    sim = make_sim(N)
+    th, box = md_snapshots(sim, N, nsteps=60, every=10)
     psi, n, _ = order(sim, th, 6, 1.5)
     psi2, n2, _ = order(sim, th, 6, 1.5)
-    assert _same_bits(psi, psi2) and np.array_equal(n, n2)
+    assert same_bits(psi, psi2) and np.array_equal(n, n2)
     for s in range(th.shape[0]):
         p1, n1, _ = order(sim, th[s], 6, 1.5)
-        assert _same_bits(p1[0], psi[s]) and np.array_equal(n1[0], n[s])
+        assert same_bits(p1[0], psi[s]) and np.array_equal(n1[0], n[s])
     c, w, _ = corr(sim, th, psi, 100, 5.0)
     c2, w2, _ = corr(sim, th, psi, 100, 5.0)
     assert np.array_equal(c, c2) and np.array_equal(w, w2)
@@ -178,7 +150,7 @@ def test_batches_at_4m():
     """Eight snapshots of 4 M particles do not fit one 512 MiB batch of the grid scratch (16 B per particle for
     psi_m, 28 B for g_m(r))."""
     N = 4194304
-    sim = _sim(N, path="cells")
+    sim = make_sim(N, path="cells")
     R, _, box = lattice_jitter(N, seed=4)
     rng = np.random.default_rng(0)
     th = np.stack([np.clip(R + rng.uniform(-0.02, 0.02, R.shape).astype(np.float32), 0, box) for _ in range(8)])
@@ -189,16 +161,16 @@ def test_batches_at_4m():
     assert launches > CELLS
     for s in (0, 7):
         p1, n1, _ = order(sim, th[s], 6, 1.5)
-        assert _same_bits(p1[0], psi[s]) and np.array_equal(n1[0], n[s])
+        assert same_bits(p1[0], psi[s]) and np.array_equal(n1[0], n[s])
         c1, w1, _ = corr(sim, th[s], psi[s], 100, 5.0)
         assert np.array_equal(c1[0], c[s]) and np.array_equal(w1[0], w[s])
-    assert np.array_equal(c, gr_counts(sim, th, 100, 5.0))
+    assert np.array_equal(c, hist_rmax(sim, th, 100, 5.0)[0])
 
 
 def test_nan_particle_rule():
     N = 4096
-    sim = _sim(N)
-    th, box = _snapshots(sim, N, nsteps=20)
+    sim = make_sim(N)
+    th, box = md_snapshots(sim, N, nsteps=20)
     X = th.copy()
     X[0, 17] = (np.nan, 1.0)
     X[1, 99, 1] = np.inf
@@ -206,9 +178,9 @@ def test_nan_particle_rule():
     assert np.isnan(psi[0, 17]).all() and n[0, 17] == 0 and np.isnan(psi[1, 99]).all() and n[1, 99] == 0
     for s in range(X.shape[0]):
         p_ref, n_ref = ref.bond_order(X[s], box, 6, 1.5)
-        assert np.array_equal(n[s], n_ref) and _same_bits(psi[s], p_ref)
+        assert np.array_equal(n[s], n_ref) and same_bits(psi[s], p_ref)
     c, w, _ = corr(sim, X, psi, 100, 5.0)
-    assert np.array_equal(c, gr_counts(sim, X, 100, 5.0))
+    assert np.array_equal(c, hist_rmax(sim, X, 100, 5.0)[0])
     for s in range(X.shape[0]):
         c_ref, w_ref = ref.bond_corr(X[s], psi[s], box, 100, 5.0)
         assert np.array_equal(c[s], c_ref) and np.array_equal(w[s], w_ref)
@@ -217,11 +189,11 @@ def test_nan_particle_rule():
 
 def test_handles_agree():
     N = 4096
-    a, b = _sim(N, path="allpairs"), _sim(N, path="cells")
-    th, _ = _snapshots(a, N, nsteps=20)
+    a, b = make_sim(N, path="allpairs"), make_sim(N, path="cells")
+    th, _ = md_snapshots(a, N, nsteps=20)
     pa, na, _ = order(a, th, 6, 1.5)
     pb, nb, _ = order(b, th, 6, 1.5)
-    assert _same_bits(pa, pb) and np.array_equal(na, nb)
+    assert same_bits(pa, pb) and np.array_equal(na, nb)
     ca, wa, _ = corr(a, th, pa, 100, 5.0)
     cb, wb, _ = corr(b, th, pb, 100, 5.0)
     assert np.array_equal(ca, cb) and np.array_equal(wa, wb)
@@ -229,7 +201,7 @@ def test_handles_agree():
 
 def test_empty_history_and_argument_errors():
     N = 4096
-    sim = _sim(N)
+    sim = make_sim(N)
     psi, n = sim.bond_order(np.zeros((0, N, 2), np.float32))
     assert psi.shape == (0, N, 2) and n.shape == (0, N)
     _, g = sim.bond_correlation(np.zeros((0, N, 2), np.float32), 5.0)

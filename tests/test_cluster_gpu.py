@@ -7,30 +7,13 @@ import pytest
 import torch
 
 import cluster_reference as ref
-from gr_reference import adversarial, edges_for
+from analysis_helpers import E_INVALID, hist_rmax, make_sim, md_snapshots, uniform_snapshots
+from gr_reference import adversarial
 from jax_tpus_benchmark_physics_simulation_b200 import lattice_jitter
-from jax_tpus_benchmark_physics_simulation_b200.md import LJSimulation
 
 pytestmark = pytest.mark.gpu
 
 LAUNCHES = 6
-E_INVALID = -1
-
-
-def _sim(N, path="auto", rho=0.8):
-    return LJSimulation(N, rho=rho, rc=2.5, dt=0.005, path=path, device=0)
-
-
-def _snapshots(sim, N, nsteps=30, every=10, seed=0):
-    R, V, box = lattice_jitter(N, seed=seed)
-    (_, _), traj = sim.run((R, V), nsteps, sample_every=every)
-    return traj.numpy(), float(box)
-
-
-def _uniform(sim, S, seed=0):
-    rng = np.random.default_rng(seed)
-    box = np.float32(sim.box_size)
-    return (rng.random((S, sim.N, 2), dtype=np.float32) * box).astype(np.float32), float(box)
 
 
 def run(sim, Rs, r_link, mask=None):
@@ -51,29 +34,16 @@ def check_ref(sim, Rs, box, r_link, mask=None):
     return labels, sizes, launches
 
 
-def gr_count(sim, Rs, r_link):
-    """ljmd_gr_hist_rmax count on the single bin [0, r_link] of every snapshot."""
-    Rs = np.ascontiguousarray(Rs, np.float32).reshape(-1, sim.N, 2)
-    Rh = torch.from_numpy(Rs).cuda()
-    e = torch.from_numpy(edges_for(r_link, 1)).cuda()
-    c = torch.full((Rs.shape[0], 1), -1, dtype=torch.int64, device="cuda")
-    rc = sim.lib.ljmd_gr_hist_rmax(sim._h, Rh.data_ptr(), Rs.shape[0], 1, e.data_ptr(),
-                                   float(edges_for(r_link, 1)[-1]), c.data_ptr())
-    assert rc == 0, sim.lib.ljmd_last_error()
-    torch.cuda.synchronize()
-    return c.cpu().numpy()[:, 0]
-
-
 @pytest.mark.parametrize("N", [400, 4096, 65536])
 def test_matches_reference(N):
-    sim = _sim(N)
-    th, box = _snapshots(sim, N)
+    sim = make_sim(N)
+    th, box = md_snapshots(sim, N)
     for r_link in (1.1, 1.5, 2.5):
         _, _, launches = check_ref(sim, th, box, r_link)
         assert launches == LAUNCHES
     for rho in (0.05, 0.3, 0.8):
-        s = _sim(N, rho=rho)
-        X, b = _uniform(s, 2, seed=int(rho * 100))
+        s = make_sim(N, rho=rho)
+        X, b = uniform_snapshots(s, 2, seed=int(rho * 100))
         for r_link in (1.1, 1.5, 2.5):
             check_ref(s, X, b, r_link)
 
@@ -81,7 +51,7 @@ def test_matches_reference(N):
 @pytest.mark.parametrize("r_link", [1.5, 1.05])
 def test_matches_reference_4m(r_link):
     N = 4194304
-    sim = _sim(N, path="cells")
+    sim = make_sim(N, path="cells")
     R, _, box = lattice_jitter(N, seed=3)
     labels, sizes, _ = check_ref(sim, R, box, r_link)
     n = int((sizes[0] > 0).sum())
@@ -90,8 +60,8 @@ def test_matches_reference_4m(r_link):
 
 
 def test_one_cell():
-    sim = _sim(400)
-    th, box = _snapshots(sim, 400)
+    sim = make_sim(400)
+    th, box = md_snapshots(sim, 400)
     assert 8.0 > box / 3
     check_ref(sim, th, box, 8.0)
     check_ref(sim, th, box, 0.9)
@@ -99,7 +69,7 @@ def test_one_cell():
 
 @pytest.mark.parametrize("N", [400, 4096])
 def test_adversarial_placements(N):
-    sim = _sim(N)
+    sim = make_sim(N)
     box = float(lattice_jitter(N)[2])
     for r_link in (1.2, 1.5, 2.5, 5.0, 8.0):
         X = adversarial(N, box, r_link, seed=5)
@@ -109,9 +79,9 @@ def test_adversarial_placements(N):
 
 
 def test_exact_distance_and_one_ulp():
-    sim = _sim(4096)
+    sim = make_sim(4096)
     box = np.float32(sim.box_size)
-    X, _ = _uniform(sim, 1, seed=3)
+    X, _ = uniform_snapshots(sim, 1, seed=3)
     X = X[0] * np.float32(0.5)                                      # leave the upper half free
     y = np.float32(0.75) * box
     X[10] = (np.float32(3.0), y)
@@ -130,7 +100,7 @@ def test_exact_distance_and_one_ulp():
 
 def test_permuted_chain_and_periodic_ring():
     N = 65536
-    sim = _sim(N)
+    sim = make_sim(N)
     box = np.float32(sim.box_size)
     rng = np.random.default_rng(7)
     X = (rng.random((N, 2), dtype=np.float32) * box * np.float32(0.4)).astype(np.float32)
@@ -152,8 +122,8 @@ def test_permuted_chain_and_periodic_ring():
 
 def test_coincident_particles():
     N = 4096
-    sim = _sim(N)
-    X, box = _uniform(sim, 1, seed=9)
+    sim = make_sim(N)
+    X, box = uniform_snapshots(sim, 1, seed=9)
     X[0, :1000] = X[0, 123]                                         # 1000 particles on one point
     labels, sizes, _ = check_ref(sim, X, box, 1.1)
     assert np.all(labels[0, :1000] == 0) and sizes[0, 0] >= 1000
@@ -161,8 +131,8 @@ def test_coincident_particles():
 
 def test_masks():
     N = 4096
-    sim = _sim(N)
-    th, box = _snapshots(sim, N)
+    sim = make_sim(N)
+    th, box = md_snapshots(sim, N)
     rng = np.random.default_rng(2)
     check_ref(sim, th, box, 1.5, rng.random(th.shape[:2]) < 0.5)
     check_ref(sim, th, box, 1.5, (rng.random(N) < 0.3).astype(np.uint8))            # broadcast (N,)
@@ -180,8 +150,8 @@ def test_masks():
 
 def test_nan_rule():
     N = 4096
-    sim = _sim(N)
-    th, box = _snapshots(sim, N, nsteps=20)
+    sim = make_sim(N)
+    th, box = md_snapshots(sim, N, nsteps=20)
     X = th.copy()
     X[0, 17] = (np.nan, 1.0)
     X[1, 99, 1] = np.inf
@@ -196,8 +166,8 @@ def test_nan_rule():
 
 @pytest.mark.parametrize("N", [400, 65536])
 def test_invariants_and_link_count(N):
-    sim = _sim(N)
-    th, box = _snapshots(sim, N)
+    sim = make_sim(N)
+    th, box = md_snapshots(sim, N)
     for r_link in (1.1, 1.5):
         labels, sizes, _ = run(sim, th, r_link)
         for s in range(th.shape[0]):
@@ -207,13 +177,13 @@ def test_invariants_and_link_count(N):
             assert np.array_equal(np.nonzero(sizes[s])[0], np.unique(on))
         assert np.array_equal(sim.last_cluster_largest.numpy(), sizes.max(axis=1))
         n_links = np.array([len(ref.links(th[s], box, r_link)) for s in range(th.shape[0])])
-        assert np.array_equal(n_links, gr_count(sim, th, r_link)), r_link
+        assert np.array_equal(n_links, hist_rmax(sim, th, 1, r_link)[0][:, 0]), r_link
 
 
 def test_determinism_and_handles():
     N = 4096
-    a, b = _sim(N, path="allpairs"), _sim(N, path="cells")
-    th, _ = _snapshots(a, N, nsteps=60, every=10)
+    a, b = make_sim(N, path="allpairs"), make_sim(N, path="cells")
+    th, _ = md_snapshots(a, N, nsteps=60, every=10)
     la, sa, _ = run(a, th, 1.5)
     la2, sa2, _ = run(a, th, 1.5)
     lb, sb, _ = run(b, th, 1.5)
@@ -227,7 +197,7 @@ def test_determinism_and_handles():
 def test_batches_at_4m():
     """Ten snapshots of 4 M particles do not fit one 512 MiB batch of the grid scratch (16 B per particle)."""
     N = 4194304
-    sim = _sim(N, path="cells")
+    sim = make_sim(N, path="cells")
     R, _, box = lattice_jitter(N, seed=4)
     rng = np.random.default_rng(0)
     th = np.stack([np.clip(R + rng.uniform(-0.05, 0.05, R.shape).astype(np.float32), 0, box)
@@ -241,8 +211,8 @@ def test_batches_at_4m():
 
 def test_distribution():
     N = 4096
-    sim = _sim(N, rho=0.3)
-    X, _ = _uniform(sim, 3, seed=11)
+    sim = make_sim(N, rho=0.3)
+    X, _ = uniform_snapshots(sim, 3, seed=11)
     _, sizes = sim.clusters(X, 1.5)
     s, n_s = sim.cluster_distribution(sizes)
     sz = sizes.numpy()
@@ -253,7 +223,7 @@ def test_distribution():
 
 def test_empty_history_and_argument_errors():
     N = 4096
-    sim = _sim(N)
+    sim = make_sim(N)
     labels, sizes = sim.clusters(np.zeros((0, N, 2), np.float32), 1.5)
     assert labels.shape == (0, N) and sizes.shape == (0, N)
     lib, h = sim.lib, sim._h
@@ -293,7 +263,7 @@ def test_driver_clusters(tmp_path, capsys, extra):
     stem = str(tmp_path / "g_r_plot")
     saved = np.load(stem + "_clusters.npy")
     assert np.allclose(np.loadtxt(stem + "_clusters.csv", delimiter=",").reshape(-1, 2), saved.T)
-    sim = _sim(400)
+    sim = make_sim(400)
     mask = None
     if extra:
         psi, _ = sim.bond_order(R_history, 6, 1.5)

@@ -2,59 +2,23 @@
 dense CPU recount (oracle.c_gr_hist), the cell-grid CPU recount (tests/gr_reference.c) and the all-pairs
 kernel (ljmd_gr_hist).  Which kernel ran is read from the launch counter: the cell grid makes four
 launches per batch of snapshots, the all-pairs histogram one."""
-import ctypes
-
 import numpy as np
 import pytest
 import torch
 
+from analysis_helpers import E_INVALID, hist_call, hist_rmax, make_sim, md_snapshots
 from gr_reference import adversarial, c_gr_hist_cells, edges_for
 from jax_tpus_benchmark_physics_simulation_b200 import lattice_jitter
-from jax_tpus_benchmark_physics_simulation_b200.md import LJSimulation
 
 pytestmark = pytest.mark.gpu
 
 CELLS, ALLPAIRS = 4, 1                  # launches of one call with one batch of snapshots
-E_INVALID = -1
-
-
-def _sim(N, path="auto"):
-    return LJSimulation(N, rc=2.5, dt=0.005, path=path, device=0)
-
-
-def _call(sim, fn, Rs, nbins, r_edges, *extra):
-    Rs = np.ascontiguousarray(Rs, dtype=np.float32).reshape(-1, sim.N, 2)
-    Rh = torch.from_numpy(Rs).cuda()
-    edges = torch.from_numpy(edges_for(r_edges, nbins)).cuda()
-    counts = torch.full((Rs.shape[0], nbins), -1, dtype=torch.int64, device="cuda")
-    l0 = sim.launch_count()
-    rc = fn(sim._h, Rh.data_ptr(), Rs.shape[0], nbins, edges.data_ptr(), *extra, counts.data_ptr())
-    assert rc == 0, sim.lib.ljmd_last_error()
-    torch.cuda.synchronize()
-    return counts.cpu().numpy(), sim.launch_count() - l0
-
-
-def hist_rmax(sim, Rs, nbins, r_edges, r_max=None):
-    """ljmd_gr_hist_rmax with edges linspace(0, r_edges, nbins + 1) and r_max (default: the last edge).
-    Returns (counts (S, nbins), launches)."""
-    r_max = edges_for(r_edges, nbins)[-1] if r_max is None else np.float32(r_max)
-    return _call(sim, sim.lib.ljmd_gr_hist_rmax, Rs, nbins, r_edges, float(r_max))
-
-
-def hist_all(sim, Rs, nbins, r_edges):
-    return _call(sim, sim.lib.ljmd_gr_hist, Rs, nbins, r_edges)[0]
-
-
-def _snapshots(sim, N, nsteps=30, every=10, seed=0):
-    R, V, box = lattice_jitter(N, seed=seed)
-    (_, _), traj = sim.run((R, V), nsteps, sample_every=every)
-    return traj.numpy(), float(box)
 
 
 @pytest.mark.parametrize("N", [400, 4096])
 def test_counts_match_dense_oracle(oracle, N):
-    sim = _sim(N)
-    th, box = _snapshots(sim, N)
+    sim = make_sim(N)
+    th, box = md_snapshots(sim, N)
     b32 = np.float32(box)
     for r_max in (2.5, 5.0, float(b32 / np.float32(3)) * (1 - 1e-5), float(b32 / np.float32(2))):
         nbins = int(np.float32(r_max) / 0.05)
@@ -67,8 +31,8 @@ def test_counts_match_dense_oracle(oracle, N):
 
 def test_calculate_g_r_uses_the_grid(oracle):
     N = 4096
-    sim = _sim(N)
-    th, box = _snapshots(sim, N)
+    sim = make_sim(N)
+    th, box = md_snapshots(sim, N)
     l0 = sim.launch_count()
     centers, g = sim.calculate_g_r(th, N, box, 100, 5.0)
     assert sim.launch_count() - l0 == CELLS
@@ -80,17 +44,17 @@ def test_calculate_g_r_uses_the_grid(oracle):
 
 def test_grid_equals_all_pairs_kernel_65536():
     N = 65536
-    sim = _sim(N, path="allpairs")
-    th, box = _snapshots(sim, N, nsteps=20)
+    sim = make_sim(N, path="allpairs")
+    th, box = md_snapshots(sim, N, nsteps=20)
     cells, launches = hist_rmax(sim, th, 100, 5.0)
     assert launches == CELLS
-    dense = hist_all(sim, th, 100, 5.0)
+    dense = hist_call(sim, sim.lib.ljmd_gr_hist, th, 100, 5.0)[0]
     assert np.array_equal(cells, dense) and dense.sum() > 0
 
 
 @pytest.mark.parametrize("N", [400, 4096])
 def test_adversarial_geometry(oracle, N):
-    sim = _sim(N)
+    sim = make_sim(N)
     box = float(lattice_jitter(N)[2])
     b32 = np.float32(box)
     k = int(box // 5.0)
@@ -108,7 +72,7 @@ def test_adversarial_geometry(oracle, N):
 def test_clumped_state(oracle):
     """Many particles in one cell and empty cells elsewhere: big cells are walked in chunks."""
     N = 4096
-    sim = _sim(N)
+    sim = make_sim(N)
     box = float(lattice_jitter(N)[2])
     rng = np.random.default_rng(11)
     X = np.zeros((N, 2), np.float32)
@@ -124,7 +88,7 @@ def test_huge_clump_overflows_to_global_counts():
     """A cell with 30,000 particles: one warp bins more pairs than its share of the CTA's 32-bit
     counters may hold, and the rest goes straight to the 64-bit counts."""
     N = 65536
-    sim = _sim(N, path="allpairs")
+    sim = make_sim(N, path="allpairs")
     box = float(lattice_jitter(N)[2])
     rng = np.random.default_rng(12)
     X = (rng.random((N, 2)) * box).astype(np.float32)
@@ -138,8 +102,8 @@ def test_huge_clump_overflows_to_global_counts():
 
 def test_rmax_below_last_edge_drops_longer_pairs():
     N = 4096
-    sim = _sim(N)
-    th, box = _snapshots(sim, N, nsteps=20)
+    sim = make_sim(N)
+    th, box = md_snapshots(sim, N, nsteps=20)
     X = np.concatenate([th, adversarial(N, box, 3.3, seed=2)[None]])
     half = float(np.float32(box) / np.float32(2))
     for r_edges, r_max, path in ((5.0, 3.3, CELLS), (5.0, 2.5, CELLS), (half, half * 0.9, ALLPAIRS)):
@@ -153,8 +117,8 @@ def test_rmax_below_last_edge_drops_longer_pairs():
 def test_config4_scale(oracle):
     """Cell-list run at N = 4,194,304; g(r) to r_max = 5 with 100 bins."""
     N = 4194304
-    sim = _sim(N, path="cells")
-    th, box = _snapshots(sim, N, nsteps=20)
+    sim = make_sim(N, path="cells")
+    th, box = md_snapshots(sim, N, nsteps=20)
     assert th.shape[0] == 2
     l0 = sim.launch_count()
     centers, g = sim.calculate_g_r(th, N, box, 100, 5.0)
@@ -172,7 +136,7 @@ def test_config4_scale(oracle):
 
 def test_empty_history_and_argument_errors():
     N = 4096
-    sim = _sim(N)
+    sim = make_sim(N)
     counts, _ = hist_rmax(sim, np.zeros((0, N, 2), np.float32), 100, 5.0)
     assert counts.shape == (0, 100)
     _, g = sim.calculate_g_r(np.zeros((0, N, 2), np.float32), N, None, 100, 5.0)

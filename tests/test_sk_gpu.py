@@ -7,18 +7,14 @@ import numpy as np
 import pytest
 import torch
 
+from analysis_helpers import E_INVALID, make_sim, md_snapshots
 from jax_tpus_benchmark_physics_simulation_b200 import lattice_jitter
-from jax_tpus_benchmark_physics_simulation_b200.md import LJSimulation, structure_factor_vectors
+from jax_tpus_benchmark_physics_simulation_b200.md import structure_factor_vectors
 from sk_reference import bound, c_density_modes
 
 pytestmark = pytest.mark.gpu
 
-E_INVALID = -1
 LAUNCHES = 2                            # per batch of snapshots and vectors
-
-
-def _sim(N, path="auto", **kw):
-    return LJSimulation(N, rc=2.5, dt=0.005, path=path, device=0, **kw)
 
 
 def _half_plane(nmax):
@@ -35,12 +31,6 @@ def modes(sim, R, nvec):
     return rho, sim.launch_count() - l0
 
 
-def _snapshots(sim, N, nsteps=30, every=10, seed=0):
-    R, V, box = lattice_jitter(N, seed=seed)
-    (_, _), traj = sim.run((R, V), nsteps, sample_every=every)
-    return traj.numpy(), box
-
-
 def _check_bound(got, ref, N, nvec, what):
     b = bound(N, nvec)
     err = np.abs(got - ref).max(axis=-1)                  # (S, K): worse of Re and Im
@@ -53,8 +43,8 @@ def _check_bound(got, ref, N, nvec, what):
 
 @pytest.mark.parametrize("N", [400, 4096])
 def test_snapshots_against_reference(N):
-    sim = _sim(N)
-    th, box = _snapshots(sim, N)
+    sim = make_sim(N)
+    th, box = md_snapshots(sim, N)
     nv = _half_plane(40)
     rho, launches = modes(sim, th, nv)
     assert rho.shape == (th.shape[0], nv.shape[0], 2) and launches == LAUNCHES
@@ -63,7 +53,7 @@ def test_snapshots_against_reference(N):
 
 def test_large_n_against_reference():
     N = 4194304
-    sim = _sim(N, path="cells")
+    sim = make_sim(N, path="cells")
     R, _, box = lattice_jitter(N, seed=3)
     nv = _half_plane(8)
     rho, launches = modes(sim, R, nv)
@@ -75,7 +65,7 @@ def test_large_n_against_reference():
 def test_square_lattice_bragg_peaks():
     m = 64
     N = m * m
-    sim = _sim(N, box_size=float(m))
+    sim = make_sim(N, box_size=float(m))
     ii, jj = np.meshgrid(np.arange(m), np.arange(m), indexing="ij")
     R = np.stack([ii.ravel(), jj.ravel()], axis=1).astype(np.float32)       # exact phase words
     nv = _half_plane(2 * m + 2)
@@ -89,7 +79,7 @@ def test_square_lattice_bragg_peaks():
 
 def test_uniform_random_points():
     N = 4096
-    sim = _sim(N)
+    sim = make_sim(N)
     box = float(sim.box_size)
     R = (np.random.default_rng(21).random((N, 2)) * box).astype(np.float32)
     nv, _ = structure_factor_vectors(box, 8.0)
@@ -102,8 +92,8 @@ def test_uniform_random_points():
 
 def test_large_wave_numbers():
     N = 400
-    sim = _sim(N)
-    th, box = _snapshots(sim, N, nsteps=10, every=10)
+    sim = make_sim(N)
+    th, box = md_snapshots(sim, N, nsteps=10, every=10)
     rng = np.random.default_rng(5)
     nv = np.concatenate([np.array([[8192, 0], [0, 8192], [8192, -8192], [-8192, 8192], [5000, 7000],
                                    [8191, 1], [1, -8191]], np.int32),
@@ -120,7 +110,7 @@ def _dyadic_state(N, box, seed):
 
 def test_periodic_images_give_the_same_bits():
     N, box = 4096, 64.0
-    sim = _sim(N, box_size=box)
+    sim = make_sim(N, box_size=box)
     R = _dyadic_state(N, box, 1)
     imgs = np.stack([R, R + np.float32(box), R - np.float32(box),
                      R + np.array([box, -2 * box], np.float32)]).astype(np.float32)
@@ -134,7 +124,7 @@ def test_periodic_images_give_the_same_bits():
 
 def test_translation_keeps_the_modulus():
     N, box = 4096, 64.0
-    sim = _sim(N, box_size=box)
+    sim = make_sim(N, box_size=box)
     R = _dyadic_state(N, box, 2)
     d = np.array([13.375, -7.5], np.float32)
     nv = _half_plane(30)
@@ -146,8 +136,8 @@ def test_translation_keeps_the_modulus():
 
 def test_deterministic_and_independent_of_the_batch():
     N = 4096
-    sim = _sim(N)
-    th, _ = _snapshots(sim, N, nsteps=50, every=10)
+    sim = make_sim(N)
+    th, _ = md_snapshots(sim, N, nsteps=50, every=10)
     nv = _half_plane(40)
     a = modes(sim, th, nv)[0]
     b = modes(sim, th, nv)[0]
@@ -162,7 +152,7 @@ def test_scratch_batches_give_the_single_batch_bits():
     """N = 2^20 has 1024 particle segments, so 16 KiB of scratch per (snapshot, vector): a call with more than
     32,768 vectors, or more snapshots than fit next to them in 512 MiB, is split into several batches."""
     N = 1 << 20
-    sim = _sim(N, path="cells")
+    sim = make_sim(N, path="cells")
     R, _, box = lattice_jitter(N, seed=9)
     nv = _half_plane(160)[:40000]
     assert nv.shape[0] == 40000
@@ -184,8 +174,8 @@ def test_scratch_batches_give_the_single_batch_bits():
 
 def test_nan_snapshot_rows():
     N = 4096
-    sim = _sim(N)
-    th, _ = _snapshots(sim, N)
+    sim = make_sim(N)
+    th, _ = md_snapshots(sim, N)
     nv = _half_plane(20)
     clean = modes(sim, th, nv)[0]
     for bad in (np.nan, np.inf, -np.inf):
@@ -200,8 +190,8 @@ def test_nan_snapshot_rows():
 
 def test_structure_factor_is_the_shell_mean():
     N = 4096
-    sim = _sim(N)
-    th, box = _snapshots(sim, N)
+    sim = make_sim(N)
+    th, box = md_snapshots(sim, N)
     k, S = sim.structure_factor(th, 4.0)
     nv, shell = structure_factor_vectors(float(box), 4.0)
     assert np.array_equal(sim.last_sk_nvec, nv) and np.array_equal(sim.last_sk_shell, shell)
@@ -226,7 +216,7 @@ def test_structure_factor_is_the_shell_mean():
 
 def test_argument_errors_and_empty_calls():
     N = 400
-    sim = _sim(N)
+    sim = make_sim(N)
     lib, h = sim.lib, sim._h
     R = torch.zeros((2, N, 2), dtype=torch.float32, device="cuda")
     nv = torch.ones((3, 2), dtype=torch.int32, device="cuda")
@@ -262,7 +252,7 @@ def test_all_pairs_and_cell_list_handles():
     nv = _half_plane(12)
     out = []
     for path in ("allpairs", "cells"):
-        sim = _sim(N, path=path)
+        sim = make_sim(N, path=path)
         rho, launches = modes(sim, R, nv)
         assert launches == LAUNCHES
         out.append(rho)

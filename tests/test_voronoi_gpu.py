@@ -8,30 +8,14 @@ import pytest
 import torch
 
 import voronoi_reference as ref
+from analysis_helpers import E_INVALID, make_sim, md_snapshots, uniform_snapshots
 from jax_tpus_benchmark_physics_simulation_b200 import lattice_jitter
-from jax_tpus_benchmark_physics_simulation_b200.md import LJSimulation, topological_defects
+from jax_tpus_benchmark_physics_simulation_b200.md import topological_defects
 
 pytestmark = pytest.mark.gpu
 
 LAUNCHES = 4
-E_INVALID = -1
 TOL = 1e-9
-
-
-def _sim(N, path="auto", rho=0.8):
-    return LJSimulation(N, rho=rho, rc=2.5, dt=0.005, path=path, device=0)
-
-
-def _snapshots(sim, N, nsteps=20, every=10, seed=0):
-    R, V, box = lattice_jitter(N, seed=seed)
-    (_, _), traj = sim.run((R, V), nsteps, sample_every=every)
-    return traj.numpy(), float(box)
-
-
-def _uniform(sim, S, seed=0):
-    rng = np.random.default_rng(seed)
-    box = np.float32(sim.box_size)
-    return (rng.random((S, sim.N, 2), dtype=np.float32) * box).astype(np.float32), float(box)
 
 
 def run(sim, Rs, m=None, adj_cap=64):
@@ -76,19 +60,19 @@ def check_ref(sim, Rs, box, ms=(4, 6)):
 
 @pytest.mark.parametrize("N", [400, 4096, 65536])
 def test_matches_reference(N):
-    sim = _sim(N)
-    th, box = _snapshots(sim, N)
+    sim = make_sim(N)
+    th, box = md_snapshots(sim, N, nsteps=20)
     _, _, _, launches = check_ref(sim, th, box)
     assert launches == LAUNCHES
     for rho in (0.05, 0.3, 0.8):
-        sr = _sim(N, rho=rho)
-        X, b = _uniform(sr, 1, seed=int(rho * 100))
+        sr = make_sim(N, rho=rho)
+        X, b = uniform_snapshots(sr, 1, seed=int(rho * 100))
         check_ref(sr, X, b)
 
 
 def test_exact_square_lattice():
     N = 4096
-    sim = _sim(N, rho=1.0)
+    sim = make_sim(N, rho=1.0)
     assert sim.box_size == 64.0
     g = np.arange(64, dtype=np.float32) + np.float32(0.5)
     X = np.stack(np.meshgrid(g, g), axis=-1).reshape(N, 2).astype(np.float32)
@@ -111,9 +95,9 @@ def _symmetric(adj):
 
 @pytest.mark.parametrize("N,path", [(4194304, "cells"), (16777216, "cells")])
 def test_large(N, path):
-    sim = _sim(N, path=path)
+    sim = make_sim(N, path=path)
     if N == 4194304:
-        th, box = _snapshots(sim, N, nsteps=10, every=10, seed=3)
+        th, box = md_snapshots(sim, N, nsteps=10, every=10, seed=3)
         X = th[0]
     else:
         R, _, box = lattice_jitter(N, seed=3)
@@ -141,8 +125,8 @@ def test_large(N, path):
 
 def test_determinism_handles_and_snapshots():
     N = 4096
-    a, b = _sim(N, path="allpairs"), _sim(N, path="cells")
-    th, _ = _snapshots(a, N, nsteps=60, every=10)
+    a, b = make_sim(N, path="allpairs"), make_sim(N, path="cells")
+    th, _ = md_snapshots(a, N, nsteps=60, every=10)
     ra = run(a, th, 6)
     ra2 = run(a, th, 6)
     rb = run(b, th, 6)
@@ -157,7 +141,7 @@ def test_determinism_handles_and_snapshots():
 def test_batches_at_4m():
     """Ten snapshots of 4 M particles do not fit one 512 MiB batch of the grid scratch (16 B per particle)."""
     N = 4194304
-    sim = _sim(N, path="cells")
+    sim = make_sim(N, path="cells")
     R, _, box = lattice_jitter(N, seed=4)
     rng = np.random.default_rng(0)
     th = np.stack([np.clip(R + rng.uniform(-0.05, 0.05, R.shape).astype(np.float32), 0, box)
@@ -172,8 +156,8 @@ def test_batches_at_4m():
 
 def test_nan_rule():
     N = 4096
-    sim = _sim(N)
-    th, box = _snapshots(sim, N, nsteps=20)
+    sim = make_sim(N)
+    th, box = md_snapshots(sim, N, nsteps=20)
     X = th.copy()
     X[0, 17] = (np.nan, 1.0)
     X[1, 99, 1] = np.inf
@@ -186,8 +170,8 @@ def test_nan_rule():
 def test_vertex_cap():
     """A particle at the centre of a ring of 70 sites would need 70 vertices: incomplete; the rest as Qhull."""
     N = 4096
-    sim = _sim(N, rho=0.3)
-    X, box = _uniform(sim, 1, seed=5)
+    sim = make_sim(N, rho=0.3)
+    X, box = uniform_snapshots(sim, 1, seed=5)
     X = X[0]
     c = np.float32(box / 2)
     far = np.hypot(X[:, 0] - c, X[:, 1] - c) > 6.0
@@ -206,12 +190,12 @@ def test_vertex_cap():
 
 
 def test_tiny_box_and_void():
-    sim = _sim(16)
-    X, box = _uniform(sim, 4, seed=2)
+    sim = make_sim(16)
+    X, box = uniform_snapshots(sim, 4, seed=2)
     nvor, _, _, _ = check_ref(sim, X, box)
     assert (nvor == -1).any() and (nvor > 0).any()               # both kinds of rows occur
-    sim = _sim(400)
-    X, box = _uniform(sim, 1, seed=6)
+    sim = make_sim(400)
+    X, box = uniform_snapshots(sim, 1, seed=6)
     X = X[0] * np.float32(0.5)                                    # everything in one quarter of the box ...
     X[7] = (np.float32(0.75) * box, np.float32(0.75) * box)      # ... but one particle
     nvor, _, _, _ = check_ref(sim, X, box)
@@ -221,8 +205,8 @@ def test_tiny_box_and_void():
 def test_coincident_sites():
     """Coincident particles share one cell; their neighbours list only the smallest index of the group."""
     N = 4096
-    sim = _sim(N)
-    X, box = _uniform(sim, 1, seed=9)
+    sim = make_sim(N)
+    X, box = uniform_snapshots(sim, 1, seed=9)
     X[0, 100:105] = X[0, 3000]
     nvor, area, adj, _ = check_ref(sim, X, box)
     for k in list(range(100, 105)):
@@ -233,7 +217,7 @@ def test_coincident_sites():
 
 def test_empty_history_and_argument_errors():
     N = 4096
-    sim = _sim(N)
+    sim = make_sim(N)
     nvor, area = sim.voronoi(np.zeros((0, N, 2), np.float32), m=6)
     assert nvor.shape == (0, N) and area.shape == (0, N)
     lib, h = sim.lib, sim._h
@@ -278,7 +262,7 @@ def test_driver_voronoi(tmp_path, capsys, N, extra):
     stem = str(tmp_path / "g_r_plot")
     saved = np.load(stem + "_voronoi.npy")
     assert np.array_equal(np.loadtxt(stem + "_voronoi.csv", delimiter=",", dtype=np.int64).reshape(-1, 8), saved)
-    sim = _sim(N)
+    sim = make_sim(N)
     nvor, _ = sim.voronoi(R_history, adj_cap=16)
     d = topological_defects(nvor, sim.last_voronoi_adj)
     assert np.array_equal(saved[:, 0], d["n5"].cpu().numpy()) and np.array_equal(saved[:, 6],
